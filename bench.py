@@ -5,6 +5,7 @@
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
          --master-port P bench.py --gpus N --steps K --warmup W
   python bench.py --impl reference --steps 5 --warmup 2      # HF fp32 CPU step on the host cores
+  python bench.py --steps 20 --warmup 5 --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
 
 A step = forward + backward + AdamW (global-norm clip 1.0, as HF Trainer runs it) on a per-GPU
 batch of 16 synthetic 384×384 images.  `value` is timed with CUDA events with the inputs already
@@ -300,6 +301,28 @@ def gemm_chain_time(plans, stream, reps=3):
     return tot_f, best, len(calls)
 
 
+DUMP_PARAM_SAMPLE = 1 << 22         # fp32 parameters kept by --dump-outputs: 16 MB of ViT-B's 344 MB (ViT-L: 1.2 GB)
+
+
+def last_step_outputs(model, B, loss):
+    """On-device copies of what the last timed training step computed, taken before any later leg overwrites it: the
+    loss, the logits (the arena buffer the module's output is cloned from; the backward and the optimizer leave it
+    alone) and a fixed seeded sample of the updated fp32 master parameters."""
+    import torch
+    flat = model.flat_parameters()
+    g = torch.Generator().manual_seed(0)
+    idx = torch.randint(0, flat.numel(), (min(DUMP_PARAM_SAMPLE, flat.numel()),), generator=g).to(flat.device)
+    return {"loss": torch.tensor([loss], dtype=torch.float32), "logits": model.engine().arena(B, True).logits.clone(),
+            "params_sample": flat[idx]}
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def build_model(conf, dev):
     import torch
     import chest_x_ray_vit_b200 as pkg
@@ -421,6 +444,7 @@ def run_ours(args):
     barrier()
     ms_max, launches, clocks, last_loss = timed(K, True)
     value = world * B * K / (ms_max / 1e3)
+    dump = last_step_outputs(model, B, last_loss) if (args.dump_outputs and rank == 0) else None
 
     # ---------------- end-to-end through the public API with host buffers (`e2e`)
     # the reference's collate contract (fp32 [B,3,S,S] + fp32 labels, ViT-Training.py:77-80) in pinned host memory, fed by
@@ -527,6 +551,8 @@ def run_ours(args):
             line["sustained"] = sustained
         if cb is not None:
             line["cpu_baseline"] = cb
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -576,6 +602,8 @@ def run_infer_sweep(args):
                           "tensor_frac_burst": ips * conf["fwd_gf"] / 1e3 / pk["tflops_burst"], "finite": bool(torch.isfinite(out).all())})
             del xs
     clocks = sampler.stop()
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"logits": out})      # the last timed forward, at the last batch size
     best = max(sweep, key=lambda r: r["images_per_s"])
     line = {"metric": conf["metric"], "value": best["images_per_s"], "unit": UNIT, "n_gpus": 1, "steps": args.steps, "warmup": max(args.warmup, 3),
             "ms_per_step": best["ms_per_forward"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "bf16",
@@ -603,15 +631,24 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch (default: the config's — 16 for ViT-B, 8 for ViT-L)")
     ap.add_argument("--batch-sweep", type=lambda v: [int(x) for x in v.split(",")], default=[1, 2, 4, 8, 16, 32, 64, 128, 256, 512],
                     help="vitb224-infer: batch sizes")
-    ap.add_argument("--sustained-seconds", type=float, default=3.0,
-                    help="after the K timed steps, keep stepping for this long and report it as `sustained` (0 = skip)")
+    ap.add_argument("--sustained-seconds", type=float, default=0.0,
+                    help="after the K timed steps, keep stepping for this long and report it as `sustained` (default 0: skip, "
+                         "so that --steps is the number of timed training steps)")
     ap.add_argument("--graph", action="store_true", help="replay the step from a captured CUDA graph (chest_x_ray_vit_b200.graph)")
     ap.add_argument("--layers-per-bucket", type=lambda v: [int(x) for x in v.split(",")], default=[3, 3, 3, 2, 1], help="encoder layers per all-reduce bucket, in the order layers finish backward; last entry repeats (3 layers = 85 MB; tapered so the all-reduce left after backward is short)")
     ap.add_argument("--sync", default="auto", choices=["auto", "peer", "nccl"],
                     help="gradient all-reduce at N>1: copy engines over NVLink peer memory (PeerGradSync) or NCCL (GradSync); auto = "
                          "peer up to 4 GPUs (measured 0.973 vs 0.953 at N=2), NCCL at 8 (0.912 vs 0.905)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32): loss, logits and a fixed "
+                         "seeded sample of the updated parameters (training), logits (vitb224-infer); inputs are seeded, "
+                         "so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

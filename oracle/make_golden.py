@@ -5,8 +5,10 @@ constructs) in fp32 on the CPU, on weights produced by ``oracle.vit_oracle.init_
 (deterministic CPU generator, so the weights themselves need not be committed), and
 writes small fixtures under tests/golden/:
 
-  tiny_b3.pt .......... TINY config, batch 3: inputs, logits, loss, ALL gradients,
-                        post-AdamW-step parameters
+  tiny_b3.pt .......... TINY config, batch 3: inputs, logits, loss, per-parameter gradient
+                        norms, and every element (tensors of at most TINY_SAMPLE elements) or
+                        TINY_SAMPLE distinct sampled elements of each gradient and of each
+                        post-AdamW-step parameter
   vitb16_384_b2.pt .... BASELINE.json configs[0] (ViT-B/16@384, batch 2): inputs,
                         logits, loss, per-parameter gradient norms and 64 sampled
                         gradient entries per parameter, same for post-step params
@@ -42,9 +44,26 @@ def hf_model(cfg: O.OracleConfig, params):
     return m, transformers.__version__
 
 
+TINY_SAMPLE = 2048       # keeps tiny_b3.pt far below 1 MB (all gradients and post-step parameters would be 2.9 MB)
+
+
 def sample_indices(name: str, numel: int, n: int = 64) -> torch.Tensor:
     g = torch.Generator().manual_seed(abs(hash_name(name)) % (2 ** 31))
     return torch.randint(0, numel, (min(n, numel),), generator=g)
+
+
+def kept_indices(name: str, numel: int, n: int) -> torch.Tensor:
+    """All elements of a tensor of at most ``n``, else ``n`` distinct ones drawn with a per-name seed (sorted)."""
+    if numel <= n:
+        return torch.arange(numel)
+    g = torch.Generator().manual_seed(abs(hash_name(name)) % (2 ** 31))
+    return torch.randperm(numel, generator=g)[:n].sort().values
+
+
+def record_indices(rec: dict, name: str, numel: int) -> torch.Tensor:
+    """Flat indices of parameter ``name`` that the ``grad_sample`` / ``post_sample`` entries of ``rec`` hold."""
+    n = rec.get("n_sample")
+    return sample_indices(name, numel) if n is None else kept_indices(name, numel, n)
 
 
 def hash_name(name: str) -> int:
@@ -54,7 +73,8 @@ def hash_name(name: str) -> int:
     return h
 
 
-def run(cfg: O.OracleConfig, batch: int, full: bool, step: bool = True):
+def run(cfg: O.OracleConfig, batch: int, n_sample=None, step: bool = True):
+    """``n_sample`` None: 64 elements per tensor drawn with replacement (sample_indices); else kept_indices(n_sample)."""
     torch.manual_seed(0)
     params = O.init_params(cfg, seed=0, perturb_seed=123)
     g = torch.Generator().manual_seed(1)
@@ -71,24 +91,21 @@ def run(cfg: O.OracleConfig, batch: int, full: bool, step: bool = True):
         opt = torch.optim.AdamW(m.parameters(), lr=2e-5, betas=(0.9, 0.999), eps=1e-8, weight_decay=0.0)
         opt.step()
         post = {k: v.detach().clone() for k, v in m.named_parameters()}
-    if full:
-        rec["grads"] = grads
-        if step:
-            rec["post"] = post
-    else:
-        rec["grad_norm"] = {k: v.norm().item() for k, v in grads.items()}
-        rec["grad_sample"] = {k: v.flatten()[sample_indices(k, v.numel())].clone() for k, v in grads.items()}
-        if step:
-            rec["post_sample"] = {k: v.flatten()[sample_indices(k, v.numel())].clone() for k, v in post.items()}
+    if n_sample is not None:
+        rec["n_sample"] = n_sample
+    rec["grad_norm"] = {k: v.norm().item() for k, v in grads.items()}
+    rec["grad_sample"] = {k: v.flatten()[record_indices(rec, k, v.numel())].clone() for k, v in grads.items()}
+    if step:
+        rec["post_sample"] = {k: v.flatten()[record_indices(rec, k, v.numel())].clone() for k, v in post.items()}
     return rec
 
 
 def main():
     os.makedirs(OUT, exist_ok=True)
     torch.set_num_threads(os.cpu_count() or 1)
-    torch.save(run(O.TINY, 3, full=True), os.path.join(OUT, "tiny_b3.pt"))
-    torch.save(run(O.VIT_B16_384, 2, full=False), os.path.join(OUT, "vitb16_384_b2.pt"))
-    r = run(O.VIT_B16_224, 2, full=False, step=False)
+    torch.save(run(O.TINY, 3, n_sample=TINY_SAMPLE), os.path.join(OUT, "tiny_b3.pt"))
+    torch.save(run(O.VIT_B16_384, 2), os.path.join(OUT, "vitb16_384_b2.pt"))
+    r = run(O.VIT_B16_224, 2, step=False)
     r = {k: r[k] for k in ("hf_version", "torch_version", "batch", "cfg", "x8", "y", "logits", "loss")}
     torch.save(r, os.path.join(OUT, "vitb16_224_b2.pt"))
     for f in sorted(os.listdir(OUT)):

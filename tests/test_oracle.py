@@ -31,17 +31,20 @@ def test_tiny_full_gradients_match_hf_golden():
     loss, logits, grads = O.forward_backward(p, cfg, x, rec["y"])
     assert torch.allclose(logits, rec["logits"], atol=2e-5, rtol=0)
     assert abs(loss.item() - rec["loss"].item()) <= 1e-6 * abs(rec["loss"].item()) + 1e-7
-    for k, g in rec["grads"].items():
+    from oracle.make_golden import record_indices
+    for k, g in rec["grad_sample"].items():
         if k.endswith("key.bias"):        # analytically zero (SURVEY App. C.6)
             assert grads[k].norm() < 1e-6
             continue
-        assert torch.allclose(grads[k], g, atol=2e-6, rtol=1e-3), k
+        nrm = rec["grad_norm"][k]
+        assert abs(grads[k].norm().item() - nrm) <= 1e-3 * nrm + 2e-6, k
+        assert torch.allclose(grads[k].flatten()[record_indices(rec, k, grads[k].numel())], g, atol=2e-6, rtol=1e-3), k
     st = {}
     O.adamw_step(p, grads, st)
-    for k, v in rec["post"].items():
+    for k, v in rec["post_sample"].items():
         if k.endswith("key.bias"):
             continue   # Adam normalises rounding noise of a zero gradient
-        assert torch.allclose(p[k], v, atol=2e-5 * 1.01, rtol=0), k
+        assert torch.allclose(p[k].flatten()[record_indices(rec, k, p[k].numel())], v, atol=2e-5 * 1.01, rtol=0), k
 
 
 def test_vitb16_384_matches_hf_golden():
