@@ -5,12 +5,15 @@
 // Replaces HF modeling_vit.py:455,641-646 + loss_utils.py:110-112.
 #include <cuda_bf16.h>
 
+#include <mutex>
+
 #include "common.cuh"
 
 namespace vitk {
 
 constexpr int kHeadThreads = 256;
 constexpr int kMaxLabels = 64;
+constexpr int kMaxHidden = 8192;   // head_bwd keeps two fp32 rows of D in shared memory: 64 KB at this limit
 
 __device__ __forceinline__ float block_sum(float v, float* scratch) {
 #pragma unroll
@@ -128,7 +131,7 @@ extern "C" VITK_API int vitk_head_fwd(const float* h, int64_t B, int64_t T, int6
                                       const float* labels, float* logits, float* loss, float* dlogits, float* mean,
                                       float* rstd, vitk_stream_t stream) {
   VITK_REQUIRE(h && gamma && beta && Wc && bc && logits, VITK_EINVAL, "head_fwd: NULL argument");
-  VITK_REQUIRE(B > 0 && T > 0 && D > 0 && C > 0 && C <= kMaxLabels && D <= 8192, VITK_EINVAL,
+  VITK_REQUIRE(B > 0 && T > 0 && D > 0 && C > 0 && C <= kMaxLabels && D <= kMaxHidden, VITK_EINVAL,
                "head_fwd: unsupported shape B=%lld T=%lld D=%lld C=%lld", (long long)B, (long long)T, (long long)D,
                (long long)C);
   if (labels) VITK_REQUIRE(loss != nullptr, VITK_EINVAL, "head_fwd: labels given but loss is NULL");
@@ -146,9 +149,17 @@ extern "C" VITK_API int vitk_head_bwd(const float* h, const float* mean, const f
                                       float* dgamma, float* dbeta, vitk_stream_t stream) {
   VITK_REQUIRE(h && mean && rstd && gamma && beta && Wc && dlogits && dh && dWc && dbc && dgamma && dbeta, VITK_EINVAL,
                "head_bwd: NULL argument");
-  VITK_REQUIRE(B > 0 && T > 0 && D > 0 && C > 0 && C <= kMaxLabels && D <= 8192, VITK_EINVAL,
+  VITK_REQUIRE(B > 0 && T > 0 && D > 0 && C > 0 && C <= kMaxLabels && D <= kMaxHidden, VITK_EINVAL,
                "head_bwd: unsupported shape B=%lld T=%lld D=%lld C=%lld", (long long)B, (long long)T, (long long)D,
                (long long)C);
+  // above 48 KB of dynamic shared memory (D > 6144) a launch needs the kernel's opt-in
+  static std::once_flag once;
+  static cudaError_t attr_err = cudaSuccess;
+  std::call_once(once, [] {
+    attr_err = cudaFuncSetAttribute(head_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    2 * kMaxHidden * static_cast<int>(sizeof(float)));
+  });
+  if (attr_err != cudaSuccess) return cuda_error(attr_err, "cudaFuncSetAttribute(head_bwd smem)");
   head_bwd_kernel<<<static_cast<unsigned>(B), kHeadThreads, 2 * D * sizeof(float), static_cast<cudaStream_t>(stream)>>>(
       h, mean, rstd, gamma, beta, Wc, (int)B, (int)T, (int)D, (int)C, dlogits, dloss, static_cast<__nv_bfloat16*>(dh),
       dWc, dbc, dgamma, dbeta);
@@ -163,6 +174,8 @@ extern "C" VITK_API int vitk_head_bwd(const float* h, const float* mean, const f
 // so no logits travel to the host.  sigmoid is evaluated in fp32 as 1/(1+exp(−x)) like ATen's, so the threshold
 // comparison sees the same rounding (logits a few ulp below 0 still round to exactly 0.5 and count as positive).
 namespace vitk {
+constexpr int kMaxCountLabels = 4096;   // [C][4] uint32 counters in shared memory: 64 KB at this limit
+
 __global__ void __launch_bounds__(256)
 multilabel_counts_kernel(const float* __restrict__ logits, const float* __restrict__ labels, long long n, int C, float threshold,
                          unsigned long long* __restrict__ counts) {
@@ -184,8 +197,17 @@ multilabel_counts_kernel(const float* __restrict__ logits, const float* __restri
 
 extern "C" VITK_API int vitk_multilabel_counts(const float* logits, const float* labels, int64_t B, int64_t C, float threshold,
                                                int64_t* counts, vitk_stream_t stream) {
-  VITK_REQUIRE(logits && labels && counts && B > 0 && C > 0 && C <= 4096, VITK_EINVAL, "multilabel_counts: bad argument");
+  VITK_REQUIRE(logits && labels && counts && B > 0 && C > 0 && C <= vitk::kMaxCountLabels, VITK_EINVAL,
+               "multilabel_counts: bad argument");
   VITK_REQUIRE(threshold > 0.f && threshold < 1.f, VITK_EINVAL, "multilabel_counts: threshold must be in (0, 1)");
+  // above 48 KB of dynamic shared memory (C > 3072) a launch needs the kernel's opt-in
+  static std::once_flag once;
+  static cudaError_t attr_err = cudaSuccess;
+  std::call_once(once, [] {
+    attr_err = cudaFuncSetAttribute(vitk::multilabel_counts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    16 * vitk::kMaxCountLabels);
+  });
+  if (attr_err != cudaSuccess) return vitk::cuda_error(attr_err, "cudaFuncSetAttribute(multilabel_counts smem)");
   const long long n = B * C;
   long long blocks = (n + 255) / 256;
   if (blocks > 4LL * vitk::num_sms()) blocks = 4LL * vitk::num_sms();

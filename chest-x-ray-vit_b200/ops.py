@@ -83,30 +83,53 @@ def patchify_f32(pix: torch.Tensor, out: Optional[torch.Tensor] = None):
 
 
 # ----------------------------------------------------------------------------- LayerNorm
+def _check_rows(what: str, t: torch.Tensor, M: int, row_stride: int, width: int) -> None:
+    # logical row r of a row_stride buffer is physical row r·row_stride of a contiguous [·, width] tensor
+    assert t.is_contiguous() and t.numel() >= ((M - 1) * row_stride + 1) * width, \
+        f"{what}: needs a contiguous buffer of at least {(M - 1) * row_stride + 1} rows of {width}"
+
+
 def layernorm_fwd(x: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float,
                   y: Optional[torch.Tensor] = None, mean: Optional[torch.Tensor] = None,
-                  rstd: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+                  rstd: Optional[torch.Tensor] = None, *, row_stride: int = 1) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """LayerNorm of the M rows of ``x`` (fp32, own row stride) into y (bf16) and mean / rstd (fp32).  With
+    ``row_stride`` > 1, logical row r goes to physical row r·row_stride of y / mean / rstd — the CLS rows of a
+    [B, T, D] buffer stay in place with row_stride = T — and the caller passes all three, sized for the physical rows."""
     M, D = x.shape
     assert x.dtype == f32 and x.stride(1) == 1
+    if row_stride != 1:
+        assert y is not None and mean is not None and rstd is not None, "layernorm_fwd: row_stride > 1 needs y, mean and rstd"
+        _check_rows("layernorm_fwd y", y, M, row_stride, D)
+        _check_rows("layernorm_fwd mean", mean, M, row_stride, 1)
+        _check_rows("layernorm_fwd rstd", rstd, M, row_stride, 1)
     if y is None:
         y = torch.empty((M, D), dtype=bf16, device=x.device)
     if mean is None:
         mean = torch.empty((M,), dtype=f32, device=x.device)
     if rstd is None:
         rstd = torch.empty((M,), dtype=f32, device=x.device)
-    _lib.check(_lib.lib().vitk_layernorm_fwd(x.data_ptr(), x.stride(0), gamma.data_ptr(), beta.data_ptr(), eps, M, D,
-                                              y.data_ptr(), mean.data_ptr(), rstd.data_ptr(), _stream()), "layernorm_fwd")
+    _lib.check(_lib.lib().vitk_layernorm_fwd_rows(x.data_ptr(), x.stride(0), gamma.data_ptr(), beta.data_ptr(), eps, M, D,
+                                                   row_stride, y.data_ptr(), mean.data_ptr(), rstd.data_ptr(), _stream()),
+               "layernorm_fwd")
     return y, mean, rstd
 
 
-def layernorm_bwd(dy, x, mean, rstd, gamma, dres, dgamma, dbeta, dx=None, dxsum=None):
-    """dx = dres + LNbwd(dy) (bf16); dgamma/dbeta (fp32) are accumulated; dxsum (optional) += Σ_rows dx."""
+def layernorm_bwd(dy, x, mean, rstd, gamma, dres, dgamma, dbeta, dx=None, dxsum=None, *, row_stride: int = 1):
+    """dx = dres + LNbwd(dy) (bf16); dgamma/dbeta (fp32) are accumulated; dxsum (optional) += Σ_rows dx.
+    With ``row_stride`` > 1, logical row r of dy / dres / dx / mean / rstd is physical row r·row_stride (x keeps its
+    own row stride), and the caller passes ``dx`` sized for the physical rows."""
     M, D = x.shape
+    if row_stride != 1:
+        assert dx is not None, "layernorm_bwd: row_stride > 1 needs dx"
+        for what, t, width in (("dy", dy, D), ("dres", dres, D), ("dx", dx, D), ("mean", mean, 1), ("rstd", rstd, 1)):
+            if t is not None:
+                _check_rows(f"layernorm_bwd {what}", t, M, row_stride, width)
     if dx is None:
         dx = torch.empty((M, D), dtype=bf16, device=x.device)
-    _lib.check(_lib.lib().vitk_layernorm_bwd(dy.data_ptr(), x.data_ptr(), x.stride(0), mean.data_ptr(), rstd.data_ptr(),
-                                              gamma.data_ptr(), _ptr(dres), M, D, dx.data_ptr(), dgamma.data_ptr(),
-                                              dbeta.data_ptr(), _ptr(dxsum), _stream()), "layernorm_bwd")
+    _lib.check(_lib.lib().vitk_layernorm_bwd_rows(dy.data_ptr(), x.data_ptr(), x.stride(0), mean.data_ptr(), rstd.data_ptr(),
+                                                   gamma.data_ptr(), _ptr(dres), M, D, row_stride, dx.data_ptr(),
+                                                   dgamma.data_ptr(), dbeta.data_ptr(), _ptr(dxsum), _stream()),
+               "layernorm_bwd")
     return dx
 
 

@@ -163,7 +163,7 @@ VITK_API int vitk_embed_bwd(const void* dh_bf16, int64_t B, int64_t T, int64_t D
  * vitk_head_fwd:  h f32 [B,T,D] (only rows t=0 are read) → logits f32 [B,C]; when labels f32
  *   [B,C] != NULL also loss f32 [1] (mean over B·C) and, when dlogits != NULL, the fused loss
  *   gradient dlogits f32 [B,C] = (σ(logit) − y)/(B·C).  mean/rstd f32 [B] (optional) are the
- *   LayerNorm statistics the backward reuses. */
+ *   LayerNorm statistics the backward reuses.  Both head entry points take C <= 64 and D <= 8192. */
 VITK_API int vitk_head_fwd(const float* h, int64_t B, int64_t T, int64_t D, int64_t C, const float* gamma,
                   const float* beta, float eps, const float* Wc, const float* bc, const float* labels, float* logits,
                   float* loss, float* dlogits, float* mean, float* rstd, vitk_stream_t stream);
@@ -189,7 +189,7 @@ VITK_API int vitk_attn_cls_bwd(const void* qkv_bf16, const void* o_bf16, const v
  * Replaces compute_metrics / the final report of /root/reference/ViT-Training.py:112-118,139-146
  * (sigmoid → >= threshold → sklearn f1_score(average="micro") / classification_report): accumulates, per class c,
  * counts[c][0..3] += {TP, FP, FN, TN} over B×C fp32 logits and {0,1} fp32 labels.  counts: int64 [C,4], caller-zeroed
- * before the first batch of an evaluation loop; sigmoid = 1/(1+exp(−x)) in fp32 as in ATen. */
+ * before the first batch of an evaluation loop; sigmoid = 1/(1+exp(−x)) in fp32 as in ATen.  C <= 4096. */
 VITK_API int vitk_multilabel_counts(const float* logits, const float* labels, int64_t B, int64_t C, float threshold,
                int64_t* counts, vitk_stream_t stream);
 

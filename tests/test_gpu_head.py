@@ -12,7 +12,8 @@ def ops():
     return pkg.ops
 
 
-@pytest.mark.parametrize("B,T,D,C", [(2, 5, 768, 14), (16, 577, 768, 14), (3, 2, 1024, 15), (1, 1, 128, 1)])
+@pytest.mark.parametrize("B,T,D,C", [(2, 5, 768, 14), (16, 577, 768, 14), (3, 2, 1024, 15), (1, 1, 128, 1),
+                                     (2, 3, 8192, 64)])     # the largest D and C the kernels accept
 def test_head_fwd_bwd(ops, B, T, D, C):
     g = torch.Generator().manual_seed(B + C)
     h = torch.randn(B, T, D, generator=g).to(dev)

@@ -35,7 +35,7 @@ def test_patchify_f32_bit_exact(ops, B, S):
     assert torch.equal(got.cpu().view(torch.int16), ref.view(torch.int16))
 
 
-@pytest.mark.parametrize("M,D", [(1, 768), (13, 768), (1154, 768), (9232, 768), (65, 128), (300, 1024)])
+@pytest.mark.parametrize("M,D", [(1, 768), (13, 768), (1154, 768), (9232, 768), (65, 128), (300, 1024), (300, 256), (77, 512)])
 def test_layernorm_fwd_bwd(ops, M, D):
     g = torch.Generator().manual_seed(M + D)
     x = (torch.randn(M, D, generator=g) * 1.7 + 0.3).to(dev)
@@ -77,10 +77,18 @@ def test_layernorm_strided_rows(ops):
     assert (y.float() - ref).abs().max() < 0.02
 
 
-@pytest.mark.parametrize("M,N", [(1, 8), (577, 768), (9232, 2304), (1000, 3072), (50, 264)])
-def test_colsum(ops, M, N):
+@pytest.mark.parametrize("M,N,row_stride", [pytest.param(M, N, 1, id=f"{M}-{N}") for M, N in
+                                              [(1, 8), (577, 768), (9232, 2304), (1000, 3072), (50, 264)]] +
+                         [(16, 768, 577), (3, 3072, 197), (1, 1024, 577)])
+def test_colsum(ops, M, N, row_stride):
+    """row_stride > 1: x is every row_stride-th row of a larger buffer whose other rows are NaN (the bias gradients
+    of the top layer sum the B CLS rows of a [B·T, N] buffer, ldx = T·N)."""
     g = torch.Generator().manual_seed(M)
     x = torch.randn(M, N, generator=g).to(dev).to(torch.bfloat16)
+    if row_stride > 1:
+        buf = torch.full((M * row_stride, N), float("nan"), device=dev, dtype=torch.bfloat16)
+        buf[::row_stride] = x
+        x = buf.view(M, row_stride * N)[:, :N]
     out = torch.ones(N, device=dev)
     ops.colsum(x, out)
     ref = 1 + x.double().sum(0)

@@ -64,3 +64,15 @@ def test_device_counter_matches_sklearn_over_batches():
     _check_against_sklearn(scores, y_true, y_pred)
     ctr.reset()
     assert ctr.compute()["f1_micro"] == 0.0
+
+
+@pytest.mark.gpu
+def test_device_counter_at_the_label_limit():
+    """C = 4096, the most labels the counter kernel accepts: its [C][4] shared-memory counters take 64 KB."""
+    g = torch.Generator().manual_seed(2)
+    B, C = 3, 4096
+    logits = torch.randn(B, C, generator=g) * 2
+    y = (torch.rand(B, C, generator=g) < 0.3).float()
+    counts = torch.zeros((C, 4), dtype=torch.int64, device="cuda")
+    pkg.ops.multilabel_counts(logits.cuda(), y.cuda(), counts)
+    assert torch.equal(counts.cpu(), _counts(y.int().numpy(), _reference_predictions(logits)))
