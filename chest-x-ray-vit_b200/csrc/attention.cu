@@ -22,17 +22,12 @@
 #include "common.cuh"
 #include "sm100_prims.cuh"
 #include "tmap.cuh"
-#include <stdlib.h>
 
 namespace vitk {
 
 // Optional per-phase timeline (vitk_debug_timeline): CTA (0,0,0) records clock64() stamps.
 long long* g_timeline = nullptr;   // also stamped by the CTA-pair GEMM (gemm2.cu)
 int g_timeline_seq = 0;            // GEMM launches since the buffer was set (per-launch min/max stamps)
-#define VITK_FSTAMP(slot)                                            \
-  do {                                                               \
-    if (tl != nullptr && blockIdx.x == 0 && lane == 0) tl[6000 + (slot)] = clock64(); \
-  } while (0)
 #define VITK_STAMP(slot)                                             \
   do {                                                               \
     if (tl != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && lane == 0) tl[(slot)] = clock64(); \
@@ -367,7 +362,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_constant
 // ============================================================================ backward
 // stats[b,h,t] = { lse·log2e, Δ = Σ_d dO·O } for t < T and { +inf, 0 } for the padding rows T ≤ t < Tpad
 // (Tpad = multiple of 128), so the main kernel reads them with unconditional aligned float4 loads and
-// padded queries get P = exp2(−inf) = 0.  One warp per token row.
+// padded queries get P = exp2(−inf) = 0.  One warp per token row; used for H > 16 heads.
 __global__ void __launch_bounds__(256) attn_delta_kernel(const __nv_bfloat16* __restrict__ o,
                                                          const __nv_bfloat16* __restrict__ d_o, const float* __restrict__ lse,
                                                          int B, int T, int Tpad, int H, float* __restrict__ lse2,
@@ -506,8 +501,7 @@ __global__ void __launch_bounds__(256) attn_delta16_kernel(const __nv_bfloat16* 
 // allocation, barrier set-up, the K/V + Q/dO round trip) behind the epilogue: 123.9 → 117.5 µs per layer all-in at
 // B = 16.  (Tried on top and dropped, 119.7 µs: K/V double-buffered in shared memory with the next item's scores queued
 // right behind the last dQ MMA — the boundary was already hidden behind the compute warps' epilogue, and the variable
-// K/V descriptor offsets cost the MMA-issue warp ≈100 cycles per sub-block.)  VITK_ATTN_BWD_PERSIST=0 launches one
-// CTA per item (the same code, one trip).
+// K/V descriptor offsets cost the MMA-issue warp ≈100 cycles per sub-block.)
 constexpr int kBwdComputeWarps = 16;
 constexpr int kBwdThreads = (kBwdComputeWarps + 2) * 32;   // 16 compute warps + MMA-issue warp + TMA-load warp
 constexpr int kQSub = 64;
@@ -895,13 +889,6 @@ __global__ void debug_stamp_kernel(long long* dst) {
 }
 extern "C" VITK_API int vitk_debug_stamp(int64_t slot, void* stream) {
   VITK_REQUIRE(g_timeline != nullptr && slot >= 0, VITK_EINVAL, "vitk_debug_stamp: no timeline buffer set");
-  static const int carve = [] {     // experiment: VITK_STAMP_CARVEOUT=100 keeps the SM in its max-shared-memory configuration
-    const char* e = getenv("VITK_STAMP_CARVEOUT");
-    const int c = e ? atoi(e) : -1;
-    if (c >= 0) cudaFuncSetAttribute(debug_stamp_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, c);
-    return c;
-  }();
-  (void)carve;
   debug_stamp_kernel<<<1, 1, 0, static_cast<cudaStream_t>(stream)>>>(g_timeline + slot);
   VITK_LAUNCH_CHECK("debug_stamp_kernel");
   return 0;
@@ -955,8 +942,7 @@ extern "C" VITK_API int vitk_attn_bwd(const void* qkv, const void* o, const void
     const __nv_bfloat16* po = static_cast<const __nv_bfloat16*>(o);
     const __nv_bfloat16* pdo = static_cast<const __nv_bfloat16*>(d_o);
     const dim3 g16(static_cast<unsigned>(B * Tpad / 16)), g8((static_cast<int>(B) * Tpad + 7) / 8);
-    static const bool legacy = [] { const char* e = getenv("VITK_ATTN_DELTA_LEGACY"); return e && atoi(e) != 0; }();
-    if (H > 16 || legacy) VITK_CUDA(launch_pdl(attn_delta_kernel, g8, dim3(256), 0, s, po, pdo, lse, (int)B, (int)T, Tpad, (int)H, lse2, delta));
+    if (H > 16) VITK_CUDA(launch_pdl(attn_delta_kernel, g8, dim3(256), 0, s, po, pdo, lse, (int)B, (int)T, Tpad, (int)H, lse2, delta));
     else if (H > 12) VITK_CUDA(launch_pdl(attn_delta16_kernel<4>, g16, dim3(256), 0, s, po, pdo, lse, (int)B, (int)T, Tpad, (int)H, lse2, delta));
     else if (H > 8) VITK_CUDA(launch_pdl(attn_delta16_kernel<3>, g16, dim3(256), 0, s, po, pdo, lse, (int)B, (int)T, Tpad, (int)H, lse2, delta));
     else if (H > 4) VITK_CUDA(launch_pdl(attn_delta16_kernel<2>, g16, dim3(256), 0, s, po, pdo, lse, (int)B, (int)T, Tpad, (int)H, lse2, delta));
@@ -965,8 +951,7 @@ extern "C" VITK_API int vitk_attn_bwd(const void* qkv, const void* o, const void
   VITK_LAUNCH_CHECK("attn_delta_kernel");
   const long long items = ((T + kTile - 1) / kTile) * H * B;
   VITK_REQUIRE(items < (1ll << 30), VITK_EINVAL, "attn_bwd: too many (key block, head, image) work items");
-  static const bool persist = [] { const char* e = getenv("VITK_ATTN_BWD_PERSIST"); return !e || atoi(e) != 0; }();
-  const long long ctas = persist && items > num_sms() ? num_sms() : items;
+  const long long ctas = items > num_sms() ? num_sms() : items;
   VITK_CUDA(launch_pdl(attn_bwd_kernel, dim3(static_cast<unsigned>(ctas)), dim3(kBwdThreads), kBwdSmemBytes, s, tm_qkv, tm_q64, tm_do, tm_dq,
                        static_cast<const float*>(lse2), static_cast<const float*>(delta), static_cast<__nv_bfloat16*>(dqkv), (int)T, Tpad,
                        (int)H, (int)B, scale, scale * kLog2e, work_counter, g_timeline));

@@ -1,6 +1,5 @@
 // Error reporting, device checks and library identity for libvitk.
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
@@ -26,11 +25,6 @@ int cuda_error(cudaError_t e, const char* what) {
 
 static std::atomic<long long> g_launches{0};
 void count_launch() { g_launches.fetch_add(1, std::memory_order_relaxed); }
-
-bool pdl_enabled() {
-  static const bool on = [] { const char* e = getenv("VITK_PDL"); return !(e && e[0] == '0'); }();
-  return on;
-}
 
 int num_sms() {
   static thread_local int cached_dev = -1;

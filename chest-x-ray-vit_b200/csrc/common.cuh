@@ -39,12 +39,11 @@ inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 // run their prologue: barrier init, TMEM allocation, descriptor prefetch) while the previous kernel in the
 // stream is still draining its last wave, and they block in pdl_wait() before touching global memory until
 // that kernel has completed and flushed.  ~300 dependent launches per step, each with a 3–4 µs
-// launch + prologue + tail bubble otherwise.  VITK_PDL=0 disables it.
+// launch + prologue + tail bubble otherwise.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 #endif
-bool pdl_enabled();
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, Args... args) {
@@ -57,7 +56,7 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 

@@ -27,10 +27,9 @@
 //   instantiations  <BN, A_MN, B_MN, AUX, EW, EPI>: AUX = epilogues that read a second matrix.  Separate because the
 //                 epilogue lives at the 168-register cap (10 warps → 3 per SM sub-partition); EW = 16 with a compile-time
 //                 epilogue EPI lives at 96 (18 warps → 5 on one sub-partition).
-// Diagnostics: VITK_GEMM_DBG ablation bits (Gemm2Params::dbg) and, in builds with -DVITK_GEMM_STAMPS=1, clock
-// stamps per K block / tile / CTA / launch (tools/gemm_timeline.py).
+// Diagnostics: in builds with -DVITK_GEMM_STAMPS=1, clock stamps per K block / tile / CTA / launch
+// (tools/gemm_timeline.py).
 #include <cuda.h>
-#include <stdlib.h>
 
 #include <mutex>
 
@@ -50,10 +49,9 @@ constexpr int k2FirstEpiWarp = 2;
 // that four warps per scheduler hide better than two.
 constexpr int threads2(int ew) { return (k2FirstEpiWarp + ew) * 32; }
 constexpr int k2ABytes = k2BM * k2BK * 2;                       // 16 KB
-#ifndef VITK_G2_SLABS
-#define VITK_G2_SLABS 2      // 2 and 4 measured equal (the epilogue is not waiting on its TMA stores)
-#endif
-constexpr int k2Slabs = VITK_G2_SLABS;                          // [32 rows × 64 B] slabs per epilogue warp (TMA stores in flight)
+// [32 rows × 64 B] slabs per epilogue warp (TMA stores in flight): 2 and 4 measured equal (the epilogue is not waiting
+// on its TMA stores)
+constexpr int k2Slabs = 2;
 constexpr int k2SlabBytes = k2Slabs * 2048;
 constexpr int staging_bytes2(int ew) { return ew * k2SlabBytes; }  // 32 KB (8 warps) / 64 KB (16 warps)
 constexpr int k2MaxSmem = 227 * 1024;
@@ -68,11 +66,9 @@ struct Cfg2 {
   // Operand bytes in flight are what hides the ≈3,200-cycle refill round trip (MMA retire → commit →
   // producer wake → TMA → L2 → complete_tx on the leader → MMA wake): measured k-block cadence ≈
   // (512 + 3200) / stages cycles, so every stage that fits in the 227 KB is used.
-#ifndef VITK_G2_STAGES
-#define VITK_G2_STAGES 6     // 4, 5 and 6 measured equal: the K-block cadence is a throughput limit, not a latency one
-#endif
+  // 4, 5 and 6 stages at BN = 256 / 192 measured equal: the K-block cadence is a throughput limit, not a latency one.
   static constexpr int kStagingBytes = staging_bytes2(EW);
-  static constexpr int kWantStages = (BN == 256) ? VITK_G2_STAGES : (BN == 192 ? VITK_G2_STAGES : VITK_G2_STAGES + 2);
+  static constexpr int kWantStages = (BN == 256 || BN == 192) ? 6 : 8;
   static constexpr int kFitStages = (k2MaxSmem - kStagingBytes - k2BiasBytes - k2BarBytes) / kStageBytes;
   static constexpr int kStages = kWantStages < kFitStages ? kWantStages : kFitStages;   // 16 epilogue warps: 5 stages at BN = 256 / 192
   static constexpr int kTmemCols = (2 * BN <= 256) ? 256 : 512;
@@ -86,14 +82,6 @@ struct Gemm2Params {
                        // (n_tiles = n_full + n_half); all full tiles come first in the work order
   int epi;
   int has_d2;
-  int l2_hints;       // VITK_L2_HINTS (default 1): the second output (GELU', saved for backward, not read again in this pass) is
-                      // stored with the L2 evict_first policy so that it does not push gelu(u) — the next GEMM's operand — out
-                      // of L2.  A/B on the step (profiles/r02_l2_hints_ab.txt): +0.5 %, at the edge of the run-to-run noise;
-                      // evict_first LOADS of the single-use multiplier / residual / LayerNorm-backward inputs changed nothing
-                      // and were removed.
-  int dbg;            // VITK_GEMM_DBG experiment bits (0 in production): 1 skip stores, 2 skip aux, 4 skip TMEM loads,
-                      // 8 every CTA loads tile (0,0) (operands always L2-resident), 16 no MMAs (load pipeline only),
-                      // 32 no TMA loads after the first ring fill (MMA pipeline only)
   const void* aux;
   long long ld_aux;
   const float* bias;
@@ -277,9 +265,9 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
     int kbi = 0;
     for (int w = pair_id; w < p.total_work; w += num_pairs) {
       const Work2 it = decode_work2<BN>(p, w);
-      const int m0 = (p.dbg & 8) ? 0 : it.m_blk * (2 * k2BM) + static_cast<int>(cta_rank) * k2BM;
+      const int m0 = it.m_blk * (2 * k2BM) + static_cast<int>(cta_rank) * k2BM;
       const bool half = it.bn != BN;                  // half-width tile: this CTA stages BN/4 rows of B
-      const int n0 = (p.dbg & 8) ? 0 : it.n0 + static_cast<int>(cta_rank) * (it.bn >> 1);
+      const int n0 = it.n0 + static_cast<int>(cta_rank) * (it.bn >> 1);
       const uint32_t stage_tx = 2 * (k2ABytes + (half ? Cfg::kBBytes / 2 : Cfg::kBBytes));
       const int kb_begin = it.kb_begin, kb_end = it.kb_end;
       for (int kb = kb_begin; kb < kb_end; ++kb) {
@@ -289,10 +277,8 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
         uint8_t* sa = smem + stage * Cfg::kStageBytes;
         uint8_t* sb = sa + k2ABytes;
         const uint32_t bar = full0_leader + stage * 8;
-        const int k0 = (p.dbg & 8) ? (kb & 7) * k2BK : kb * k2BK;
-        if ((p.dbg & 32) && kbi > kStages) {       // experiment: MMAs re-read stale stages, no TMA traffic at all
-          if (L && leader) mbar_arrive(&full_bar[stage]);
-        } else if (elect_one()) {                  // elect.sync: ptxas issues the TMA instructions straight from uniform registers
+        const int k0 = kb * k2BK;
+        if (elect_one()) {                         // elect.sync: ptxas issues the TMA instructions straight from uniform registers
           if (leader) mbar_arrive_expect_tx(&full_bar[stage], stage_tx);
           if (!A_MN) {
             tma_load_2d_pair(sa, &tma_a, bar, k0, m0);
@@ -346,12 +332,10 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
           // elect/broadcast/retry loop whose latency (≈110 cycles per MMA, 670 per K block) — not the tensor pipe
           // (512) — paced the main loop, for N = 128 and N = 256 alike.
           if (elect_one()) {
-            if (!(p.dbg & 16)) {
 #pragma unroll
-              for (int k = 0; k < k2BK / 16; ++k)
-                tc_mma_bf16_pair(d_tmem, a_desc0 + soff + k * a_kstep, b_desc0 + soff + k * b_kstep, idesc,
-                                 (kb > kb_begin || k > 0) ? 1u : 0u);
-            }
+            for (int k = 0; k < k2BK / 16; ++k)
+              tc_mma_bf16_pair(d_tmem, a_desc0 + soff + k * a_kstep, b_desc0 + soff + k * b_kstep, idesc,
+                               (kb > kb_begin || k > 0) ? 1u : 0u);
             tc_commit_pair(&empty_bar[stage], 3);                         // both CTAs' producers may refill
             if (kb == kb_end - 1) tc_commit_pair(&acc_full[acc], 3);   // both CTAs' epilogues may drain
           }
@@ -387,7 +371,7 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
     float* bias_base = reinterpret_cast<float*>(staging + k2StagingBytes) + part * (2 * kBiasPart);   // [tile parity][kBiasPart], shared by the 4 warps of this column part
     const int epi = EPI >= 0 ? EPI : p.epi;
     const bool out_f32 = epi == VITK_EPI_BIAS_RESID_F32 || epi == VITK_EPI_ACCUM_F32 || epi == VITK_EPI_STORE_F32;
-    const bool has_aux = AUX && !(p.dbg & 2) && (epi == VITK_EPI_BIAS_RESID_F32 || epi == VITK_EPI_MUL_BF16 || epi == VITK_EPI_DGELU_BF16);
+    const bool has_aux = AUX && (epi == VITK_EPI_BIAS_RESID_F32 || epi == VITK_EPI_MUL_BF16 || epi == VITK_EPI_DGELU_BF16);
     const bool has_bias = p.bias != nullptr && (epi == VITK_EPI_BIAS_BF16 || epi == VITK_EPI_BIAS_GELU_BF16 ||
                                                 epi == VITK_EPI_BIAS_GELUG_BF16 || epi == VITK_EPI_BIAS_RESID_F32);
     const int cw = out_f32 ? 16 : 32;                      // chunk width in columns
@@ -403,7 +387,6 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
     auto tile_row0 = [&](const Work2& it) { return it.m_blk * (2 * k2BM) + static_cast<int>(cta_rank) * k2BM + quad * 32; };
     auto tile_col0 = [&](const Work2& it) { return it.n0 + part * (it.bn / kParts); };   // this warp's column part of the tile
 
-    const bool d2_stream = (p.l2_hints & 1) != 0;   // (the policy is created where it is used: 2 registers the epilogue does not have to spare)
     uint4 axA[4], axB[4];  // aux chunks in flight (coalesced layout); named, never indexed dynamically, so they stay in registers
     auto load_aux = [&](uint4 (&dst)[4], int row0, int col) {
       const uint8_t* base = reinterpret_cast<const uint8_t*>(p.aux) +
@@ -431,8 +414,9 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
       *col = tile_col0(nxt) + (c - nch) * cw;
       return true;
     };
+    // stream_out: store with the L2 evict_first policy (the policy is created here, where it is used: 2 registers the
+    // epilogue does not have to spare)
     auto emit = [&](const CUtensorMap* map, int col, int row0, const uint4 (&q)[4], bool stream_out = false) {
-      if (p.dbg & 1) return;
       // wait until the store issued `nout` stores ago has finished reading its slab, then reuse it
       if (elect_one()) { if (nout == k2Slabs) tma_store_wait_read<k2Slabs - 1>(); else tma_store_wait_read<k2Slabs - 2>(); }
       __syncwarp();
@@ -499,10 +483,7 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
       for (int c = 0; c < nchunks; ++c) {
         const int col = col0 + c * cw;
         uint32_t r[32];
-        if (p.dbg & 4) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) r[i] = 0;
-        } else if (out_f32) {
+        if (out_f32) {
           uint32_t r16[16];
           tmem_ld_32x16(t_row + c * 16, r16);
 #pragma unroll
@@ -585,7 +566,11 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
               qg[j] = make_uint4(wg[0], wg[1], wg[2], wg[3]);
             }
             emit(&tma_d, col, row0, q);
-            if (p.has_d2) emit(&tma_d2, col, row0, qg, d2_stream);
+            // GELU' is saved for backward and not read again in this pass: evict_first keeps it from pushing gelu(u),
+            // the next GEMM's operand, out of L2.  A/B on the step (profiles/r02_l2_hints_ab.txt): +0.5 %, at the edge
+            // of the run-to-run noise; evict_first LOADS of the single-use multiplier / residual / LayerNorm-backward
+            // inputs changed nothing and were removed.
+            if (p.has_d2) emit(&tma_d2, col, row0, qg, true);
             break;
           }
           case VITK_EPI_MUL_BF16:
@@ -723,10 +708,9 @@ static int dispatch_major2(const vitk_gemm_args& a, const Gemm2Params& p, int pa
 // output (tests/test_gpu_gemm.py::test_sixteen_warp_epilogues_equal_eight_warp).  The same treatment of the multiplier
 // and fp32-residual epilogues was measured and dropped: those launches move 128 / 71 MB for 43.6 / 10.9 GF and sit on
 // the HBM side of the roofline, not on the epilogue's instruction latency (no change at 49.2 / 28.7 / 47.1 µs).
-// VITK_GEMM_EW16=0 switches the instantiation off (A/B); variant 3 does the same per call.
+// Variant 3 keeps the 8-warp instantiation (the reference the 16-warp one is tested against).
 static bool launch_heavy2(const vitk_gemm_args& a, const Gemm2Params& p, int bn, int pairs, cudaStream_t s, int* rc) {
-  static const int on = [] { const char* e = getenv("VITK_GEMM_EW16"); return e ? atoi(e) : 1; }();
-  if (!on || a.variant == 3) return false;
+  if (a.variant == 3) return false;
   if (a.epilogue == VITK_EPI_BIAS_GELUG_BF16 && !a.a_mn_major && !a.b_mn_major && bn == 256) {
     *rc = launch_gemm2<256, false, false, false, 16, VITK_EPI_BIAS_GELUG_BF16>(a, p, pairs, s);
     return true;
@@ -735,11 +719,9 @@ static bool launch_heavy2(const vitk_gemm_args& a, const Gemm2Params& p, int bn,
 }
 
 // cycles a CTA pair spends per 64-wide K block of a tile of `bn` columns (tools/gemm_timeline.py, B200): the MMAs of a
-// 256-wide tile occupy the tensor pipe for 4 × 122 cycles; narrower tiles are bound by operand delivery instead
-#ifndef VITK_K192
-#define VITK_K192 440.0   // A/B on the full step: 440 (192-wide tiles for K-major N = 768) beats 500 (mixed 256+128 there) by 0.9 %
-#endif
-static double kblock_cycles(int bn) { return bn == 256 ? 500.0 : (bn == 192 ? VITK_K192 : 390.0); }
+// 256-wide tile occupy the tensor pipe for 4 × 122 cycles; narrower tiles are bound by operand delivery instead.
+// 192: A/B on the full step, 440 (192-wide tiles for K-major N = 768) beats 500 (mixed 256+128 there) by 0.9 %.
+static double kblock_cycles(int bn) { return bn == 256 ? 500.0 : (bn == 192 ? 440.0 : 390.0); }
 constexpr double kTileFixedCycles = 1500.0;   // accumulator hand-over + pipeline refill per tile
 
 static void choose_tiling2(const vitk_gemm_args& a, int pairs, int* bn_out, int* splits_out, int* n_half_out,
@@ -747,7 +729,6 @@ static void choose_tiling2(const vitk_gemm_args& a, int pairs, int* bn_out, int*
   const long long mt = (a.M + 2 * k2BM - 1) / (2 * k2BM);
   const long long kb_total = (a.K + k2BK - 1) / k2BK;
   double best = 1e30;
-  static const int mixed_allowed = [] { const char* e = getenv("VITK_GEMM_MIXED"); return e ? atoi(e) : 1; }();
   const int cands[3] = {256, 192, 128};
   for (int bn : cands) {
     if (a.N % bn) continue;
@@ -772,7 +753,7 @@ static void choose_tiling2(const vitk_gemm_args& a, int pairs, int* bn_out, int*
     // Mixed widths (BN = 256 only): replace some of each band's 256-column tiles by pairs of 128-column tiles so that
     // the static round-robin order gives every CTA pair the same amount of work (e.g. N = 768 on 74 pairs: 3 full
     // tiles per band = 1.5 waves of full tiles; 2 full + 2 half = one full and one half tile for every pair).
-    if (bn == 256 && splits == 1 && a.epilogue != VITK_EPI_ACCUM_F32 && a.tile_n == 0 && mixed_allowed) {
+    if (bn == 256 && splits == 1 && a.epilogue != VITK_EPI_ACCUM_F32 && a.tile_n == 0) {
       const int n_tiles256 = static_cast<int>(a.N / 256);
       const double cf = kb_total * kblock_cycles(256) + kTileFixedCycles, ch = kb_total * kblock_cycles(128) + kTileFixedCycles;
       for (int nh = 2; nh <= 2 * n_tiles256; nh += 2) {
@@ -848,12 +829,6 @@ int gemm2_try_launch(const vitk_gemm_args& a, cudaStream_t stream, bool* handled
   p.total_work = p.mn_tiles * p.k_splits;
   p.epi = a.epilogue;
   p.has_d2 = a.d2 != nullptr;
-  {
-    static const int dbg = [] { const char* e = getenv("VITK_GEMM_DBG"); return e ? atoi(e) : 0; }();
-    p.dbg = dbg;
-    static const int hints = [] { const char* e = getenv("VITK_L2_HINTS"); return e ? atoi(e) : 1; }();
-    p.l2_hints = hints;
-  }
   p.aux = a.aux;
   p.ld_aux = a.ld_aux;
   p.bias = a.bias;

@@ -167,14 +167,9 @@ __global__ void __launch_bounds__(256) layernorm_fwd_kernel(const float* __restr
 // rows with a grid stride; one smem reduction + one atomicAdd per column per block at the end.
 // rs: logical row r lives at physical row r·rs of dy / dres / dx / mean / rstd (x has its own ldx); rs = T walks
 // only the CLS rows of a [B,T,D] tensor.
-#ifndef VITK_LN_BWD_BLOCKS
-#define VITK_LN_BWD_BLOCKS 2      // resident blocks per SM the register budget is cut for (tools/build_variants.sh A/B)
-#endif
-#ifndef VITK_LN_BWD_PREFETCH
-#define VITK_LN_BWD_PREFETCH 1    // 1: the next row is loaded while this one is reduced (24 more registers); 0: rely on occupancy
-#endif
+constexpr int kLnBwdBlocks = 2;   // resident blocks per SM the register budget is cut for (3 or 4 spilled and were slower)
 template <int VPL>
-__global__ void __launch_bounds__(256, VITK_LN_BWD_BLOCKS) layernorm_bwd_kernel(const __nv_bfloat16* __restrict__ dy, const float* __restrict__ x,
+__global__ void __launch_bounds__(256, kLnBwdBlocks) layernorm_bwd_kernel(const __nv_bfloat16* __restrict__ dy, const float* __restrict__ x,
                                                                long long ldx, const float* __restrict__ mean,
                                                                const float* __restrict__ rstd, const float* __restrict__ gamma,
                                                                const __nv_bfloat16* __restrict__ dres, int M, long long rs,
@@ -198,7 +193,8 @@ __global__ void __launch_bounds__(256, VITK_LN_BWD_BLOCKS) layernorm_bwd_kernel(
     db[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     dsx[i] = make_float4(0.f, 0.f, 0.f, 0.f);
   }
-  // software pipeline: the next row's x / dy / dres are in flight while this row is reduced and written
+  // software pipeline: the next row's x / dy / dres are in flight while this row is reduced and written (24 more
+  // registers than loading each row when it is reached)
   const int row_step = gridDim.x * nslots;
   int row = blockIdx.x * nslots + slot;
   float4 xn[V];
@@ -214,17 +210,16 @@ __global__ void __launch_bounds__(256, VITK_LN_BWD_BLOCKS) layernorm_bwd_kernel(
       rn[i] = dres ? __ldg(reinterpret_cast<const uint2*>(dres + pr * D) + c0 + 32 * i) : make_uint2(0u, 0u);
     }
   };
-  if (VITK_LN_BWD_PREFETCH && row < M) fetch(row);
+  if (row < M) fetch(row);
   int parity = 0;
   for (; row < M; row += row_step, parity ^= 1) {
     const long long prow = static_cast<long long>(row) * rs;
     const float mu = __ldg(mean + prow), r = __ldg(rstd + prow);
-    if (!VITK_LN_BWD_PREFETCH) fetch(row);
     float4 xv[V];
     uint2 dw[V], rw_[V];
 #pragma unroll
     for (int i = 0; i < V; ++i) { xv[i] = xn[i]; dw[i] = dn[i]; rw_[i] = rn[i]; }
-    if (VITK_LN_BWD_PREFETCH && row + row_step < M) fetch(row + row_step);
+    if (row + row_step < M) fetch(row + row_step);
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
     for (int i = 0; i < V; ++i) {
@@ -382,7 +377,7 @@ static int ln_bwd_launch(const __nv_bfloat16* dy, const float* x, long long ldx,
                          float* dbeta, float* dxsum, cudaStream_t s) {
   const int warps = 8;
   const int slots = (VPL % 2 == 0) ? warps / 2 : warps;      // rows in flight per block (a warp pair per row)
-  int grid = num_sms() * VITK_LN_BWD_BLOCKS;
+  int grid = num_sms() * kLnBwdBlocks;
   const int need = (M + slots - 1) / slots;
   if (grid > need) grid = need;
   const size_t smem = static_cast<size_t>(slots) * VPL * 128 * sizeof(float);

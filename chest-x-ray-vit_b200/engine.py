@@ -19,71 +19,57 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
-from typing import Callable, Dict, List, Optional, Tuple
+from typing import Callable, Dict, List, Optional, Set, Tuple
 
 import torch
 
 from . import _lib, ops
 from ._lib import (EPI_ACCUM_F32, EPI_BIAS_BF16, EPI_BIAS_GELUG_BF16, EPI_BIAS_RESID_F32, EPI_MUL_BF16, EPI_PATCH_F32,
-                   EPI_STORE_BF16, GemmArgs)
+                   EPI_STORE_BF16)
 
 bf16, f32 = torch.bfloat16, torch.float32
-_PLAN_GRAPHS = os.environ.get("VITK_PLAN_GRAPHS", "1") != "0"
 
 
 class _Plan:
-    """A list of (cfunc, args) launches; ``run`` appends the stream and checks return codes."""
+    """A list of (cfunc, args) launches; ``run`` appends the stream and checks return codes.  Steps marked with
+    ``side(True)`` run on ``side_stream`` (on the main stream when it is None)."""
 
-    tail_stream: Optional[torch.cuda.Stream] = None    # optional second auxiliary stream (fork(2) / join(2)); unused by default
-
-    def __init__(self):
+    def __init__(self, side_stream: Optional[torch.cuda.Stream] = None):
         self.steps: List[Tuple[object, tuple, str]] = []
         self.gemm_flops: Dict[int, float] = {}      # step index → 2·M·N·K (bench.py's roofline leg)
-        self.step_stream: Dict[int, int] = {}       # step index → 1 (side stream: weight gradients) | 2 (tail stream)
-        self._segments = {}                         # (callbacks?, side stream?) → [(CUDAGraph | None, callback | None)]
+        self.side_stream = side_stream
+        self.side_steps: Set[int] = set()           # indices of the steps launched on the side stream
+        self._segments = {}                         # callbacks? → [(CUDAGraph | None, callback | None)]
         self._warm = set()
         self._keep = []      # keeps GemmArgs structs alive
-        self._side = 0
+        self._side = False
         self.sync_points: List[Tuple[torch.cuda.Event, Callable]] = []
 
     def side(self, on: bool):
-        """Steps added while on=True are launched on the engine's side stream (weight-gradient work that only the
-        optimizer consumes); fork()/join() order it against the main chain."""
-        self._side = 1 if on else 0
+        """Steps added while on=True are launched on the side stream (weight-gradient work that only the optimizer
+        consumes); fork()/join() order it against the main chain."""
+        self._side = on
 
-    def fork(self, which: int = 1):
-        self.steps.append((None, (which,), "fork"))  # stream `which` waits for everything enqueued on main so far
+    def fork(self):
+        self.steps.append((None, (), "fork"))  # the side stream waits for everything enqueued on main so far
 
-    def join(self, which: int = 1):
-        self.steps.append((None, (which,), "join"))  # main stream waits for everything enqueued on stream `which` so far
+    def join(self):
+        self.steps.append((None, (), "join"))  # the main stream waits for everything enqueued on the side stream so far
+
+    def _launch(self, fn, args: tuple, name: str):
+        if self._side:
+            self.side_steps.add(len(self.steps))
+        self.steps.append((fn, args, name))
 
     def add(self, name: str, *args):
-        if self._side:
-            self.step_stream[len(self.steps)] = self._side
-        self.steps.append((getattr(_lib.lib(), name), args, name))
+        self._launch(getattr(_lib.lib(), name), args, name)
 
-    def gemm(self, a, b, M, N, K, d, epilogue, a_mn=False, b_mn=False, d2=None, bias=None, aux=None, rows_in=0,
-             rows_out=0, row_off=0, ldd=None, ld_aux=None, split_k=0, tile_n=0, variant=0, max_ctas=0):
-        self._gemm_one(a, b, M, N, K, d, epilogue, a_mn, b_mn, d2, bias, aux, rows_in, rows_out, row_off, ldd, ld_aux, split_k,
-                       tile_n, variant, max_ctas)
-
-    def _gemm_one(self, a, b, M, N, K, d, epilogue, a_mn, b_mn, d2, bias, aux, rows_in, rows_out, row_off, ldd, ld_aux, split_k,
-                  tile_n, variant, max_ctas):
-        g = GemmArgs()
-        g.a, g.b, g.M, g.N, g.K = a.data_ptr(), b.data_ptr(), M, N, K
-        g.lda, g.ldb = a.stride(0), b.stride(0)
-        g.a_mn_major, g.b_mn_major, g.epilogue, g.split_k = int(a_mn), int(b_mn), epilogue, split_k
-        g.d, g.ldd = d.data_ptr(), (ldd if ldd is not None else d.stride(0))
-        g.d2 = None if d2 is None else d2.data_ptr()
-        g.bias = None if bias is None else bias.data_ptr()
-        g.aux = None if aux is None else aux.data_ptr()
-        g.ld_aux = (ld_aux if ld_aux is not None else (aux.stride(0) if aux is not None else 0))
-        g.rows_in, g.rows_out, g.row_off, g.tile_n, g.max_ctas, g.variant = rows_in, rows_out, row_off, tile_n, max_ctas, variant
+    def gemm(self, a, b, M, N, K, d, epilogue, **kw):
+        """One vitk_gemm_bf16 launch; keyword arguments as for ops.gemm_args."""
+        g = ops.gemm_args(a, b, M, N, K, d, epilogue=epilogue, **kw)
         self._keep.append(g)
         self.gemm_flops[len(self.steps)] = 2.0 * M * N * K
-        if self._side:
-            self.step_stream[len(self.steps)] = self._side
-        self.steps.append((_lib.lib().vitk_gemm_bf16, (C.byref(g),), "vitk_gemm_bf16"))
+        self._launch(_lib.lib().vitk_gemm_bf16, (C.byref(g),), "vitk_gemm_bf16")
 
     def call(self, fn: Callable[[], None]):
         self.steps.append((None, (fn,), "python"))
@@ -97,9 +83,9 @@ class _Plan:
         self.steps.append((None, (ev,), "record"))
         self.sync_points.append((ev, after))
 
-    def _run_range(self, lo: int, hi: int, stream: int, side_stream: Optional[torch.cuda.Stream], run_py: bool = True):
-        streams = {1: side_stream, 2: self.tail_stream}
-        handles = {k: (v.cuda_stream if v is not None else stream) for k, v in streams.items()}
+    def _run_range(self, lo: int, hi: int, stream: int, run_py: bool = True):
+        side = self.side_stream
+        side_handle = side.cuda_stream if side is not None else stream
         for i in range(lo, hi):
             fn, args, name = self.steps[i]
             if fn is None:
@@ -108,46 +94,42 @@ class _Plan:
                         args[0]()
                 elif name == "record":
                     args[0].record(torch.cuda.current_stream())
-                elif streams[args[0]] is not None:
-                    other = streams[args[0]]
+                elif side is not None:
                     main = torch.cuda.current_stream()
                     ev = torch.cuda.Event()
                     if name == "fork":
                         ev.record(main)
-                        other.wait_event(ev)
+                        side.wait_event(ev)
                     else:
-                        ev.record(other)
+                        ev.record(side)
                         main.wait_event(ev)
                 continue
-            which = self.step_stream.get(i, 0)
-            rc = fn(*args, handles[which] if which else stream)
+            rc = fn(*args, side_handle if i in self.side_steps else stream)
             if rc != 0:
                 _lib.check(rc, name)
 
-    def run(self, stream: int, side_stream: Optional[torch.cuda.Stream] = None, callbacks: bool = True):
+    def run(self, stream: int, callbacks: bool = True):
         """Enqueue the plan on the current stream.  The first call launches kernel by kernel (it also initialises
         per-kernel attributes and the tensor-map cache); the second call captures every run of launches between two
         Python callbacks into a CUDA graph (side-stream forks/joins become parallel branches), and from then on a
         plan costs one cudaGraphLaunch per segment instead of one ctypes call + cudaLaunchKernelEx per kernel
-        (≈140 per plan).  ``callbacks=False`` skips the Python callbacks (no gradient sync attached): one segment.
-        VITK_PLAN_GRAPHS=0 keeps the kernel-by-kernel path."""
-        self._enqueue(stream, side_stream, callbacks)
+        (≈140 per plan).  ``callbacks=False`` skips the Python callbacks (no gradient sync attached): one segment."""
+        self._enqueue(stream, callbacks)
         if callbacks:
             for ev, after in self.sync_points:
                 after(ev)
 
-    def _enqueue(self, stream: int, side_stream: Optional[torch.cuda.Stream], callbacks: bool):
-        if not _PLAN_GRAPHS or torch.cuda.is_current_stream_capturing():
-            self._run_range(0, len(self.steps), stream, side_stream, callbacks)
+    def _enqueue(self, stream: int, callbacks: bool):
+        if torch.cuda.is_current_stream_capturing():
+            self._run_range(0, len(self.steps), stream, callbacks)
             return
-        key = (callbacks, side_stream is not None, self.tail_stream is not None)
-        segs = self._segments.get(key)
+        segs = self._segments.get(callbacks)
         if segs is None:
-            if key not in self._warm:
-                self._warm.add(key)
-                self._run_range(0, len(self.steps), stream, side_stream, callbacks)
+            if callbacks not in self._warm:
+                self._warm.add(callbacks)
+                self._run_range(0, len(self.steps), stream, callbacks)
                 return
-            segs = self._segments[key] = self._capture(side_stream, callbacks)
+            segs = self._segments[callbacks] = self._capture(callbacks)
         for g, fn in segs:
             if fn is None:
                 g[0].replay()
@@ -155,7 +137,7 @@ class _Plan:
             else:
                 fn()
 
-    def _capture(self, side_stream, callbacks: bool):
+    def _capture(self, callbacks: bool):
         bounds, lo = [], 0
         for i, (fn, args, name) in enumerate(self.steps):
             if fn is None and name == "python" and callbacks:
@@ -173,7 +155,7 @@ class _Plan:
             g = torch.cuda.CUDAGraph()
             n0 = ops.direct_launch_count()
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                self._run_range(lo, hi, torch.cuda.current_stream().cuda_stream, side_stream, run_py=False)
+                self._run_range(lo, hi, torch.cuda.current_stream().cuda_stream, run_py=False)
             segs.append(((g, ops.direct_launch_count() - n0), None))
         return segs
 
@@ -304,7 +286,7 @@ class Arena:
         D, Fi, H, L, Cn = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.num_labels
         T, P, B, M = cfg.seq_len, cfg.num_patches, self.B, self.M
         scale = 64 ** -0.5
-        pl = _Plan()
+        pl = _Plan(eng.side_stream)
         # one external-event sync point per gradient bucket (no host callback, no break in the CUDA graph)
         ends = eng.grad_sync.bucket_end_layers() if eng.grad_sync is not None else set()
         done_hi = [L - 1]
@@ -314,12 +296,6 @@ class Arena:
                 lo, hi = l, done_hi[0]
                 done_hi[0] = l - 1
                 pl.sync_point(lambda ev, lo=lo, hi=hi: eng._layers_grads_ready(lo, hi, ev))
-        mc = eng.comm_reserved_ctas()         # GEMMs of the backward leave SMs to the overlapped all-reduce
-        _gemm = pl.gemm
-
-        def gemm_capped(*a, **k):
-            return _gemm(*a, max_ctas=mc, **k)
-        pl.gemm = gemm_capped
         dh, dh1 = self.dh
         pl.add("vitk_head_bwd", _p(self.h_last), _p(self.hstat[0]), _p(self.hstat[1]), _p(w["gf"]), _p(w["bf"]), _p(w["wc"]),
                B, T, D, Cn, _p(self.dlogits if from_loss else self.dlogits_in), _p(self.dloss) if from_loss else None,
@@ -337,27 +313,27 @@ class Arena:
         lw, lg, st = w["layers"][l], g["layers"][l], self.st[l]
         dh_c, dh1_c, dn_c, do_c = cls_rows(dh), cls_rows(dh1), cls_rows(self.dn), cls_rows(self.do)
         du_c, a_c, gp_c, n2_c, o_c = cls_rows(self.du), cls_rows(self.a[l]), cls_rows(self.gp[l]), cls_rows(self.n2[l]), cls_rows(self.o[l])
-        pl.gemm(dh_c, a_c, D, Fi, B, lg["w2"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+        pl.gemm(dh_c, a_c, D, Fi, B, lg["w2"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
         pl.add("vitk_colsum_bf16", _p(dh_c), B, D, T * D, _p(lg["bf2"]))
-        pl.gemm(dh_c, lw["w2_16"], B, Fi, D, du_c, EPI_MUL_BF16, b_mn=True, aux=gp_c)
-        pl.gemm(du_c, n2_c, Fi, D, B, lg["w1"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+        pl.gemm(dh_c, lw["w2_16"], B, Fi, D, du_c, EPI_MUL_BF16, b_mn_major=True, aux=gp_c)
+        pl.gemm(du_c, n2_c, Fi, D, B, lg["w1"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
         pl.add("vitk_colsum_bf16", _p(du_c), B, Fi, T * Fi, _p(lg["bf1"]))
-        pl.gemm(du_c, lw["w1_16"], B, D, Fi, dn_c, EPI_STORE_BF16, b_mn=True)
+        pl.gemm(du_c, lw["w1_16"], B, D, Fi, dn_c, EPI_STORE_BF16, b_mn_major=True)
         pl.add("vitk_fill_zero", _p(dh1), dh1.numel() * 2)
         pl.add("vitk_layernorm_bwd_rows", _p(self.dn), _p(self.h1[l]), T * D, _p(st[2]), _p(st[3]), _p(lw["g2"]), _p(dh), B, D, T,
                _p(dh1), _p(lg["g2"]), _p(lg["b2"]), _p(lg["bo"]))
-        pl.gemm(dh1_c, o_c, D, D, B, lg["wo"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+        pl.gemm(dh1_c, o_c, D, D, B, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
         if eng.cls_only_top:
-            pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn=True)
+            pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_cls_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale, _p(self.dqkv))
         else:
             pl.add("vitk_fill_zero", _p(self.do), self.do.numel() * 2)
-            pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn=True)
+            pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale,
                    _p(self.dqkv), _p(self.attn_ws))
-        pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+        pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
         pl.add("vitk_colsum_bf16", _p(self.dqkv), M, 3 * D, 3 * D, _p(lg["bqkv"]))
-        pl.gemm(self.dqkv, lw["wqkv16"], M, D, 3 * D, self.dn, EPI_STORE_BF16, b_mn=True)
+        pl.gemm(self.dqkv, lw["wqkv16"], M, D, 3 * D, self.dn, EPI_STORE_BF16, b_mn_major=True)
         pl.add("vitk_layernorm_bwd", _p(self.dn), _p(self.h[l]), D, _p(st[0]), _p(st[1]), _p(lw["g1"]), _p(dh1), M, D,
                _p(dh), _p(lg["g1"]), _p(lg["b1"]), _p(g["layers"][l - 1]["bf2"]) if l > 0 else None)
         layer_done(l)
@@ -371,37 +347,37 @@ class Arena:
             # MLP
             pl.fork()
             pl.side(True)
-            pl.gemm(dh, self.a[l], D, Fi, M, lg["w2"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+            pl.gemm(dh, self.a[l], D, Fi, M, lg["w2"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
             pl.side(False)
-            pl.gemm(dh, lw["w2_16"], M, Fi, D, self.du, EPI_MUL_BF16, b_mn=True, aux=self.gp[l])
+            pl.gemm(dh, lw["w2_16"], M, Fi, D, self.du, EPI_MUL_BF16, b_mn_major=True, aux=self.gp[l])
             pl.fork()
             pl.side(True)
-            pl.gemm(self.du, self.n2[l], Fi, D, M, lg["w1"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+            pl.gemm(self.du, self.n2[l], Fi, D, M, lg["w1"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
             pl.add("vitk_colsum_bf16", _p(self.du), M, Fi, Fi, _p(lg["bf1"]))
             pl.side(False)
-            pl.gemm(self.du, lw["w1_16"], M, D, Fi, self.dn, EPI_STORE_BF16, b_mn=True)
+            pl.gemm(self.du, lw["w1_16"], M, D, Fi, self.dn, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_layernorm_bwd", _p(self.dn), _p(self.h1[l]), D, _p(st[2]), _p(st[3]), _p(lw["g2"]), _p(dh), M, D,
                    _p(dh1), _p(lg["g2"]), _p(lg["b2"]), _p(lg["bo"]))
             # attention
             pl.fork()
             pl.side(True)
-            pl.gemm(dh1, self.o[l], D, D, M, lg["wo"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+            pl.gemm(dh1, self.o[l], D, D, M, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
             pl.side(False)
-            pl.gemm(dh1, lw["wo16"], M, D, D, self.do, EPI_STORE_BF16, b_mn=True)
+            pl.gemm(dh1, lw["wo16"], M, D, D, self.do, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale,
                    _p(self.dqkv), _p(self.attn_ws))
             pl.fork()
             pl.side(True)
-            pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+            pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
             pl.add("vitk_colsum_bf16", _p(self.dqkv), M, 3 * D, 3 * D, _p(lg["bqkv"]))
             pl.side(False)
-            pl.gemm(self.dqkv, lw["wqkv16"], M, D, 3 * D, self.dn, EPI_STORE_BF16, b_mn=True)
+            pl.gemm(self.dqkv, lw["wqkv16"], M, D, 3 * D, self.dn, EPI_STORE_BF16, b_mn_major=True)
             pl.join()          # side work of this layer read dh / du / dh1 / dqkv, which the next kernels overwrite
             pl.add("vitk_layernorm_bwd", _p(self.dn), _p(self.h[l]), D, _p(st[0]), _p(st[1]), _p(lw["g1"]), _p(dh1), M, D,
                    _p(dh), _p(lg["g1"]), _p(lg["b1"]), _p(g["layers"][l - 1]["bf2"]) if l > 0 else None)
             layer_done(l)
         pl.add("vitk_embed_bwd", _p(dh), B, T, D, _p(g["pos"]), _p(g["cls"]), _p(g["bp"]), _p(self.dpatch))
-        pl.gemm(self.dpatch, self.apatch, D, 768, B * P, g["wp"], EPI_ACCUM_F32, a_mn=True, b_mn=True)
+        pl.gemm(self.dpatch, self.apatch, D, 768, B * P, g["wp"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
         if eng.grad_sync is not None:
             pl.sync_point(lambda ev: eng._rest_grads_ready(ev))
         return pl
@@ -415,7 +391,7 @@ class Engine:
         self.ticket = 0
         self.arenas: Dict[Tuple[int, bool], Arena] = {}
         self.grad_sync = None            # parallel.GradSync, set by the caller for N>1
-        self.side_stream = torch.cuda.Stream(device=self.dev) if os.environ.get("VITK_SIDE_STREAM", "1") != "0" else None
+        self.side_stream = torch.cuda.Stream(device=self.dev)    # weight-gradient work of the backward plans
         # top encoder layer computed for the CLS rows only (forward and backward); VITK_CLS_ONLY_TOP=0 runs it densely
         self.cls_only_top = os.environ.get("VITK_CLS_ONLY_TOP", "1") != "0"
         self.w = self._weight_views(model.flat_parameters(), model.shadow())
@@ -473,16 +449,6 @@ class Engine:
                 "g1": v(p + "layernorm_before.weight"), "b1": v(p + "layernorm_before.bias"),
                 "g2": v(p + "layernorm_after.weight"), "b2": v(p + "layernorm_after.bias")})
         return out
-
-    def comm_reserved_ctas(self) -> int:
-        """Persistent-grid cap for backward GEMMs while gradient buckets are being all-reduced: NCCL's
-        CTAs need SMs, and a CTA pair that cannot be placed at launch starts (and ends) a whole tile late.
-        0 = no cap (single GPU)."""
-        if self.grad_sync is None or getattr(self.grad_sync, "world", 1) == 1:
-            return 0
-        reserve = int(os.environ.get("VITK_COMM_SMS", "0"))   # measured at N=4: reserving 8–32 SMs costs more than it saves
-        sms = torch.cuda.get_device_properties(self.dev).multi_processor_count
-        return max(2, sms - reserve) if reserve > 0 else 0
 
     def arena(self, B: int, train: bool) -> Arena:
         key = (B, train)
@@ -553,13 +519,13 @@ class Engine:
         stream = torch.cuda.current_stream().cuda_stream
         if dloss is not None and dlogits is None:
             ar.dloss.copy_(dloss.reshape(1), non_blocking=True)
-            ar.backward_plan(True, staged).run(stream, self.side_stream, callbacks=self.grad_sync is not None)
+            ar.backward_plan(True, staged).run(stream, callbacks=self.grad_sync is not None)
         else:
             if dloss is not None:      # both the loss and the logits were used downstream
                 torch.add(dlogits.to(f32), ar.dlogits * dloss.to(f32), out=ar.dlogits_in)
             else:
                 ar.dlogits_in.copy_(dlogits)
-            ar.backward_plan(False, staged).run(stream, self.side_stream, callbacks=self.grad_sync is not None)
+            ar.backward_plan(False, staged).run(stream, callbacks=self.grad_sync is not None)
         ar.ticket = -1
         if needs is None:
             needs = (True,) * n

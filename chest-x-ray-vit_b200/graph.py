@@ -125,7 +125,7 @@ class GraphedTrainStep:
         with torch.cuda.graph(graph):
             s = torch.cuda.current_stream().cuda_stream
             ar.fwd_loss.run(s)
-            ar.backward_plan(True, False).run(s, eng.side_stream)
+            ar.backward_plan(True, False).run(s)
             opt._enqueue(g, p, segs, True, 0, (self._step_dev, self._bc_dev))
         n = ops.direct_launch_count() - n0
         model._grads_clean = True

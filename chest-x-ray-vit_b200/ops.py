@@ -134,12 +134,13 @@ def layernorm_bwd(dy, x, mean, rstd, gamma, dres, dgamma, dbeta, dx=None, dxsum=
 
 
 # ----------------------------------------------------------------------------- GEMM
-def gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, d: torch.Tensor, *, epilogue: int,
-         a_mn_major: bool = False, b_mn_major: bool = False, lda: Optional[int] = None, ldb: Optional[int] = None,
-         ldd: Optional[int] = None, d2: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None,
-         aux: Optional[torch.Tensor] = None, ld_aux: int = 0, rows_in: int = 0, rows_out: int = 0, row_off: int = 0,
-         split_k: int = 0, tile_n: int = 0, max_ctas: int = 0, variant: int = 0) -> torch.Tensor:
-    """D[M,N] = A·Bᵀ (logical A [M,K], B [N,K]) on tcgen05 with a fused epilogue; see vitk.h."""
+def gemm_args(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, d: torch.Tensor, *, epilogue: int,
+              a_mn_major: bool = False, b_mn_major: bool = False, lda: Optional[int] = None, ldb: Optional[int] = None,
+              ldd: Optional[int] = None, d2: Optional[torch.Tensor] = None, bias: Optional[torch.Tensor] = None,
+              aux: Optional[torch.Tensor] = None, ld_aux: Optional[int] = None, rows_in: int = 0, rows_out: int = 0,
+              row_off: int = 0, split_k: int = 0, tile_n: int = 0, max_ctas: int = 0, variant: int = 0) -> GemmArgs:
+    """The vitk_gemm_bf16 argument struct of D[M,N] = A·Bᵀ.  Leading dimensions left out (None, or 0 for ld_aux) are the
+    row strides of the tensors."""
     g = GemmArgs()
     g.a, g.b = a.data_ptr(), b.data_ptr()
     g.M, g.N, g.K = M, N, K
@@ -154,6 +155,13 @@ def gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, d: torch.Tens
     g.ld_aux = ld_aux if ld_aux else (aux.stride(0) if aux is not None else 0)
     g.rows_in, g.rows_out, g.row_off = rows_in, rows_out, row_off
     g.tile_n, g.max_ctas, g.variant = tile_n, max_ctas, variant
+    return g
+
+
+def gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, d: torch.Tensor, **kw) -> torch.Tensor:
+    """D[M,N] = A·Bᵀ (logical A [M,K], B [N,K]) on tcgen05 with a fused epilogue; see vitk.h.  Keyword arguments
+    (``epilogue`` is required) as for gemm_args."""
+    g = gemm_args(a, b, M, N, K, d, **kw)
     _lib.check(_lib.lib().vitk_gemm_bf16(C.byref(g), _stream()), "gemm_bf16")
     return d
 

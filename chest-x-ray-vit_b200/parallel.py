@@ -12,7 +12,6 @@ compute stream only waits after the last bucket, right before the optimizer need
 """
 from __future__ import annotations
 
-import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -190,7 +189,6 @@ class PeerGradSync(GradSync):
         # room for a second CTA), so the small mean / barrier kernels only get SMs at kernel boundaries — and must get them
         # FIRST there, or they starve (measured: 485 µs for a 20 µs kernel at default priority)
         self.comm = torch.cuda.Stream(device=dev, priority=-1)
-        self.mean_ctas = int(os.environ.get("VITK_PEER_MEAN_CTAS", "0"))      # 0 = two CTAs per SM: short and wide
         self._chan = 0
         self._last = None
         self.timeout_ms = 20000           # a protocol bug traps after 20 s instead of hanging the GPUs
@@ -265,8 +263,7 @@ class PeerGradSync(GradSync):
                 off += n
             mark()
             for lo, n, o in mine:
-                ops.shard_mean(flat[lo:lo + n], self.scratch[o:], self.max_shard, self.world - 1, 1.0 / self.world,
-                               max_ctas=self.mean_ctas)
+                ops.shard_mean(flat[lo:lo + n], self.scratch[o:], self.max_shard, self.world - 1, 1.0 / self.world)
             mark()
             self._barrier()                                           # every owner has reduced its shards
             mark()

@@ -31,7 +31,8 @@ def _ref(qkv, do, scale):
 # 8 key blocks (1024: the 3-deep K/V ring is recycled)
 @pytest.mark.parametrize("B,T,H", [(1, 128, 1), (1, 64, 2), (2, 17, 2), (2, 129, 3), (2, 197, 12), (1, 256, 2), (2, 577, 12),
                                    (1, 300, 16), (1, 385, 2), (1, 640, 2), (1, 1024, 1), (16, 577, 12),
-                                   (1, 130, 6), (1, 70, 20)])      # head counts of every attn_delta instantiation (≤4, ≤8, ≤12, ≤16, >16)
+                                   (1, 130, 6), (1, 70, 20),       # head counts of every attn_delta instantiation (≤4, ≤8, ≤12, ≤16, >16)
+                                   (2, 129, 20)])                  # H > 16 (attn_delta_kernel) with two images and two key blocks
 def test_attention_fwd_bwd(ops, B, T, H):
     g = torch.Generator().manual_seed(T * 10 + H)
     qkv = (torch.randn(B, T, 3, H, 64, generator=g)).to(dev).to(bf16)

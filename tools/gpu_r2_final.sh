@@ -1,6 +1,5 @@
 #!/bin/bash
-# what the driver runs at round end, plus the diagnostics kept under profiles/: full GPU test-suite, smoke, benches, launch list,
-# ncu --set full of the kernels that changed last (fc1 + GELU GEMM with 16 epilogue warps, persistent attention backward, attn_delta16)
+# end-of-round check: full GPU test-suite, smoke, benches (default, ViT-L, inference, reference arm)
 mkdir -p gpurun_out
 O=gpurun_out
 timeout 1200 python -m pytest tests -q -m gpu -x --timeout 900 > $O/pytest_gpu_all.log 2>&1; echo "pytest -m gpu rc=$?"; tail -3 $O/pytest_gpu_all.log
@@ -9,13 +8,3 @@ timeout 400 python bench.py > $O/bench.json 2> $O/bench.err; echo "bench rc=$?";
 timeout 300 python bench.py --config vitl384 --steps 10 --warmup 3 --no-cpu-baseline > $O/bench_vitl.json 2> $O/bench_vitl.err; echo "vitl rc=$?"; cut -c1-200 $O/bench_vitl.json
 timeout 300 python bench.py --config vitb224-infer --steps 20 --warmup 3 > $O/bench_infer.json 2> $O/bench_infer.err; echo "infer rc=$?"
 timeout 300 python bench.py --impl reference --steps 3 --warmup 1 > $O/bench_ref.json 2> $O/bench_ref.err; echo "reference rc=$?"; cut -c1-200 $O/bench_ref.json
-P="python tools/profile_step.py"
-timeout 200 $P > $O/plain.log 2>&1 &&
-timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none --profile-from-start off --csv --log-file $O/launches.csv $P > $O/ncu_launches.log 2>&1; echo "launch list rc=$?"
-rm -f $O/prof_*.ncu-rep
-full() {   # name, kernel regex, skip, count
-  timeout 300 ncu --set full --clock-control none --import-source on --profile-from-start off -k regex:"$2" -s $3 -c $4 -f -o $O/prof_$1 $P > $O/ncu_$1.log 2>&1
-  echo "$1 rc=$?"
-}
-full gemm_fwd "gemm2_bf16" 20 4
-full attn "attn_(fwd|bwd|delta|dq_store)" 20 4      # forward launches 0..11, then 4 per backward layer: skip 12 fwd + 2 layers
