@@ -52,6 +52,7 @@ _PROTOS = {
     "vitk_gemm_bf16": (C.c_int, [C.POINTER(GemmArgs), _p]),
     "vitk_colsum_bf16": (C.c_int, [_p, _i64, _i64, _i64, _p, _p]),
     "vitk_attn_fwd": (C.c_int, [_p, _i64, _i64, _i64, _f, _p, _p, _p]),
+    "vitk_attn_probs": (C.c_int, [_p, _p, _i64, _i64, _i64, _f, _p, _p]),
     "vitk_attn_cls_fwd": (C.c_int, [_p, _i64, _i64, _i64, _f, _p, _p, _p]),
     "vitk_attn_cls_bwd": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _i64, _f, _p, _p]),
     "vitk_attn_bwd_workspace_bytes": (_sz, [_i64, _i64, _i64]),

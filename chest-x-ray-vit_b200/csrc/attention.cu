@@ -18,6 +18,7 @@
 #include <math.h>
 
 #include <atomic>
+#include <mutex>
 
 #include "common.cuh"
 #include "sm100_prims.cuh"
@@ -816,6 +817,144 @@ attn_bwd_kernel(const __grid_constant__ CUtensorMap tma_qkv, const __grid_consta
   }
 }
 
+// ============================================================================ attention probabilities
+// probs[b,h,i,j] = exp2(S[i,j]·scale_log2 − lse[b,h,i]·log2e) as fp32 [B,H,T,T]: the softmax rows HF's
+// eager_attention_forward returns (modeling_vit.py:185-190), recomputed from the qkv buffer and the lse attn_fwd wrote,
+// with attn_fwd's scale_log2, so each row is the one whose P·V produced o.  Bound by the HBM write (T² floats per
+// head and image, never read again on the GPU), not by the recompute.
+// CTA = (128 queries, head, image): a control warp loads Q once and 128-key K blocks through a 3-deep TMA ring and
+// issues S_j = Q·K_jᵀ (SS-MMA, M = N = 128) into one of two TMEM buffers, so block j+1's MMA overlaps block j's
+// epilogue.  Four epilogue warps (thread = query row = TMEM lane) read 32-column chunks, exponentiate, transpose them
+// through a padded [32 × 33] shared-memory slab per warp and store them as 128-byte rows (32 consecutive keys of one
+// query) with streaming stores.  Row stride T·4 bytes is not 16-byte aligned for odd T (577), which rules out TMA and
+// vector stores.  Keys and queries ≥ T (the zero-filled TMA padding) are never stored.  (Eight epilogue warps per CTA,
+// two per TMEM lane quadrant, wrote no faster: see DESIGN.md §4 for what bounds the kernel.)
+// ≈81 KB of shared memory → two CTAs per SM, whose 2 × 256 TMEM columns fill the SM's 512.
+constexpr int kPrbEpiWarps = 4;
+constexpr int kPrbThreads = (kPrbEpiWarps + 1) * 32;        // epilogue warps + control warp
+constexpr int kPrbKRing = 3;
+constexpr int kPrbSmemQ = 0;
+constexpr int kPrbSmemK = kPrbSmemQ + kTileBytes;
+constexpr int kPrbSmemStage = kPrbSmemK + kPrbKRing * kTileBytes;    // 4 warps × [32 rows × 33 floats]
+constexpr int kPrbStageFloats = 32 * 33;
+constexpr int kPrbSmemBar = kPrbSmemStage + kPrbEpiWarps * kPrbStageFloats * 4;
+constexpr int kPrbSmemBytes = kPrbSmemBar + 128 + 1024;
+constexpr int kPrbTmemCols = 256;                           // two 128-column score buffers
+
+__global__ void __launch_bounds__(kPrbThreads, 2)
+attn_probs_kernel(const __grid_constant__ CUtensorMap tma_qk, const float* __restrict__ lse, int T, int H, float scale_log2,
+                  float* __restrict__ probs) {
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  uint8_t* sQ = smem + kPrbSmemQ;
+  uint8_t* sK = smem + kPrbSmemK;
+  uint64_t* bar_q = reinterpret_cast<uint64_t*>(smem + kPrbSmemBar);
+  uint64_t* bar_k = bar_q + 1;        // [3] K block landed
+  uint64_t* bar_kfree = bar_q + 4;    // [3] the MMA reading this K slot retired
+  uint64_t* bar_s = bar_q + 7;        // [2] scores of this TMEM buffer ready
+  uint64_t* bar_tfree = bar_q + 9;    // [2] the 4 epilogue warps have read this TMEM buffer
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_q + 11);
+
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int qb = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
+  const int nkb = (T + kTile - 1) / kTile;
+
+  if (tid == 0) {
+    tma_prefetch_desc(&tma_qk);
+    for (int i = 0; i < 11; ++i) mbar_init(bar_q + i, (i == 9 || i == 10) ? kPrbEpiWarps : 1);
+    fence_mbar_init();
+  }
+  if (warp == kPrbEpiWarps) tmem_alloc(tmem_slot, kPrbTmemCols);
+  tc_fence_before_sync();
+  __syncthreads();
+  tc_fence_after_sync();
+  pdl_wait();
+  pdl_launch_dependents();
+  const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);
+
+  if (warp == kPrbEpiWarps) {
+    // ------------------------------------------------------------------ control warp: TMA + MMA issue (under elect.sync)
+    const int colq = h * kDh, colk = (H + h) * kDh;
+    auto load_k = [&](int j) {
+      const int s = j % kPrbKRing;
+      if (elect_one()) {
+        mbar_arrive_expect_tx(&bar_k[s], kTileBytes);
+        tma_load_3d(sK + s * kTileBytes, &tma_qk, &bar_k[s], colk, j * kTile, b);
+      }
+    };
+    if (elect_one()) {
+      mbar_arrive_expect_tx(bar_q, kTileBytes);
+      tma_load_3d(sQ, &tma_qk, bar_q, colq, qb * kTile, b);
+    }
+    for (int j = 0; j < nkb && j < kPrbKRing; ++j) load_k(j);
+    const uint64_t q_desc = umma_smem_desc(smem_u32(sQ), 0, 1024);
+    const uint64_t k_desc = umma_smem_desc(smem_u32(sK), 0, 1024);
+    constexpr uint32_t idesc = umma_idesc_bf16(kTile, kTile, 0, 0);
+    mbar_wait(bar_q, 0);
+    for (int j = 0; j < nkb; ++j) {
+      const int s = j % kPrbKRing, x = j & 1;
+      const uint32_t ph = (j / kPrbKRing) & 1;
+      mbar_wait(&bar_k[s], ph);
+      if (j >= 2) mbar_wait(&bar_tfree[x], ((j - 2) >> 1) & 1);
+      tc_fence_after_sync();
+      const uint64_t bk = k_desc + static_cast<uint64_t>(s * (kTileBytes >> 4));
+      if (elect_one()) {
+#pragma unroll
+        for (int k = 0; k < kDh / 16; ++k) tc_mma_bf16(tmem_base + x * kTile, q_desc + 2 * k, bk + 2 * k, idesc, k > 0);
+        tc_commit(&bar_s[x]);
+        tc_commit(&bar_kfree[s]);
+      }
+      __syncwarp();
+      if (j + kPrbKRing < nkb) {
+        mbar_wait(&bar_kfree[s], ph);
+        load_k(j + kPrbKRing);
+      }
+    }
+    __syncwarp();
+  } else {
+    // ------------------------------------------------------------------ epilogue warps
+    const uint32_t lane_field = static_cast<uint32_t>(warp * 32) << 16;
+    const int row0 = qb * kTile + warp * 32;          // first query row of this warp
+    const bool live = row0 < T;                        // false: all 32 rows are padding beyond T
+    const long long bh = static_cast<long long>(b) * H + h;
+    const int my_row = row0 + lane;
+    const float lse2 = my_row < T ? __ldg(lse + bh * T + my_row) * kLog2e : 0.f;
+    const int nrows = min(32, T - row0);
+    float* stage = reinterpret_cast<float*>(smem + kPrbSmemStage) + warp * kPrbStageFloats;
+    float* out_rows = probs + (bh * T + row0) * T;      // row row0 of this (image, head)
+    for (int j = 0; j < nkb; ++j) {
+      const int x = j & 1;
+      mbar_wait(&bar_s[x], (j >> 1) & 1);
+      tc_fence_after_sync();
+      const int nchunk = (min(kTile, T - j * kTile) + 31) >> 5;
+      for (int c = 0; live && c < nchunk; ++c) {
+        uint32_t r[32];
+        tmem_ld_32x32(tmem_base + lane_field + x * kTile + c * 32, r);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 32; ++i)     // (≤ 1: a row's maximum can round a few ulp above its lse)
+          stage[lane * 33 + i] = fminf(fast_exp2(fmaf(__uint_as_float(r[i]), scale_log2, -lse2)), 1.0f);
+        __syncwarp();
+        const int col = j * kTile + c * 32 + lane;
+        if (col < T) {
+#pragma unroll 8
+          for (int i = 0; i < nrows; ++i) __stcs(out_rows + static_cast<long long>(i) * T + col, stage[i * 33 + lane]);
+        }
+        __syncwarp();
+      }
+      tc_fence_before_sync();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bar_tfree[x]);
+    }
+  }
+  tc_fence_before_sync();
+  __syncthreads();
+  if (warp == kPrbEpiWarps) {
+    tc_fence_after_sync();
+    tmem_dealloc(tmem_base, kPrbTmemCols);
+  }
+}
+
 // dq_acc fp32 [B,T,H,64] · scale → dqkv[b,t,0,h,:] bf16
 __global__ void __launch_bounds__(256) attn_dq_store_kernel(const float* __restrict__ dq_acc, int BT, int H, float scale,
                                                             __nv_bfloat16* __restrict__ dqkv) {
@@ -873,6 +1012,28 @@ extern "C" VITK_API int vitk_attn_fwd(const void* qkv, int64_t B, int64_t T, int
   VITK_CUDA(launch_pdl(attn_fwd_kernel, grid, dim3(kFwdThreads), kFwdSmemBytes, static_cast<cudaStream_t>(stream), tm, tm_kv,
                        tm_o, lse, static_cast<int>(T), static_cast<int>(H), scale * kLog2e, g_timeline));
   VITK_LAUNCH_CHECK("attn_fwd_kernel");
+  return 0;
+}
+
+extern "C" VITK_API int vitk_attn_probs(const void* qkv, const float* lse, int64_t B, int64_t T, int64_t H, float scale,
+                                        float* probs, vitk_stream_t stream) {
+  VITK_REQUIRE(qkv && lse && probs, VITK_EINVAL, "attn_probs: NULL argument");
+  if (int rc = check_shape("attn_probs", B, T, H)) return rc;
+  VITK_REQUIRE(aligned16(qkv) && (reinterpret_cast<uintptr_t>(lse) & 3u) == 0 && (reinterpret_cast<uintptr_t>(probs) & 3u) == 0,
+               VITK_EALIGN, "attn_probs: qkv must be 16-byte aligned, lse and probs 4-byte aligned");
+  VITK_REQUIRE(scale > 0.f, VITK_EINVAL, "attn_probs: scale must be positive");
+  CUtensorMap tm;
+  if (int rc = qkv_tensor_map(&tm, qkv, B, T, 3 * H * kDh)) return rc;
+  static std::once_flag once;
+  static cudaError_t attr_err = cudaSuccess;
+  std::call_once(once, [] {
+    attr_err = cudaFuncSetAttribute(attn_probs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPrbSmemBytes);
+  });
+  if (attr_err != cudaSuccess) return cuda_error(attr_err, "cudaFuncSetAttribute(attn_probs smem)");
+  const dim3 grid(static_cast<unsigned>((T + kTile - 1) / kTile), static_cast<unsigned>(H), static_cast<unsigned>(B));
+  VITK_CUDA(launch_pdl(attn_probs_kernel, grid, dim3(kPrbThreads), kPrbSmemBytes, static_cast<cudaStream_t>(stream), tm, lse,
+                       static_cast<int>(T), static_cast<int>(H), scale * kLog2e, probs));
+  VITK_LAUNCH_CHECK("attn_probs_kernel");
   return 0;
 }
 

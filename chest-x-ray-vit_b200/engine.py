@@ -198,6 +198,11 @@ class Arena:
         self.hstat = new((2, B), f32)
         self.fwd = self._build_forward(eng, with_labels=False)
         self.fwd_loss = self._build_forward(eng, with_labels=True)
+        self._eng = eng
+        self._outputs_plans: Dict[bool, _Plan] = {}
+        self.hs: Optional[torch.Tensor] = None         # eval arena, outputs plans: the residual stream of every layer
+        self.qkv_all: List[torch.Tensor] = self.qkv if train else []
+        self.lse_all: List[torch.Tensor] = self.lse if train else []
         if train:
             self.dh = [new((M, D), bf16) for _ in range(2)]
             self.dn = new((M, D), bf16)
@@ -209,7 +214,6 @@ class Arena:
             self.dloss = new((1,), f32)
             self.dlogits_in = new((B, Cn), f32)
             self._bwd_plans: Dict[Tuple[bool, bool], _Plan] = {}
-            self._eng = eng
             self.bwd_loss = self.backward_plan(True, False)
             self.bwd_logits = self.backward_plan(False, False)
 
@@ -223,15 +227,46 @@ class Arena:
             pl = self._bwd_plans[key] = self._build_backward(eng, from_loss, eng.g_stage() if staged else eng.g)
         return pl
 
+    def outputs_plan(self, with_labels: bool) -> _Plan:
+        """Forward plan that keeps what hidden states and attention maps are read from (built on first use): the top layer
+        runs on every token, and every layer's input stream, qkv and lse stay in buffers of their own — in the train arena
+        those that backward keeps anyway; the eval arena gets a [L+1, M, D] stream buffer and L qkv / lse buffers here."""
+        pl = self._outputs_plans.get(with_labels)
+        if pl is None:
+            eng = self._eng
+            cfg = eng.cfg
+            D, H, L, T = cfg.hidden_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.seq_len
+            if not self.train and self.hs is None:
+                self.hs = torch.empty((L + 1, self.M, D), dtype=f32, device=eng.dev)
+                self.qkv_all = [torch.empty((self.M, 3 * D), dtype=bf16, device=eng.dev) for _ in range(L)]
+                self.lse_all = [torch.empty((self.B, H, T), dtype=f32, device=eng.dev) for _ in range(L)]
+            pl = self._outputs_plans[with_labels] = self._build_forward(eng, with_labels, outputs=True)
+        return pl
+
+    def hidden_states(self) -> Tuple[torch.Tensor, ...]:
+        """Copies of the L+1 residual-stream tensors an outputs plan left behind, each fp32 [B, T, D]."""
+        cfg = self._eng.cfg
+        L, T, D = cfg.num_hidden_layers, cfg.seq_len, cfg.hidden_size
+        hs = torch.stack(self.h) if self.train else self.hs.clone()
+        return hs.view(L + 1, self.B, T, D).unbind(0)
+
     # ------------------------------------------------------------------ forward plan
-    def _build_forward(self, eng: "Engine", with_labels: bool) -> _Plan:
+    def _build_forward(self, eng: "Engine", with_labels: bool, outputs: bool = False) -> _Plan:
         cfg, w = eng.cfg, eng.w
         D, Fi, H, L, Cn = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.num_labels
         T, P, B, M = cfg.seq_len, cfg.num_patches, self.B, self.M
         eps = cfg.layer_norm_eps
         scale = 64 ** -0.5
         pl = _Plan()
-        h0 = self.h[0]
+        # residual stream before / after each layer, and where each layer's qkv / lse go: the train arena keeps them all;
+        # the eval arena updates one buffer in place, except in an outputs plan
+        if self.train:
+            hs, qkv, lse = self.h, self.qkv, self.lse
+        elif outputs:
+            hs, qkv, lse = self.hs, self.qkv_all, self.lse_all
+        else:
+            hs, qkv, lse = [self.h[0]] * (L + 1), [self.qkv[0]] * L, [self.lse[0]] * L
+        h0 = hs[0]
         pl.add("vitk_embed_cls", _p(w["cls"]), _p(w["pos"]), B, T, D, _p(h0))
         pl.gemm(self.apatch, w["wp16"], B * P, D, 768, h0, EPI_PATCH_F32, bias=w["bp"], aux=w["pos"], rows_in=P, rows_out=T,
                 row_off=1, ldd=D, ld_aux=D)
@@ -241,20 +276,20 @@ class Arena:
 
         for l in range(L):
             i = l if self.train else 0
-            hin = self.h[l] if self.train else self.h[0]
-            h1 = self.h1[i] if self.train else self.h[0]
-            hout = self.h[l + 1] if self.train else self.h[0]
+            hin, hout = hs[l], hs[l + 1]
+            h1 = self.h1[i] if self.train else hout
             lw = w["layers"][l]
             st = self.st[i]
             pl.add("vitk_layernorm_fwd", _p(hin), D, _p(lw["g1"]), _p(lw["b1"]), eps, M, D, _p(self.n1[i]), _p(st[0]), _p(st[1]))
-            pl.gemm(self.n1[i], lw["wqkv16"], M, 3 * D, D, self.qkv[i], EPI_BIAS_BF16, bias=lw["bqkv"])
-            if l == L - 1 and eng.cls_only_top:
+            pl.gemm(self.n1[i], lw["wqkv16"], M, 3 * D, D, qkv[l], EPI_BIAS_BF16, bias=lw["bqkv"])
+            if l == L - 1 and eng.cls_only_top and not outputs:
                 # ---- top layer: the classifier reads sequence_output[:, 0] only (HF modeling_vit.py:641), so after the keys
                 # and values of all tokens exist, everything else of this layer is computed for the B CLS rows alone —
                 # attention of one query per head, then out-proj / LN / MLP on strided [B, ·] views that leave the rows
                 # where the (CLS-only) backward of this layer expects them.  Dead rows are never read; FLOPs in bench.py
-                # stay on the dense convention.
-                pl.add("vitk_attn_cls_fwd", _p(self.qkv[i]), B, T, H, scale, _p(self.o[i]), _p(self.lse[i]))
+                # stay on the dense convention.  (An outputs plan needs every row, and runs this layer densely: the rows
+                # the CLS-only backward reads are among those the dense layer writes.)
+                pl.add("vitk_attn_cls_fwd", _p(qkv[l]), B, T, H, scale, _p(self.o[i]), _p(lse[l]))
                 o_c, hin_c, h1_c, hout_c = cls_rows(self.o[i]), cls_rows(hin), cls_rows(h1), cls_rows(hout)
                 n2_c, a_c = cls_rows(self.n2[i]), cls_rows(self.a[i])
                 pl.gemm(o_c, lw["wo16"], B, D, D, h1_c, EPI_BIAS_RESID_F32, bias=lw["bo"], aux=hin_c)
@@ -264,13 +299,13 @@ class Arena:
                         bias=lw["bf1"])
                 pl.gemm(a_c, lw["w2_16"], B, D, Fi, hout_c, EPI_BIAS_RESID_F32, bias=lw["bf2"], aux=h1_c)
                 continue
-            pl.add("vitk_attn_fwd", _p(self.qkv[i]), B, T, H, scale, _p(self.o[i]), _p(self.lse[i]))
+            pl.add("vitk_attn_fwd", _p(qkv[l]), B, T, H, scale, _p(self.o[i]), _p(lse[l]))
             pl.gemm(self.o[i], lw["wo16"], M, D, D, h1, EPI_BIAS_RESID_F32, bias=lw["bo"], aux=hin)
             pl.add("vitk_layernorm_fwd", _p(h1), D, _p(lw["g2"]), _p(lw["b2"]), eps, M, D, _p(self.n2[i]), _p(st[2]), _p(st[3]))
             pl.gemm(self.n2[i], lw["w1_16"], M, Fi, D, self.a[i], EPI_BIAS_GELUG_BF16, d2=self.gp[i] if self.train else None,
                     bias=lw["bf1"])
             pl.gemm(self.a[i], lw["w2_16"], M, D, Fi, hout, EPI_BIAS_RESID_F32, bias=lw["bf2"], aux=h1)
-        hl = self.h[L] if self.train else self.h[0]
+        hl = hs[L]
         self.h_last = hl
         if with_labels:
             pl.add("vitk_head_fwd", _p(hl), B, T, D, Cn, _p(w["gf"]), _p(w["bf"]), eps, _p(w["wc"]), _p(w["bc"]), _p(self.labels),
@@ -458,7 +493,11 @@ class Engine:
         return a
 
     # ------------------------------------------------------------------ forward
-    def forward(self, pixel_values: torch.Tensor, labels: Optional[torch.Tensor], save: bool):
+    def forward(self, pixel_values: torch.Tensor, labels: Optional[torch.Tensor], save: bool, output_attentions: bool = False,
+                output_hidden_states: bool = False):
+        """Runs the forward plan → (loss | None, logits, hidden_states | None, attentions | None), all fresh tensors.
+        Either flag selects the arena's outputs plan; the attention maps are then recomputed per layer by
+        vitk_attn_probs straight into one [L, B, H, T, T] allocation."""
         cfg = self.cfg
         B = pixel_values.shape[0]
         ar = self.arena(B, save)
@@ -473,12 +512,24 @@ class Engine:
             ops.patchify_f32(x if x.is_contiguous() else x.contiguous(), out=ar.apatch)
         if labels is not None:
             ar.labels.copy_(labels.reshape(B, cfg.num_labels), non_blocking=True)
-        (ar.fwd_loss if labels is not None else ar.fwd).run(torch.cuda.current_stream().cuda_stream)
+        if output_attentions or output_hidden_states:
+            plan = ar.outputs_plan(labels is not None)
+        else:
+            plan = ar.fwd_loss if labels is not None else ar.fwd
+        plan.run(torch.cuda.current_stream().cuda_stream)
         if save:
             self.ticket += 1
             ar.ticket = self.ticket
+        hidden = ar.hidden_states() if output_hidden_states else None
+        attn = None
+        if output_attentions:
+            H, L, T = cfg.num_attention_heads, cfg.num_hidden_layers, cfg.seq_len
+            probs = torch.empty((L, B, H, T, T), dtype=f32, device=self.dev)
+            for l in range(L):
+                ops.attn_probs(ar.qkv_all[l], ar.lse_all[l], B, T, H, 64 ** -0.5, out=probs[l])
+            attn = probs.unbind(0)
         loss = ar.loss[0].clone() if labels is not None else None
-        return loss, ar.logits.clone()
+        return loss, ar.logits.clone(), hidden, attn
 
     # ------------------------------------------------------------------ backward
     def bind_grads(self) -> None:

@@ -7,6 +7,8 @@ transformers/models/vit/modeling_vit.py:605-653 (HF 5.5.0):
     model = ViTForImageClassification(config)            # same parameter names / shapes as HF
     out = model(pixel_values=x, labels=y)                # ImageClassifierOutput(loss, logits)
     out.loss.backward(); optimizer.step()                # fp32 grads land in param.grad
+    out = model(pixel_values=x, output_attentions=True,  # + hidden_states (L+1 × [B,T,D]) and attentions
+              output_hidden_states=True)                 #   (L × [B,H,T,T]), as HF's eager attention returns them
 
 Every FLOP and byte of forward/backward runs in libvitk's sm_100a kernels through the C ABI
 (include/vitk.h); PyTorch provides device memory, streams and the autograd hook only.  There is
@@ -50,6 +52,8 @@ class ViTConfig:
     label2id: Optional[Dict[str, int]] = None
     image_mean: Tuple[float, float, float] = (0.5, 0.5, 0.5)
     image_std: Tuple[float, float, float] = (0.5, 0.5, 0.5)
+    output_attentions: bool = False         # defaults of forward()'s keyword arguments, as in HF PretrainedConfig
+    output_hidden_states: bool = False
 
     @classmethod
     def from_hf(cls, hf_config, **overrides) -> "ViTConfig":
@@ -370,26 +374,40 @@ class ViTForImageClassification(nn.Module):
             raise ValueError(f"Input image size ({h}*{w}) doesn't match model ({cfg.image_size}*{cfg.image_size}).")  # HF:161-165
 
     def forward(self, pixel_values: Optional[torch.Tensor] = None, labels: Optional[torch.Tensor] = None,
-                interpolate_pos_encoding: Optional[bool] = None, **kwargs) -> ImageClassifierOutput:
+                interpolate_pos_encoding: Optional[bool] = None, output_attentions: Optional[bool] = None,
+                output_hidden_states: Optional[bool] = None, **kwargs) -> ImageClassifierOutput:
         """HF ViTForImageClassification.forward (modeling_vit.py:620-653).  ``pixel_values``:
         fp32 [B,3,H,W] (the collate_fn contract) or uint8 grayscale [B,H,W] (normalised on the
-        GPU with config.image_mean/std).  Unknown kwargs (``num_items_in_batch``) are ignored."""
+        GPU with config.image_mean/std).  Unknown kwargs (``num_items_in_batch``) are ignored.
+
+        ``output_hidden_states`` (default ``config.output_hidden_states``): ``hidden_states`` is a tuple of L+1 fp32
+        [B,T,D] tensors — the embeddings output, then the output of each encoder layer; the last one is taken before
+        the final LayerNorm, as in HF.  ``output_attentions`` (default ``config.output_attentions``): ``attentions`` is
+        a tuple of L fp32 [B,H,T,T] softmax probabilities per layer, what HF's ``eager`` attention returns (HF's default
+        ``sdpa`` attention returns an empty tuple there).  Both are fresh tensors outside autograd
+        (``requires_grad=False``): ``loss.backward()`` gives the same gradients as without them, and no gradient flows
+        through them.  Requesting either runs the top encoder layer on every token instead of the CLS rows alone."""
         if pixel_values is None:
             raise ValueError("You have to specify pixel_values")                               # HF:440-441
         if interpolate_pos_encoding:
             raise ValueError("interpolate_pos_encoding is not supported by the B200 kernel path")
-        if kwargs.get("output_attentions") or kwargs.get("output_hidden_states"):
-            raise ValueError("output_attentions / output_hidden_states are not supported by the B200 kernel path")
+        cfg = self.config
+        want_attn = bool(cfg.output_attentions if output_attentions is None else output_attentions)
+        want_hidden = bool(cfg.output_hidden_states if output_hidden_states is None else output_hidden_states)
         self._check_inputs(pixel_values)
         eng = self.engine()
-        if labels is not None and self.config.problem_type is None:
-            self.config.problem_type = "multi_label_classification"     # HF loss_utils.py:92-98 (float labels)
+        if labels is not None and cfg.problem_type is None:
+            cfg.problem_type = "multi_label_classification"     # HF loss_utils.py:92-98 (float labels)
         need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.param_list())
+        extras = {"attentions": want_attn, "hidden_states": want_hidden}
         if need_grad:
-            loss, logits = _VitFunction.apply(self, pixel_values, labels, *self.param_list())
+            loss, logits = _VitFunction.apply(self, pixel_values, labels, extras, *self.param_list())
+            hidden, attn = extras["out"]
         else:
-            loss, logits = eng.forward(pixel_values, labels, save=False)
-        return ImageClassifierOutput(loss=loss if labels is not None else None, logits=logits)
+            loss, logits, hidden, attn = eng.forward(pixel_values, labels, save=False, output_attentions=want_attn,
+                                                     output_hidden_states=want_hidden)
+        return ImageClassifierOutput(loss=loss if labels is not None else None, logits=logits, hidden_states=hidden,
+                                     attentions=attn)
 
 
 class _VitFunction(torch.autograd.Function):
@@ -399,12 +417,15 @@ class _VitFunction(torch.autograd.Function):
     reducer all see what they expect.  The returned gradients are views of one flat fp32 buffer the kernels wrote:
     when ``param.grad`` is None autograd adopts the view without a copy, so the optimizer still finds all gradients
     contiguous; when ``param.grad`` is already populated (gradient accumulation) the kernels write a second buffer
-    and autograd adds it in place."""
+    and autograd adds it in place.  Requested hidden states / attention maps leave through ``extras["out"]``, outside
+    autograd."""
 
     @staticmethod
-    def forward(ctx, model: ViTForImageClassification, pixel_values, labels, *params):
+    def forward(ctx, model: ViTForImageClassification, pixel_values, labels, extras, *params):
         eng = model.engine()
-        loss, logits = eng.forward(pixel_values, labels, save=True)
+        loss, logits, hidden, attn = eng.forward(pixel_values, labels, save=True, output_attentions=extras["attentions"],
+                                                 output_hidden_states=extras["hidden_states"])
+        extras["out"] = (hidden, attn)
         ctx.model = model
         ctx.ticket = eng.ticket
         ctx.has_labels = labels is not None
@@ -416,5 +437,5 @@ class _VitFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dloss, dlogits):
         model = ctx.model
-        grads = model.engine().backward(ctx.ticket, dloss if ctx.has_labels else None, dlogits, ctx.needs_input_grad[3:])
-        return (None, None, None) + grads
+        grads = model.engine().backward(ctx.ticket, dloss if ctx.has_labels else None, dlogits, ctx.needs_input_grad[4:])
+        return (None, None, None, None) + grads

@@ -197,6 +197,23 @@ def attn_fwd(qkv: torch.Tensor, B: int, T: int, H: int, scale: float, o: Optiona
     return o, lse
 
 
+def attn_probs(qkv: torch.Tensor, lse: torch.Tensor, B: int, T: int, H: int, scale: float,
+               out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Softmax probabilities of attn_fwd, recomputed from its qkv bf16 [B,T,3,H,64] and lse fp32 [B,H,T]:
+    fp32 [B,H,T,T] (HF eager attention's attn_weights).  ``out``: a contiguous fp32 CUDA tensor of B·H·T² elements."""
+    assert qkv.dtype == bf16 and qkv.is_cuda and qkv.is_contiguous() and qkv.numel() == B * T * 3 * H * 64, \
+        "attn_probs: qkv must be a contiguous bf16 CUDA tensor of B·T·3·H·64 elements"
+    assert lse.dtype == f32 and lse.is_cuda and lse.is_contiguous() and lse.numel() == B * H * T, \
+        "attn_probs: lse must be a contiguous fp32 CUDA tensor of B·H·T elements"
+    if out is None:
+        out = torch.empty((B, H, T, T), dtype=f32, device=qkv.device)
+    assert out.dtype == f32 and out.is_cuda and out.is_contiguous() and out.numel() == B * H * T * T, \
+        "attn_probs: out must be a contiguous fp32 CUDA tensor of B·H·T² elements"
+    _lib.check(_lib.lib().vitk_attn_probs(qkv.data_ptr(), lse.data_ptr(), B, T, H, scale, out.data_ptr(), _stream()),
+               "attn_probs")
+    return out
+
+
 def attn_bwd_workspace_bytes(B: int, T: int, H: int) -> int:
     return int(_lib.lib().vitk_attn_bwd_workspace_bytes(B, T, H))
 

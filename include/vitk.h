@@ -144,6 +144,11 @@ VITK_API int vitk_colsum_bf16(const void* x_bf16, int64_t M, int64_t N, int64_t 
  * o bf16 [B,T,H*64]; lse fp32 [B,H,T] (natural-log sum-exp of the scaled scores). */
 VITK_API int vitk_attn_fwd(const void* qkv_bf16, int64_t B, int64_t T, int64_t H, float scale, void* o_bf16, float* lse,
                   vitk_stream_t stream);
+/* p[b,h,i,j] = exp(scale·q_i·k_j − lse[b,h,i]) as fp32 [B,H,T,T] (contiguous), from the qkv buffer and the lse that
+ * vitk_attn_fwd wrote — HF eager_attention_forward's attn_weights (modeling_vit.py:185-190).  Writes exactly B·H·T²
+ * floats and nothing else.  qkv 16-byte aligned; lse and probs 4-byte aligned. */
+VITK_API int vitk_attn_probs(const void* qkv_bf16, const float* lse, int64_t B, int64_t T, int64_t H, float scale,
+                             float* probs, vitk_stream_t stream);
 /* dqkv bf16 [B,T,3,H,64].  workspace: vitk_attn_bwd_workspace_bytes(B,T,H) bytes. */
 VITK_API size_t vitk_attn_bwd_workspace_bytes(int64_t B, int64_t T, int64_t H);
 VITK_API int vitk_attn_bwd(const void* qkv_bf16, const void* o_bf16, const void* do_bf16, const float* lse, int64_t B,
