@@ -19,6 +19,7 @@ EPI_ACCUM_F32 = 6
 EPI_STORE_F32 = 7
 EPI_BIAS_GELUG_BF16 = 8
 EPI_MUL_BF16 = 9
+EPI_UNPATCH_F32 = 10
 
 
 class GemmArgs(C.Structure):

@@ -158,6 +158,28 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, int row, int
   }
 }
 
+// VITK_EPI_UNPATCH_F32 (the input gradient, col2im of dh·Wp), in kernel instantiations of its own: a further case in
+// epilogue_chunk costs the existing instantiations 36-40 registers, even left unused.  Row = token t of image g; tokens
+// before row_off (CLS) carry no pixels.  Columns col0 … col0+31 are channel c, patch rows ky and ky+1
+// (k = c·256 + ky·16 + kx): two 64-byte runs of the NCHW image, whose width is ldd = 16·G.
+__device__ __forceinline__ void unpatch_chunk(const GemmParams& p, int row, int col0, const float (&v)[32]) {
+  if (row >= p.M) return;
+  const int g = row / p.rows_out;
+  const int t = row - g * p.rows_out - p.row_off;
+  if (t < 0) return;
+  const int G = static_cast<int>(p.ldd >> 4);
+  const int py = t / G, px = t - py * G;
+  const int c = col0 >> 8, ky = (col0 >> 4) & 15;
+  float4* o4 = reinterpret_cast<float4*>(reinterpret_cast<float*>(p.d) +
+                                         ((static_cast<long long>(g) * 3 + c) * p.ldd + py * 16 + ky) * p.ldd + px * 16);
+  const long long next = p.ldd >> 2;    // one image row, in float4
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    o4[i] = make_float4(v[4 * i + 0], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
+    o4[next + i] = make_float4(v[16 + 4 * i + 0], v[16 + 4 * i + 1], v[16 + 4 * i + 2], v[16 + 4 * i + 3]);
+  }
+}
+
 struct WorkItem {
   int m_blk, n_blk, kb_begin, kb_end;
 };
@@ -174,7 +196,7 @@ __device__ __forceinline__ WorkItem decode_work(const GemmParams& p, int w) {
   return it;
 }
 
-template <int BN, bool A_MN, bool B_MN>
+template <int BN, bool A_MN, bool B_MN, bool UNPATCH>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                  const GemmParams p) {
@@ -304,7 +326,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         float v[32];
 #pragma unroll
         for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-        epilogue_chunk(p, row, it.n_blk * BN + cc * 32, v);
+        if constexpr (UNPATCH) unpatch_chunk(p, row, it.n_blk * BN + cc * 32, v);
+        else epilogue_chunk(p, row, it.n_blk * BN + cc * 32, v);
       }
       tc_fence_before_sync();
       __syncwarp();
@@ -323,7 +346,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 }
 
 // ------------------------------------------------------------------------- host side
-template <int BN, bool A_MN, bool B_MN>
+template <int BN, bool A_MN, bool B_MN, bool UNPATCH>
 static int launch_gemm(const vitk_gemm_args& a, const GemmParams& p, int grid, cudaStream_t stream) {
   using Cfg = TileCfg<BN>;
   CUtensorMap ta, tb;
@@ -342,7 +365,7 @@ static int launch_gemm(const vitk_gemm_args& a, const GemmParams& p, int grid, c
     rc = make_tensor_map_bf16(&tb, a.b, 2, dims, str, box);
     if (rc) return rc;
   }
-  auto kern = gemm_bf16_kernel<BN, A_MN, B_MN>;
+  auto kern = gemm_bf16_kernel<BN, A_MN, B_MN, UNPATCH>;
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;
   std::call_once(once, [&] {
@@ -355,12 +378,12 @@ static int launch_gemm(const vitk_gemm_args& a, const GemmParams& p, int grid, c
   return 0;
 }
 
-template <int BN>
+template <int BN, bool UNPATCH>
 static int dispatch_major(const vitk_gemm_args& a, const GemmParams& p, int grid, cudaStream_t s) {
-  if (!a.a_mn_major && !a.b_mn_major) return launch_gemm<BN, false, false>(a, p, grid, s);
-  if (!a.a_mn_major && a.b_mn_major) return launch_gemm<BN, false, true>(a, p, grid, s);
-  if (a.a_mn_major && !a.b_mn_major) return launch_gemm<BN, true, false>(a, p, grid, s);
-  return launch_gemm<BN, true, true>(a, p, grid, s);
+  if (!a.a_mn_major && !a.b_mn_major) return launch_gemm<BN, false, false, UNPATCH>(a, p, grid, s);
+  if (!a.a_mn_major && a.b_mn_major) return launch_gemm<BN, false, true, UNPATCH>(a, p, grid, s);
+  if (a.a_mn_major && !a.b_mn_major) return launch_gemm<BN, true, false, UNPATCH>(a, p, grid, s);
+  return launch_gemm<BN, true, true, UNPATCH>(a, p, grid, s);
 }
 
 // Pick the N tile that wastes the fewest tile-slots in the last wave (cost ∝ waves × BN).
@@ -399,11 +422,27 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
   VITK_REQUIRE(a.lda % 8 == 0 && a.ldb % 8 == 0, VITK_EALIGN, "gemm: lda/ldb must be multiples of 8 elements");
   VITK_REQUIRE(a.lda >= (a.a_mn_major ? a.M : a.K) && a.ldb >= (a.b_mn_major ? a.N : a.K), VITK_EINVAL,
                "gemm: leading dimension smaller than the contiguous extent");
-  VITK_REQUIRE(a.epilogue >= 0 && a.epilogue <= VITK_EPI_MUL_BF16, VITK_EINVAL, "gemm: unknown epilogue %d", a.epilogue);
+  VITK_REQUIRE(a.epilogue >= 0 && a.epilogue <= VITK_EPI_UNPATCH_F32, VITK_EINVAL, "gemm: unknown epilogue %d", a.epilogue);
   const bool f32_out = a.epilogue == VITK_EPI_BIAS_RESID_F32 || a.epilogue == VITK_EPI_PATCH_F32 ||
                        a.epilogue == VITK_EPI_ACCUM_F32 || a.epilogue == VITK_EPI_STORE_F32;
-  VITK_REQUIRE(a.ldd % (f32_out ? 4 : 8) == 0 && a.ldd >= a.N, VITK_EALIGN, "gemm: ldd=%lld not aligned / too small",
-               (long long)a.ldd);
+  if (a.epilogue == VITK_EPI_UNPATCH_F32) {
+    // d is the fp32 NCHW image [M/rows_out, 3, 16·G, 16·G] of G×G patches; ldd is its width
+    VITK_REQUIRE(a.N == 768, VITK_EINVAL, "gemm: UNPATCH_F32 needs N = 768 (3 channels × 16 × 16), got N=%lld", (long long)a.N);
+    VITK_REQUIRE(a.row_off >= 0 && a.rows_out > a.row_off && a.rows_out < (1ll << 31), VITK_EINVAL,
+                 "gemm: UNPATCH_F32 needs rows_out > row_off >= 0 (rows_out=%lld, row_off=%lld)", (long long)a.rows_out,
+                 (long long)a.row_off);
+    const long long P = a.rows_out - a.row_off;
+    long long G = 0;
+    while ((G + 1) * (G + 1) <= P) ++G;
+    VITK_REQUIRE(G * G == P, VITK_EINVAL, "gemm: UNPATCH_F32 needs a square number of patches, got rows_out - row_off = %lld", P);
+    VITK_REQUIRE(a.ldd == 16 * G, VITK_EINVAL, "gemm: UNPATCH_F32 needs ldd = image width = 16·%lld, got ldd=%lld", G,
+                 (long long)a.ldd);
+    VITK_REQUIRE(a.M % a.rows_out == 0, VITK_EINVAL, "gemm: UNPATCH_F32 needs M %% rows_out == 0 (M=%lld, rows_out=%lld)",
+                 (long long)a.M, (long long)a.rows_out);
+  } else {
+    VITK_REQUIRE(a.ldd % (f32_out ? 4 : 8) == 0 && a.ldd >= a.N, VITK_EALIGN, "gemm: ldd=%lld not aligned / too small",
+                 (long long)a.ldd);
+  }
   if (a.epilogue == VITK_EPI_BIAS_GELU_BF16)
     VITK_REQUIRE(a.d2 != nullptr && aligned16(a.d2), VITK_EINVAL, "gemm: BIAS_GELU needs d2");
   if (a.epilogue == VITK_EPI_BIAS_GELUG_BF16 && a.d2 != nullptr)
@@ -456,9 +495,10 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
   int grid = p.total_work < sms ? p.total_work : sms;
   if (a.max_ctas > 0 && grid > a.max_ctas) grid = a.max_ctas;
 
+  const bool unpatch = a.epilogue == VITK_EPI_UNPATCH_F32;
   switch (bn) {
-    case 256: return dispatch_major<256>(a, p, grid, stream);
-    case 192: return dispatch_major<192>(a, p, grid, stream);
-    default: return dispatch_major<128>(a, p, grid, stream);
+    case 256: return unpatch ? dispatch_major<256, true>(a, p, grid, stream) : dispatch_major<256, false>(a, p, grid, stream);
+    case 192: return unpatch ? dispatch_major<192, true>(a, p, grid, stream) : dispatch_major<192, false>(a, p, grid, stream);
+    default: return unpatch ? dispatch_major<128, true>(a, p, grid, stream) : dispatch_major<128, false>(a, p, grid, stream);
   }
 }

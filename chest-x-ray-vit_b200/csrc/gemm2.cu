@@ -795,7 +795,7 @@ int gemm2_try_launch(const vitk_gemm_args& a, cudaStream_t stream, bool* handled
   *handled = false;
   if (a.variant == 1) return 0;
   const bool aux_epi = a.epilogue == VITK_EPI_BIAS_RESID_F32 || a.epilogue == VITK_EPI_MUL_BF16 || a.epilogue == VITK_EPI_DGELU_BF16;
-  const bool eligible = a.epilogue != VITK_EPI_PATCH_F32 && a.N % 128 == 0 && (a.max_ctas == 0 || a.max_ctas >= 2) &&
+  const bool eligible = a.epilogue != VITK_EPI_PATCH_F32 && a.epilogue != VITK_EPI_UNPATCH_F32 && a.N % 128 == 0 && (a.max_ctas == 0 || a.max_ctas >= 2) &&
                         !(aux_epi && a.a_mn_major) &&     // the aux instantiations exist for K-major A only
                         (a.tile_n == 0 || a.tile_n == 128 || a.tile_n == 192 || a.tile_n == 256) &&
                         !(a.tile_n == 192 && a.b_mn_major);

@@ -25,7 +25,7 @@ import torch
 
 from . import _lib, ops
 from ._lib import (EPI_ACCUM_F32, EPI_BIAS_BF16, EPI_BIAS_GELUG_BF16, EPI_BIAS_RESID_F32, EPI_MUL_BF16, EPI_PATCH_F32,
-                   EPI_STORE_BF16)
+                   EPI_STORE_BF16, EPI_UNPATCH_F32)
 
 bf16, f32 = torch.bfloat16, torch.float32
 
@@ -214,6 +214,8 @@ class Arena:
             self.dloss = new((1,), f32)
             self.dlogits_in = new((B, Cn), f32)
             self._bwd_plans: Dict[Tuple[bool, bool], _Plan] = {}
+            self._data_plans: Dict[bool, _Plan] = {}
+            self._sink: Optional[dict] = None
             self.bwd_loss = self.backward_plan(True, False)
             self.bwd_logits = self.backward_plan(False, False)
 
@@ -225,6 +227,26 @@ class Arena:
         if pl is None:
             eng = self._eng
             pl = self._bwd_plans[key] = self._build_backward(eng, from_loss, eng.g_stage() if staged else eng.g)
+        return pl
+
+    def data_backward_plan(self, from_loss: bool) -> _Plan:
+        """Launch plan of the backward pass that computes only the data gradients, down to ``dh[0]`` (the gradient of
+        the embeddings output), for a model none of whose parameters requires grad (built on first use).  It is the
+        backward plan without the weight-gradient GEMMs, the bias column sums, the embeddings backward, the side stream
+        and the gradient-sync points; it never touches a flat gradient buffer.  The parameter gradients the head and
+        LayerNorm entry points must still write go to a small scratch buffer, (C + 2)·D + C floats per arena."""
+        pl = self._data_plans.get(from_loss)
+        if pl is None:
+            eng = self._eng
+            if self._sink is None:
+                cfg = eng.cfg
+                D, Cn = cfg.hidden_size, cfg.num_labels
+                buf = torch.empty(((Cn + 2) * D + Cn,), dtype=f32, device=eng.dev)
+                gf, bf = buf[Cn * D:(Cn + 1) * D], buf[(Cn + 1) * D:(Cn + 2) * D]
+                layer = {"g1": gf, "b1": bf, "g2": gf, "b2": bf, "bo": None, "bf2": None}     # None: no bias column sum
+                self._sink = {"wc": buf[:Cn * D].view(Cn, D), "gf": gf, "bf": bf, "bc": buf[(Cn + 2) * D:],
+                              "layers": [layer] * cfg.num_hidden_layers}
+            pl = self._data_plans[from_loss] = self._build_backward(eng, from_loss, self._sink, data_only=True)
         return pl
 
     def outputs_plan(self, with_labels: bool) -> _Plan:
@@ -316,14 +338,16 @@ class Arena:
         return pl
 
     # ------------------------------------------------------------------ backward plan
-    def _build_backward(self, eng: "Engine", from_loss: bool, g: dict) -> _Plan:
+    def _build_backward(self, eng: "Engine", from_loss: bool, g: dict, data_only: bool = False) -> _Plan:
+        """data_only: leave out every launch that only produces parameter gradients (see data_backward_plan)."""
         cfg, w = eng.cfg, eng.w
         D, Fi, H, L, Cn = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.num_labels
         T, P, B, M = cfg.seq_len, cfg.num_patches, self.B, self.M
         scale = 64 ** -0.5
-        pl = _Plan(eng.side_stream)
+        wgrad = not data_only
+        pl = _Plan(eng.side_stream if wgrad else None)
         # one external-event sync point per gradient bucket (no host callback, no break in the CUDA graph)
-        ends = eng.grad_sync.bucket_end_layers() if eng.grad_sync is not None else set()
+        ends = eng.grad_sync.bucket_end_layers() if eng.grad_sync is not None and wgrad else set()
         done_hi = [L - 1]
 
         def layer_done(l):
@@ -348,16 +372,19 @@ class Arena:
         lw, lg, st = w["layers"][l], g["layers"][l], self.st[l]
         dh_c, dh1_c, dn_c, do_c = cls_rows(dh), cls_rows(dh1), cls_rows(self.dn), cls_rows(self.do)
         du_c, a_c, gp_c, n2_c, o_c = cls_rows(self.du), cls_rows(self.a[l]), cls_rows(self.gp[l]), cls_rows(self.n2[l]), cls_rows(self.o[l])
-        pl.gemm(dh_c, a_c, D, Fi, B, lg["w2"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-        pl.add("vitk_colsum_bf16", _p(dh_c), B, D, T * D, _p(lg["bf2"]))
+        if wgrad:
+            pl.gemm(dh_c, a_c, D, Fi, B, lg["w2"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+            pl.add("vitk_colsum_bf16", _p(dh_c), B, D, T * D, _p(lg["bf2"]))
         pl.gemm(dh_c, lw["w2_16"], B, Fi, D, du_c, EPI_MUL_BF16, b_mn_major=True, aux=gp_c)
-        pl.gemm(du_c, n2_c, Fi, D, B, lg["w1"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-        pl.add("vitk_colsum_bf16", _p(du_c), B, Fi, T * Fi, _p(lg["bf1"]))
+        if wgrad:
+            pl.gemm(du_c, n2_c, Fi, D, B, lg["w1"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+            pl.add("vitk_colsum_bf16", _p(du_c), B, Fi, T * Fi, _p(lg["bf1"]))
         pl.gemm(du_c, lw["w1_16"], B, D, Fi, dn_c, EPI_STORE_BF16, b_mn_major=True)
         pl.add("vitk_fill_zero", _p(dh1), dh1.numel() * 2)
         pl.add("vitk_layernorm_bwd_rows", _p(self.dn), _p(self.h1[l]), T * D, _p(st[2]), _p(st[3]), _p(lw["g2"]), _p(dh), B, D, T,
                _p(dh1), _p(lg["g2"]), _p(lg["b2"]), _p(lg["bo"]))
-        pl.gemm(dh1_c, o_c, D, D, B, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+        if wgrad:
+            pl.gemm(dh1_c, o_c, D, D, B, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
         if eng.cls_only_top:
             pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_cls_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale, _p(self.dqkv))
@@ -366,8 +393,9 @@ class Arena:
             pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale,
                    _p(self.dqkv), _p(self.attn_ws))
-        pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-        pl.add("vitk_colsum_bf16", _p(self.dqkv), M, 3 * D, 3 * D, _p(lg["bqkv"]))
+        if wgrad:
+            pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+            pl.add("vitk_colsum_bf16", _p(self.dqkv), M, 3 * D, 3 * D, _p(lg["bqkv"]))
         pl.gemm(self.dqkv, lw["wqkv16"], M, D, 3 * D, self.dn, EPI_STORE_BF16, b_mn_major=True)
         pl.add("vitk_layernorm_bwd", _p(self.dn), _p(self.h[l]), D, _p(st[0]), _p(st[1]), _p(lw["g1"]), _p(dh1), M, D,
                _p(dh), _p(lg["g1"]), _p(lg["b1"]), _p(g["layers"][l - 1]["bf2"]) if l > 0 else None)
@@ -380,41 +408,47 @@ class Arena:
         for l in reversed(range(L - 1)):
             lw, lg, st = w["layers"][l], g["layers"][l], self.st[l]
             # MLP
-            pl.fork()
-            pl.side(True)
-            pl.gemm(dh, self.a[l], D, Fi, M, lg["w2"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-            pl.side(False)
+            if wgrad:
+                pl.fork()
+                pl.side(True)
+                pl.gemm(dh, self.a[l], D, Fi, M, lg["w2"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+                pl.side(False)
             pl.gemm(dh, lw["w2_16"], M, Fi, D, self.du, EPI_MUL_BF16, b_mn_major=True, aux=self.gp[l])
-            pl.fork()
-            pl.side(True)
-            pl.gemm(self.du, self.n2[l], Fi, D, M, lg["w1"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-            pl.add("vitk_colsum_bf16", _p(self.du), M, Fi, Fi, _p(lg["bf1"]))
-            pl.side(False)
+            if wgrad:
+                pl.fork()
+                pl.side(True)
+                pl.gemm(self.du, self.n2[l], Fi, D, M, lg["w1"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+                pl.add("vitk_colsum_bf16", _p(self.du), M, Fi, Fi, _p(lg["bf1"]))
+                pl.side(False)
             pl.gemm(self.du, lw["w1_16"], M, D, Fi, self.dn, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_layernorm_bwd", _p(self.dn), _p(self.h1[l]), D, _p(st[2]), _p(st[3]), _p(lw["g2"]), _p(dh), M, D,
                    _p(dh1), _p(lg["g2"]), _p(lg["b2"]), _p(lg["bo"]))
             # attention
-            pl.fork()
-            pl.side(True)
-            pl.gemm(dh1, self.o[l], D, D, M, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-            pl.side(False)
+            if wgrad:
+                pl.fork()
+                pl.side(True)
+                pl.gemm(dh1, self.o[l], D, D, M, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+                pl.side(False)
             pl.gemm(dh1, lw["wo16"], M, D, D, self.do, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale,
                    _p(self.dqkv), _p(self.attn_ws))
-            pl.fork()
-            pl.side(True)
-            pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-            pl.add("vitk_colsum_bf16", _p(self.dqkv), M, 3 * D, 3 * D, _p(lg["bqkv"]))
-            pl.side(False)
+            if wgrad:
+                pl.fork()
+                pl.side(True)
+                pl.gemm(self.dqkv, self.n1[l], 3 * D, D, M, lg["wqkv"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+                pl.add("vitk_colsum_bf16", _p(self.dqkv), M, 3 * D, 3 * D, _p(lg["bqkv"]))
+                pl.side(False)
             pl.gemm(self.dqkv, lw["wqkv16"], M, D, 3 * D, self.dn, EPI_STORE_BF16, b_mn_major=True)
-            pl.join()          # side work of this layer read dh / du / dh1 / dqkv, which the next kernels overwrite
+            if wgrad:
+                pl.join()      # side work of this layer read dh / du / dh1 / dqkv, which the next kernels overwrite
             pl.add("vitk_layernorm_bwd", _p(self.dn), _p(self.h[l]), D, _p(st[0]), _p(st[1]), _p(lw["g1"]), _p(dh1), M, D,
                    _p(dh), _p(lg["g1"]), _p(lg["b1"]), _p(g["layers"][l - 1]["bf2"]) if l > 0 else None)
             layer_done(l)
-        pl.add("vitk_embed_bwd", _p(dh), B, T, D, _p(g["pos"]), _p(g["cls"]), _p(g["bp"]), _p(self.dpatch))
-        pl.gemm(self.dpatch, self.apatch, D, 768, B * P, g["wp"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-        if eng.grad_sync is not None:
-            pl.sync_point(lambda ev: eng._rest_grads_ready(ev))
+        if wgrad:
+            pl.add("vitk_embed_bwd", _p(dh), B, T, D, _p(g["pos"]), _p(g["cls"]), _p(g["bp"]), _p(self.dpatch))
+            pl.gemm(self.dpatch, self.apatch, D, 768, B * P, g["wp"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
+            if eng.grad_sync is not None:
+                pl.sync_point(lambda ev: eng._rest_grads_ready(ev))
         return pl
 
 
@@ -543,46 +577,72 @@ class Engine:
                 p.grad = gv
 
     def backward(self, ticket: int, dloss: Optional[torch.Tensor], dlogits: Optional[torch.Tensor],
-                 needs: Optional[Tuple[bool, ...]] = None) -> tuple:
-        """Runs the backward launch plan and returns one gradient per parameter (HF order; None where ``needs`` is
-        False): fresh views of the flat buffer the kernels wrote.  If no ``param.grad`` is populated the main flat
-        buffer is used (autograd adopts the views, no copy); otherwise — gradient accumulation — the kernels write the
-        staging buffer and autograd adds it onto ``param.grad``."""
+                 needs: Optional[Tuple[bool, ...]] = None, input_grad: bool = False) -> Tuple[tuple, Optional[torch.Tensor]]:
+        """Runs the backward launch plan and returns (one gradient per parameter (HF order; None where ``needs`` is
+        False), the gradient of ``pixel_values`` or None).  The parameter gradients are fresh views of the flat buffer the
+        kernels wrote.  If no ``param.grad`` is populated the main flat buffer is used (autograd adopts the views, no
+        copy); otherwise — gradient accumulation — the kernels write the staging buffer and autograd adds it onto
+        ``param.grad``.  When no parameter needs a gradient and ``input_grad`` is set, the arena's data-only plan runs
+        instead: no weight-gradient work, no flat gradient buffer and no gradient sync.  With ``input_grad`` the input
+        gradient fp32 [B, 3, S, S] is one UNPATCH_F32 GEMM from the final ``dh`` into a fresh tensor."""
         ar = next((a for a in self.arenas.values() if a.train and a.ticket == ticket), None)
         if ar is None:
             raise RuntimeError("chest_x_ray_vit_b200: the activations of this forward were overwritten by a later "
                                "forward with the same batch size; call backward() before the next forward()")
         n = len(self._plist)
         if dloss is None and dlogits is None:
-            return (None,) * n
-        model = self.model
-        staged = any(p.grad is not None for p in self._plist)
-        if staged:
-            flat = model.stage_grads()
-            ops.fill_zero(flat)
+            return (None,) * n, None
+        if needs is None:
+            needs = (True,) * n
+        data_only = input_grad and not any(needs)
+        if data_only:
+            plan_for = ar.data_backward_plan
         else:
-            flat = model.flat_grads()
-            if not model._grads_clean:
+            model = self.model
+            staged = any(p.grad is not None for p in self._plist)
+            if staged:
+                flat = model.stage_grads()
                 ops.fill_zero(flat)
-            model._grads_clean = False
-        if self.grad_sync is not None:
-            self.grad_sync.begin(flat)
+            else:
+                flat = model.flat_grads()
+                if not model._grads_clean:
+                    ops.fill_zero(flat)
+                model._grads_clean = False
+            if self.grad_sync is not None:
+                self.grad_sync.begin(flat)
+
+            def plan_for(from_loss: bool) -> _Plan:
+                return ar.backward_plan(from_loss, staged)
         stream = torch.cuda.current_stream().cuda_stream
+        callbacks = self.grad_sync is not None and not data_only
         if dloss is not None and dlogits is None:
             ar.dloss.copy_(dloss.reshape(1), non_blocking=True)
-            ar.backward_plan(True, staged).run(stream, callbacks=self.grad_sync is not None)
+            plan_for(True).run(stream, callbacks=callbacks)
         else:
             if dloss is not None:      # both the loss and the logits were used downstream
                 torch.add(dlogits.to(f32), ar.dlogits * dloss.to(f32), out=ar.dlogits_in)
             else:
                 ar.dlogits_in.copy_(dlogits)
-            ar.backward_plan(False, staged).run(stream, callbacks=self.grad_sync is not None)
+            plan_for(False).run(stream, callbacks=callbacks)
+        dx = self._input_grad(ar) if input_grad else None
         ar.ticket = -1
-        if needs is None:
-            needs = (True,) * n
+        if data_only:
+            return (None,) * n, dx
         chunks = flat.split_with_sizes(self._split_sizes)
         return tuple((chunks[i].view(sh) if chunks[i].numel() == k else chunks[i][:k].view(sh)) if nd else None
-                     for (i, k, sh), nd in zip(self._spans, needs))
+                     for (i, k, sh), nd in zip(self._spans, needs)), dx
+
+    def _input_grad(self, ar: Arena) -> torch.Tensor:
+        """d loss / d pixel_values = col2im(dh[:, 1:] · Wp): the final ``dh`` (layer 0's LayerNorm backward wrote it) times
+        the bf16 patch weight [D, 768], scattered into a fresh fp32 [B, 3, S, S] tensor by the UNPATCH_F32 epilogue.
+        vitk_patchify_f32 only reorders and rounds its input, so this is the gradient of the fp32 pixels as passed.
+        Fresh because autograd adopts it as ``x.grad`` without a copy."""
+        cfg = self.cfg
+        S = cfg.image_size
+        dx = torch.empty((ar.B, 3, S, S), dtype=f32, device=self.dev)
+        ops.gemm(ar.dh[0], self.w["wp16"], ar.M, 768, cfg.hidden_size, dx, epilogue=EPI_UNPATCH_F32, b_mn_major=True,
+                 ldd=S, rows_out=cfg.seq_len, row_off=1)
+        return dx
 
     def _layers_grads_ready(self, lo: int, hi: int, ev=None) -> None:
         if self.grad_sync is not None:

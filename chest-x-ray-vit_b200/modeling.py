@@ -7,6 +7,7 @@ transformers/models/vit/modeling_vit.py:605-653 (HF 5.5.0):
     model = ViTForImageClassification(config)            # same parameter names / shapes as HF
     out = model(pixel_values=x, labels=y)                # ImageClassifierOutput(loss, logits)
     out.loss.backward(); optimizer.step()                # fp32 grads land in param.grad
+    x.requires_grad_(); model(pixel_values=x).logits[:, c].sum().backward()   # x.grad: saliency / attribution
     out = model(pixel_values=x, output_attentions=True,  # + hidden_states (L+1 × [B,T,D]) and attentions
               output_hidden_states=True)                 #   (L × [B,H,T,T]), as HF's eager attention returns them
 
@@ -386,7 +387,13 @@ class ViTForImageClassification(nn.Module):
         a tuple of L fp32 [B,H,T,T] softmax probabilities per layer, what HF's ``eager`` attention returns (HF's default
         ``sdpa`` attention returns an empty tuple there).  Both are fresh tensors outside autograd
         (``requires_grad=False``): ``loss.backward()`` gives the same gradients as without them, and no gradient flows
-        through them.  Requesting either runs the top encoder layer on every token instead of the CLS rows alone."""
+        through them.  Requesting either runs the top encoder layer on every token instead of the CLS rows alone.
+
+        Gradients reach a floating-point ``pixel_values`` that requires grad, as in HF: ``x.grad`` is the gradient with
+        respect to ``pixel_values`` as passed (for the collate_fn contract, the normalised image), in its dtype and on its
+        device — saliency maps, SmoothGrad, Integrated Gradients.  With every parameter frozen
+        (``model.requires_grad_(False)``) backward computes only that gradient: no weight gradients, no ``param.grad``,
+        no data-parallel gradient sync.  uint8 input cannot require grad (torch forbids it)."""
         if pixel_values is None:
             raise ValueError("You have to specify pixel_values")                               # HF:440-441
         if interpolate_pos_encoding:
@@ -398,7 +405,8 @@ class ViTForImageClassification(nn.Module):
         eng = self.engine()
         if labels is not None and cfg.problem_type is None:
             cfg.problem_type = "multi_label_classification"     # HF loss_utils.py:92-98 (float labels)
-        need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in self.param_list())
+        need_grad = torch.is_grad_enabled() and (any(p.requires_grad for p in self.param_list()) or
+                                                 (pixel_values.is_floating_point() and pixel_values.requires_grad))
         extras = {"attentions": want_attn, "hidden_states": want_hidden}
         if need_grad:
             loss, logits = _VitFunction.apply(self, pixel_values, labels, extras, *self.param_list())
@@ -417,8 +425,9 @@ class _VitFunction(torch.autograd.Function):
     reducer all see what they expect.  The returned gradients are views of one flat fp32 buffer the kernels wrote:
     when ``param.grad`` is None autograd adopts the view without a copy, so the optimizer still finds all gradients
     contiguous; when ``param.grad`` is already populated (gradient accumulation) the kernels write a second buffer
-    and autograd adds it in place.  Requested hidden states / attention maps leave through ``extras["out"]``, outside
-    autograd."""
+    and autograd adds it in place.  ``pixel_values`` gets its gradient when it requires one (a fresh tensor: the
+    engine's input-gradient GEMM allocates it).  Requested hidden states / attention maps leave through
+    ``extras["out"]``, outside autograd."""
 
     @staticmethod
     def forward(ctx, model: ViTForImageClassification, pixel_values, labels, extras, *params):
@@ -429,6 +438,7 @@ class _VitFunction(torch.autograd.Function):
         ctx.model = model
         ctx.ticket = eng.ticket
         ctx.has_labels = labels is not None
+        ctx.x_dtype, ctx.x_device = pixel_values.dtype, pixel_values.device
         ctx.set_materialize_grads(False)
         if loss is None:
             loss = logits.new_zeros(())
@@ -437,5 +447,8 @@ class _VitFunction(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dloss, dlogits):
         model = ctx.model
-        grads = model.engine().backward(ctx.ticket, dloss if ctx.has_labels else None, dlogits, ctx.needs_input_grad[4:])
-        return (None, None, None, None) + grads
+        grads, dx = model.engine().backward(ctx.ticket, dloss if ctx.has_labels else None, dlogits, ctx.needs_input_grad[4:],
+                                            input_grad=ctx.needs_input_grad[1])
+        if dx is not None and (dx.dtype != ctx.x_dtype or dx.device != ctx.x_device):
+            dx = dx.to(device=ctx.x_device, dtype=ctx.x_dtype)
+        return (None, dx, None, None) + grads

@@ -14,7 +14,8 @@ import torch
 
 from . import _lib
 from ._lib import (EPI_ACCUM_F32, EPI_BIAS_BF16, EPI_BIAS_GELU_BF16, EPI_BIAS_GELUG_BF16, EPI_BIAS_RESID_F32,  # noqa: F401
-                   EPI_DGELU_BF16, EPI_MUL_BF16, EPI_PATCH_F32, EPI_STORE_BF16, EPI_STORE_F32, GemmArgs)
+                   EPI_DGELU_BF16, EPI_MUL_BF16, EPI_PATCH_F32, EPI_STORE_BF16, EPI_STORE_F32, EPI_UNPATCH_F32,
+                   GemmArgs)
 
 bf16, f32 = torch.bfloat16, torch.float32
 

@@ -106,7 +106,13 @@ enum vitk_epilogue {
   VITK_EPI_ACCUM_F32 = 6,       /* d f32 += acc (red.global.add; split-K allowed) (wgrad)  */
   VITK_EPI_STORE_F32 = 7,       /* d f32 = acc                                             */
   VITK_EPI_BIAS_GELUG_BF16 = 8, /* u = acc + bias; d bf16 = gelu_erf(u); d2 bf16 (optional) = gelu_erf'(u)  (fc1, training) */
-  VITK_EPI_MUL_BF16 = 9         /* d bf16 = acc * aux_bf16[m,n]                  (fc2 dgrad with saved gelu') */
+  VITK_EPI_MUL_BF16 = 9,        /* d bf16 = acc * aux_bf16[m,n]                  (fc2 dgrad with saved gelu') */
+  VITK_EPI_UNPATCH_F32 = 10     /* inverse of PATCH_F32 (input gradient, col2im of dh·Wp): row m is token
+                                   t = m % rows_out of image g = m / rows_out; rows with t < row_off are dropped, patch
+                                   q = t − row_off sits at (q / G, q % G) with G² = rows_out − row_off; column
+                                   n = c·256 + ky·16 + kx goes to d f32 [g, c, 16·(q/G) + ky, 16·(q%G) + kx] of the NCHW
+                                   image [M/rows_out, 3, 16G, 16G].  N = 768, ldd = 16G (the image width),
+                                   M % rows_out == 0; no bias, no aux; every element of d written exactly once */
 };
 
 typedef struct vitk_gemm_args {
@@ -127,7 +133,7 @@ typedef struct vitk_gemm_args {
   int32_t tile_n;        /* 0 = library chooses; else 128, 192 or 256 */
   int32_t max_ctas;      /* 0 = all SMs; else cap on the persistent grid, leaving SMs to a concurrent collective */
   int32_t variant;       /* 0 = library chooses; 1 = single-CTA 128×N tiles (gemm.cu); 2 = CTA pair,
-                            256×N tiles, TMA-store epilogue (gemm2.cu; not for VITK_EPI_PATCH_F32); 3 = as 2 but
+                            256×N tiles, TMA-store epilogue (gemm2.cu; not for VITK_EPI_PATCH_F32 / UNPATCH_F32); 3 = as 2 but
                             always with 8 epilogue warps (the A/B reference of the 16-warp heavy-epilogue
                             instantiations, which produce the same bits) */
 } vitk_gemm_args;
