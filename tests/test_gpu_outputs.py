@@ -45,7 +45,7 @@ def _check_rows(p):
     assert (p.sum(-1) - 1).abs().max() <= 1e-3
 
 
-# the shapes of test_gpu_attention.py: T from 17 to 1024, H up to 20, and the benchmarked B = 16 at T = 577
+# shapes like test_gpu_attention.py's: T from 17 to 1024, H up to 20, and the benchmarked B = 16 at T = 577
 @pytest.mark.parametrize("B,T,H", [(1, 128, 1), (1, 64, 2), (2, 17, 2), (2, 129, 3), (2, 197, 12), (1, 256, 2), (2, 577, 12),
                                    (1, 300, 16), (1, 385, 2), (1, 640, 2), (1, 1024, 1), (16, 577, 12),
                                    (1, 130, 6), (1, 70, 20), (2, 129, 20)])
