@@ -72,8 +72,7 @@ _PROTOS = {
     "vitk_shard_mean": (C.c_int, [_p, _p, _i64, _i64, C.c_int, _f, C.c_int, _p]),
     "vitk_clip_scale": (C.c_int, [_p, _f, _p, _p]),
     "vitk_launch_count": (C.c_int64, []),
-    "vitk_gemm_plan": (C.c_int, [C.POINTER(GemmArgs), C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
-                                 C.POINTER(C.c_int)]),
+    "vitk_gemm_plan": (C.c_int, [C.POINTER(GemmArgs), C.c_int] + [C.POINTER(C.c_int)] * 6),
     "vitk_debug_timeline": (C.c_int, [_p]),
     "vitk_debug_stamp": (C.c_int, [C.c_int64, _p]),
 }

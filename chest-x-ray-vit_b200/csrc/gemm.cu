@@ -16,8 +16,8 @@
 
 #include "common.cuh"
 #include "gemm_epilogue.cuh"
+#include "gemm_host.cuh"
 #include "sm100_prims.cuh"
-#include "tmap.cuh"
 
 namespace vitk {
 
@@ -350,21 +350,8 @@ template <int BN, bool A_MN, bool B_MN, bool UNPATCH>
 static int launch_gemm(const vitk_gemm_args& a, const GemmParams& p, int grid, cudaStream_t stream) {
   using Cfg = TileCfg<BN>;
   CUtensorMap ta, tb;
-  {
-    // A: K-major → dims {K, M}, box {64, 128};  MN-major → dims {M, K}, box {64, 64}
-    uint64_t dims[2], str[1];
-    uint32_t box[2];
-    if (!A_MN) { dims[0] = a.K; dims[1] = a.M; box[0] = kBK; box[1] = kBM; }
-    else       { dims[0] = a.M; dims[1] = a.K; box[0] = 64;  box[1] = kBK; }
-    str[0] = static_cast<uint64_t>(a.lda) * 2;
-    int rc = make_tensor_map_bf16(&ta, a.a, 2, dims, str, box);
-    if (rc) return rc;
-    if (!B_MN) { dims[0] = a.K; dims[1] = a.N; box[0] = kBK; box[1] = BN; }
-    else       { dims[0] = a.N; dims[1] = a.K; box[0] = 64;  box[1] = kBK; }
-    str[0] = static_cast<uint64_t>(a.ldb) * 2;
-    rc = make_tensor_map_bf16(&tb, a.b, 2, dims, str, box);
-    if (rc) return rc;
-  }
+  if (int rc = operand_map(&ta, a.a, A_MN, a.M, a.K, a.lda, kBM)) return rc;
+  if (int rc = operand_map(&tb, a.b, B_MN, a.N, a.K, a.ldb, BN)) return rc;
   auto kern = gemm_bf16_kernel<BN, A_MN, B_MN, UNPATCH>;
   static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;
@@ -386,7 +373,10 @@ static int dispatch_major(const vitk_gemm_args& a, const GemmParams& p, int grid
   return launch_gemm<BN, true, true, UNPATCH>(a, p, grid, s);
 }
 
-// Pick the N tile that wastes the fewest tile-slots in the last wave (cost ∝ waves × BN).
+// ------------------------------------------------------------------------- launch planning
+// Both kernels use 128-row CTA tiles and 64-wide K blocks (kBM, kBK); the pair kernel's tiles are 256-row bands.
+
+// Single-CTA kernel: the N tile that wastes the fewest tile-slots in the last wave (cost ∝ waves × BN).
 static int choose_tile_n(long long M, long long N, int sms) {
   const long long mt = (M + kBM - 1) / kBM;
   int best = 128;
@@ -403,16 +393,90 @@ static int choose_tile_n(long long M, long long N, int sms) {
   return best;
 }
 
-int gemm2_try_launch(const vitk_gemm_args& a, cudaStream_t stream, bool* handled);   // gemm2.cu
+// cycles a CTA pair spends per 64-wide K block of a tile of `bn` columns (tools/gemm_timeline.py, B200): the MMAs of a
+// 256-wide tile occupy the tensor pipe for 4 × 122 cycles; narrower tiles are bound by operand delivery instead.
+// 192: A/B on the full step, 440 (192-wide tiles for K-major N = 768) beats 500 (mixed 256+128 there) by 0.9 %.
+static double kblock_cycles(int bn) { return bn == 256 ? 500.0 : (bn == 192 ? 440.0 : 390.0); }
+constexpr double kTileFixedCycles = 1500.0;   // accumulator hand-over + pipeline refill per tile
 
-}  // namespace vitk
+// CTA-pair kernel: tile width, split count and half-width tiles per band with the lowest modelled cost (bn = 0 when
+// no width fits N and tile_n).
+static void choose_tiling2(const vitk_gemm_args& a, int pairs, int* bn_out, int* splits_out, int* n_half_out,
+                           double* cost_out) {
+  const long long mt = (a.M + 2 * kBM - 1) / (2 * kBM);
+  const long long kb_total = (a.K + kBK - 1) / kBK;
+  double best = 1e30;
+  const int cands[3] = {256, 192, 128};
+  for (int bn : cands) {
+    if (a.N % bn) continue;
+    if (a.b_mn_major && bn == 192) continue;
+    if (a.tile_n && a.tile_n != bn) continue;
+    const long long tiles = mt * (a.N / bn);
+    int splits = 1;
+    if (a.epilogue == VITK_EPI_ACCUM_F32) {
+      if (a.split_k > 0) splits = a.split_k;
+      else if (tiles < pairs) {
+        splits = static_cast<int>(pairs / tiles);
+        const long long cap = kb_total / 4 > 0 ? kb_total / 4 : 1;
+        if (splits > cap) splits = static_cast<int>(cap);
+        if (splits < 1) splits = 1;
+      }
+    }
+    const long long kb_per = (kb_total + splits - 1) / splits;
+    const long long items = tiles * ((kb_total + kb_per - 1) / kb_per);
+    const long long waves = (items + pairs - 1) / pairs;
+    const double cost = static_cast<double>(waves) * (kb_per * kblock_cycles(bn) + kTileFixedCycles);
+    if (cost < best - 1e-9) { best = cost; *bn_out = bn; *splits_out = splits; *n_half_out = 0; }
+    // Mixed widths (BN = 256 only): replace some of each band's 256-column tiles by pairs of 128-column tiles so that
+    // the static round-robin order gives every CTA pair the same amount of work (e.g. N = 768 on 74 pairs: 3 full
+    // tiles per band = 1.5 waves of full tiles; 2 full + 2 half = one full and one half tile for every pair).
+    if (bn == 256 && splits == 1 && a.epilogue != VITK_EPI_ACCUM_F32 && a.tile_n == 0) {
+      const int n_tiles256 = static_cast<int>(a.N / 256);
+      const double cf = kb_total * kblock_cycles(256) + kTileFixedCycles, ch = kb_total * kblock_cycles(128) + kTileFixedCycles;
+      for (int nh = 2; nh <= 2 * n_tiles256; nh += 2) {
+        const int nf = n_tiles256 - nh / 2;
+        const long long full_items = mt * nf, all_items = mt * (nf + nh);
+        double worst = 0;
+        for (int pr = 0; pr < pairs && pr < all_items; ++pr) {
+          double c = 0;
+          for (long long w = pr; w < all_items; w += pairs) c += w < full_items ? cf : ch;
+          if (c > worst) worst = c;
+        }
+        if (worst < best - 1e-9) { best = worst; *bn_out = 256; *splits_out = 1; *n_half_out = nh; }
+      }
+    }
+  }
+  *cost_out = best;
+}
 
-using namespace vitk;
+// Data-gradient GEMMs (K-major A, MN-major B, plain bf16 store) whose M is ragged against the pair kernel's 256-row bands
+// can quantise badly on 74 pairs yet perfectly on 148 single CTAs with 128-row bands — ViT-L at batch 8: M = 4616 → 19
+// bands × 4 tiles of 256 columns = 76 tiles (two pairs get a second tile) against 37 × 4 = 148 tiles = exactly one wave.
+// Measured there (tools/bench_gemm.py, VITK_BG_M=4616 VITK_BG_D=1024 VITK_BG_F=4096): fc1 dgrad 43.2 → 35.7 µs,
+// qkv dgrad 35.8 → 28.8 µs, out dgrad 19.5 → 16.5 µs.  Per K block a single CTA (which stages the whole B tile itself)
+// costs ≈ 1.1 × the pair kernel's 256-wide block for this operand layout.  The cost is that of 256-wide single-CTA
+// tiles; the launch then takes choose_tile_n's width, which is 256 for the model's shapes but can be 128 for others.
+static bool single_cta_wins(const vitk_gemm_args& a, double pair_cost, int sms) {
+  if (a.variant != 0 || a.tile_n != 0 || a.max_ctas != 0 || a.a_mn_major || !a.b_mn_major || a.epilogue != VITK_EPI_STORE_BF16 ||
+      a.N % 256 != 0)
+    return false;
+  const long long tiles = ((a.M + 127) / 128) * (a.N / 256);
+  const long long waves = (tiles + sms - 1) / sms;
+  const long long kb = (a.K + kBK - 1) / kBK;
+  const double cost = static_cast<double>(waves) * (kb * 1.1 * kblock_cycles(256) + kTileFixedCycles);
+  return cost < 0.9 * pair_cost;
+}
 
-extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t stream_) {
-  VITK_REQUIRE(args != nullptr, VITK_EINVAL, "gemm: args is NULL");
-  const vitk_gemm_args& a = *args;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+// K blocks per split and work items once mn_tiles and kb_total are set; the split count is clamped to the K blocks
+// and every split is non-empty.
+static void set_splits(GemmPlan* p, int splits) {
+  if (splits > p->kb_total) splits = p->kb_total;
+  p->kb_per_split = (p->kb_total + splits - 1) / splits;
+  p->k_splits = (p->kb_total + p->kb_per_split - 1) / p->kb_per_split;
+  p->total_work = p->mn_tiles * p->k_splits;
+}
+
+int plan_gemm(const vitk_gemm_args& a, int sms, GemmPlan* out) {
   VITK_REQUIRE(a.M > 0 && a.N > 0 && a.K > 0, VITK_EINVAL, "gemm: M,N,K must be positive (%lld,%lld,%lld)",
                (long long)a.M, (long long)a.N, (long long)a.K);
   VITK_REQUIRE(a.M < (1ll << 31) && a.N < (1ll << 31) && a.K < (1ll << 31), VITK_EINVAL, "gemm: dims exceed int32");
@@ -423,8 +487,7 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
   VITK_REQUIRE(a.lda >= (a.a_mn_major ? a.M : a.K) && a.ldb >= (a.b_mn_major ? a.N : a.K), VITK_EINVAL,
                "gemm: leading dimension smaller than the contiguous extent");
   VITK_REQUIRE(a.epilogue >= 0 && a.epilogue <= VITK_EPI_UNPATCH_F32, VITK_EINVAL, "gemm: unknown epilogue %d", a.epilogue);
-  const bool f32_out = a.epilogue == VITK_EPI_BIAS_RESID_F32 || a.epilogue == VITK_EPI_PATCH_F32 ||
-                       a.epilogue == VITK_EPI_ACCUM_F32 || a.epilogue == VITK_EPI_STORE_F32;
+  const EpiTraits& epi = kEpiTraits[a.epilogue];
   if (a.epilogue == VITK_EPI_UNPATCH_F32) {
     // d is the fp32 NCHW image [M/rows_out, 3, 16·G, 16·G] of G×G patches; ldd is its width
     VITK_REQUIRE(a.N == 768, VITK_EINVAL, "gemm: UNPATCH_F32 needs N = 768 (3 channels × 16 × 16), got N=%lld", (long long)a.N);
@@ -440,7 +503,7 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
     VITK_REQUIRE(a.M % a.rows_out == 0, VITK_EINVAL, "gemm: UNPATCH_F32 needs M %% rows_out == 0 (M=%lld, rows_out=%lld)",
                  (long long)a.M, (long long)a.rows_out);
   } else {
-    VITK_REQUIRE(a.ldd % (f32_out ? 4 : 8) == 0 && a.ldd >= a.N, VITK_EALIGN, "gemm: ldd=%lld not aligned / too small",
+    VITK_REQUIRE(a.ldd % (epi.f32_out ? 4 : 8) == 0 && a.ldd >= a.N, VITK_EALIGN, "gemm: ldd=%lld not aligned / too small",
                  (long long)a.ldd);
   }
   if (a.epilogue == VITK_EPI_BIAS_GELU_BF16)
@@ -448,8 +511,7 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
   if (a.epilogue == VITK_EPI_BIAS_GELUG_BF16 && a.d2 != nullptr)
     VITK_REQUIRE(aligned16(a.d2), VITK_EALIGN, "gemm: d2 must be 16-byte aligned");
   VITK_REQUIRE(a.variant >= 0 && a.variant <= 3, VITK_EINVAL, "gemm: variant must be 0 (auto), 1 (single-CTA), 2 (CTA pair) or 3 (CTA pair, 8 epilogue warps)");
-  if (a.epilogue == VITK_EPI_BIAS_RESID_F32 || a.epilogue == VITK_EPI_PATCH_F32 || a.epilogue == VITK_EPI_DGELU_BF16 ||
-      a.epilogue == VITK_EPI_MUL_BF16)
+  if (epi.aux)
     VITK_REQUIRE(a.aux != nullptr && aligned16(a.aux) && a.ld_aux % 8 == 0 && a.ld_aux >= a.N, VITK_EINVAL,
                  "gemm: epilogue %d needs aux with ld_aux >= N, multiple of 8", a.epilogue);
   if (a.epilogue == VITK_EPI_PATCH_F32)
@@ -459,23 +521,56 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
   VITK_REQUIRE(a.split_k >= 0 && (a.split_k <= 1 || a.epilogue == VITK_EPI_ACCUM_F32), VITK_EINVAL,
                "gemm: split_k > 1 requires VITK_EPI_ACCUM_F32");
 
-  {
-    bool handled = false;
-    const int rc = gemm2_try_launch(a, stream, &handled);
-    if (rc != 0 || handled) return rc;
+  GemmPlan& p = *out;
+  p.kb_total = static_cast<int>((a.K + kBK - 1) / kBK);
+
+  // The CTA-pair kernel wherever it applies (variant 0, 2, 3), unless the single-CTA kernel quantises better.
+  if (a.variant != 1) {
+    const bool eligible = epi.pair && (a.max_ctas == 0 || a.max_ctas >= 2) &&
+                          !(epi.aux && a.a_mn_major) &&     // the aux instantiations exist for K-major A only
+                          (a.tile_n == 0 || a.tile_n == 128 || a.tile_n == 192 || a.tile_n == 256) &&
+                          !(a.tile_n == 192 && a.b_mn_major);
+    VITK_REQUIRE(eligible || a.variant < 2, VITK_EINVAL,
+                 "gemm: the CTA-pair kernel does not support this problem (epilogue %d, tile_n %d)", a.epilogue, a.tile_n);
+    // max_ctas leaves SMs free for a concurrent NCCL all-reduce (tile choice then balances waves over fewer pairs)
+    const int pairs = (a.max_ctas > 0 && a.max_ctas < sms ? a.max_ctas : sms) / 2;
+    int bn = 0, splits = 1, n_half = 0;
+    double pair_cost = 0;
+    if (eligible) {
+      choose_tiling2(a, pairs, &bn, &splits, &n_half, &pair_cost);
+      VITK_REQUIRE(bn != 0 || a.variant < 2, VITK_EINVAL, "gemm: no CTA-pair tiling for N=%lld tile_n=%d", (long long)a.N,
+                   a.tile_n);
+    }
+    if (bn != 0 && !single_cta_wins(a, pair_cost, sms)) {
+      // fc1 forward (+bias, GELU, optional GELU') runs on 16 epilogue warps with the epilogue fixed at compile time
+      // (see the pair kernel's template comment): 2 MUFU + 13 FP32 operations per element are a chain of dependent
+      // latencies that four warps per scheduler hide better than two — 51.4 → 47.1 µs at M = 9232
+      // (profiles/r02_bench_gemm_ew16.txt), bit-identical output (tests/test_gpu_gemm.py::
+      // test_sixteen_warp_epilogues_equal_eight_warp).  The same treatment of the multiplier and fp32-residual
+      // epilogues was measured and dropped: those launches move 128 / 71 MB for 43.6 / 10.9 GF and sit on the HBM side
+      // of the roofline, not on the epilogue's instruction latency (no change at 49.2 / 28.7 / 47.1 µs).  Variant 3
+      // keeps 8 warps (the reference the 16-warp instantiation is tested against).
+      const bool ew16 = a.variant != 3 && a.epilogue == VITK_EPI_BIAS_GELUG_BF16 && !a.a_mn_major && !a.b_mn_major && bn == 256;
+      p.kernel = ew16 ? GEMM_PAIR_EW16 : GEMM_PAIR;
+      p.bn = bn;
+      p.n_half = n_half;
+      p.n_tiles = static_cast<int>(a.N / bn) - n_half / 2 + n_half;
+      p.mn_tiles = static_cast<int>((a.M + 2 * kBM - 1) / (2 * kBM)) * p.n_tiles;
+      set_splits(&p, splits);
+      p.ctas = 2 * (p.total_work < pairs ? p.total_work : pairs);
+      return 0;
+    }
   }
 
-  const int sms = num_sms();
-  int bn = a.tile_n ? a.tile_n : choose_tile_n(a.M, a.N, sms);
+  // The single-CTA kernel: variant 1, the epilogues and operand layouts the pair kernel lacks, and ragged data gradients.
+  const int bn = a.tile_n ? a.tile_n : choose_tile_n(a.M, a.N, sms);
   VITK_REQUIRE((bn == 128 || bn == 192 || bn == 256) && a.N % bn == 0, VITK_EINVAL, "gemm: tile_n=%d invalid for N=%lld",
                bn, (long long)a.N);
-
-  GemmParams p;
-  p.M = static_cast<int>(a.M); p.N = static_cast<int>(a.N); p.K = static_cast<int>(a.K);
-  const int m_tiles = (p.M + kBM - 1) / kBM;
-  p.n_tiles = p.N / bn;
-  p.mn_tiles = m_tiles * p.n_tiles;
-  p.kb_total = (p.K + kBK - 1) / kBK;
+  p.kernel = GEMM_SINGLE_CTA;
+  p.bn = bn;
+  p.n_half = 0;
+  p.n_tiles = static_cast<int>(a.N / bn);
+  p.mn_tiles = static_cast<int>((a.M + kBM - 1) / kBM) * p.n_tiles;
   int splits = a.split_k;
   if (splits == 0) {
     splits = 1;
@@ -484,21 +579,54 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
       if (splits > p.kb_total / 4) splits = p.kb_total / 4 > 0 ? p.kb_total / 4 : 1;
     }
   }
-  if (splits > p.kb_total) splits = p.kb_total;
-  p.kb_per_split = (p.kb_total + splits - 1) / splits;
-  p.k_splits = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;  // every split non-empty
-  p.total_work = p.mn_tiles * p.k_splits;
+  set_splits(&p, splits);
+  p.ctas = p.total_work < sms ? p.total_work : sms;
+  if (a.max_ctas > 0 && p.ctas > a.max_ctas) p.ctas = a.max_ctas;
+  return 0;
+}
+
+}  // namespace vitk
+
+using namespace vitk;
+
+extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t stream_) {
+  VITK_REQUIRE(args != nullptr, VITK_EINVAL, "gemm: args is NULL");
+  const vitk_gemm_args& a = *args;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  GemmPlan plan;
+  if (int rc = plan_gemm(a, num_sms(), &plan)) return rc;
+  if (plan.kernel != GEMM_SINGLE_CTA) return launch_pair(a, plan, stream);
+
+  GemmParams p;
+  p.M = static_cast<int>(a.M); p.N = static_cast<int>(a.N); p.K = static_cast<int>(a.K);
+  p.n_tiles = plan.n_tiles; p.mn_tiles = plan.mn_tiles; p.k_splits = plan.k_splits;
+  p.kb_per_split = plan.kb_per_split; p.kb_total = plan.kb_total; p.total_work = plan.total_work;
   p.epi = a.epilogue;
   p.d = a.d; p.d2 = a.d2; p.bias = a.bias; p.aux = a.aux;
   p.ldd = a.ldd; p.ld_aux = a.ld_aux;
   p.rows_in = static_cast<int>(a.rows_in); p.rows_out = static_cast<int>(a.rows_out); p.row_off = static_cast<int>(a.row_off);
-  int grid = p.total_work < sms ? p.total_work : sms;
-  if (a.max_ctas > 0 && grid > a.max_ctas) grid = a.max_ctas;
-
+  const int grid = plan.ctas;
   const bool unpatch = a.epilogue == VITK_EPI_UNPATCH_F32;
-  switch (bn) {
+  switch (plan.bn) {
     case 256: return unpatch ? dispatch_major<256, true>(a, p, grid, stream) : dispatch_major<256, false>(a, p, grid, stream);
     case 192: return unpatch ? dispatch_major<192, true>(a, p, grid, stream) : dispatch_major<192, false>(a, p, grid, stream);
     default: return unpatch ? dispatch_major<128, true>(a, p, grid, stream) : dispatch_major<128, false>(a, p, grid, stream);
   }
+}
+
+// Host-only view of plan_gemm (no device needed): the launch vitk_gemm_bf16 makes for these arguments on a GPU with
+// `sms` SMs.
+extern "C" VITK_API int vitk_gemm_plan(const vitk_gemm_args* a, int sms, int* tile_n, int* split_k, int* n_half, int* work_items,
+                                       int* kernel, int* ctas) {
+  VITK_REQUIRE(a != nullptr && tile_n && split_k && n_half && work_items && kernel && ctas && sms >= 2, VITK_EINVAL,
+               "gemm_plan: bad argument");
+  GemmPlan plan;
+  if (int rc = plan_gemm(*a, sms, &plan)) return rc;
+  *tile_n = plan.bn;
+  *split_k = plan.k_splits;
+  *n_half = plan.n_half;
+  *work_items = plan.total_work;
+  *kernel = plan.kernel;
+  *ctas = plan.ctas;
+  return 0;
 }

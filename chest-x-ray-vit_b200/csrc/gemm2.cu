@@ -35,8 +35,8 @@
 
 #include "common.cuh"
 #include "gemm_epilogue.cuh"
+#include "gemm_host.cuh"
 #include "sm100_prims.cuh"
-#include "tmap.cuh"
 
 namespace vitk {
 
@@ -642,6 +642,8 @@ gemm2_bf16_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_consta
 }
 
 // ------------------------------------------------------------------------- host side
+static_assert(k2BM == 128 && k2BK == 64, "plan_gemm (gemm.cu) plans 256-row bands of 64-wide K blocks");
+
 // [32 rows × 64 B] output boxes (32 bf16 or 16 fp32 columns), 64-byte swizzle
 static int out_map(CUtensorMap* m, const void* base, bool f32, long long rows, long long cols, long long ld) {
   const uint64_t dims[2] = {static_cast<uint64_t>(cols), static_cast<uint64_t>(rows)};
@@ -651,28 +653,16 @@ static int out_map(CUtensorMap* m, const void* base, bool f32, long long rows, l
 }
 
 template <int BN, bool A_MN, bool B_MN, bool AUX, int EW = 8, int EPI = -1>
-static int launch_gemm2(const vitk_gemm_args& a, const Gemm2Params& p, int pairs, cudaStream_t stream) {
+static int launch_gemm2(const vitk_gemm_args& a, const Gemm2Params& p, int ctas, cudaStream_t stream) {
   using Cfg = Cfg2<BN, EW>;
   CUtensorMap ta, tb, tbh, td, td2;
-  {
-    uint64_t dims[2], str[1];
-    uint32_t box[2];
-    if (!A_MN) { dims[0] = a.K; dims[1] = a.M; box[0] = k2BK; box[1] = k2BM; }
-    else       { dims[0] = a.M; dims[1] = a.K; box[0] = 64;   box[1] = k2BK; }
-    str[0] = static_cast<uint64_t>(a.lda) * 2;
-    if (int rc = make_tensor_map_bf16(&ta, a.a, 2, dims, str, box)) return rc;
-    if (!B_MN) { dims[0] = a.K; dims[1] = a.N; box[0] = k2BK; box[1] = Cfg::kBHalfRows; }
-    else       { dims[0] = a.N; dims[1] = a.K; box[0] = 64;   box[1] = k2BK; }
-    str[0] = static_cast<uint64_t>(a.ldb) * 2;
-    if (int rc = make_tensor_map_bf16(&tb, a.b, 2, dims, str, box)) return rc;
-    tbh = tb;
-    if (!B_MN && p.n_half > 0) {       // half-width tiles stage BN/4 rows of a K-major B per CTA
-      box[1] = Cfg::kBHalfRows / 2;
-      if (int rc = make_tensor_map_bf16(&tbh, a.b, 2, dims, str, box)) return rc;
-    }
+  if (int rc = operand_map(&ta, a.a, A_MN, a.M, a.K, a.lda, k2BM)) return rc;
+  if (int rc = operand_map(&tb, a.b, B_MN, a.N, a.K, a.ldb, Cfg::kBHalfRows)) return rc;
+  tbh = tb;
+  if (!B_MN && p.n_half > 0) {       // half-width tiles stage BN/4 rows of a K-major B per CTA
+    if (int rc = operand_map(&tbh, a.b, false, a.N, a.K, a.ldb, Cfg::kBHalfRows / 2)) return rc;
   }
-  const bool f32_out = a.epilogue == VITK_EPI_BIAS_RESID_F32 || a.epilogue == VITK_EPI_ACCUM_F32 || a.epilogue == VITK_EPI_STORE_F32;
-  if (int rc = out_map(&td, a.d, f32_out, a.M, a.N, a.ldd)) return rc;
+  if (int rc = out_map(&td, a.d, kEpiTraits[a.epilogue].f32_out, a.M, a.N, a.ldd)) return rc;
   td2 = td;
   if (a.d2 != nullptr) { if (int rc = out_map(&td2, a.d2, false, a.M, a.N, a.ldd)) return rc; }
   auto kern = gemm2_bf16_kernel<BN, A_MN, B_MN, AUX, EW, EPI>;
@@ -682,151 +672,33 @@ static int launch_gemm2(const vitk_gemm_args& a, const Gemm2Params& p, int pairs
     attr_err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::kSmemBytes);
   });
   if (attr_err != cudaSuccess) return cuda_error(attr_err, "cudaFuncSetAttribute(gemm2 smem)");
-  if (cudaError_t e = launch_pdl(kern, dim3(2 * pairs), dim3(threads2(EW)), Cfg::kSmemBytes, stream, ta, tb, tbh, td, td2, p); e != cudaSuccess)
+  if (cudaError_t e = launch_pdl(kern, dim3(ctas), dim3(threads2(EW)), Cfg::kSmemBytes, stream, ta, tb, tbh, td, td2, p); e != cudaSuccess)
     return cuda_error(e, "gemm2_bf16_kernel launch");
   VITK_LAUNCH_CHECK("gemm2_bf16_kernel");
   return 0;
 }
 
 template <int BN, bool AUX>
-static int dispatch_major2(const vitk_gemm_args& a, const Gemm2Params& p, int pairs, cudaStream_t s) {
-  if (!a.a_mn_major && !a.b_mn_major) return launch_gemm2<BN, false, false, AUX>(a, p, pairs, s);
+static int dispatch_major2(const vitk_gemm_args& a, const Gemm2Params& p, int ctas, cudaStream_t s) {
+  if (!a.a_mn_major && !a.b_mn_major) return launch_gemm2<BN, false, false, AUX>(a, p, ctas, s);
   if constexpr (!AUX) {          // wgrad layouts (MN-major A) never carry an aux tile
-    if (a.a_mn_major && !a.b_mn_major) return launch_gemm2<BN, true, false, false>(a, p, pairs, s);
+    if (a.a_mn_major && !a.b_mn_major) return launch_gemm2<BN, true, false, false>(a, p, ctas, s);
   }
   if constexpr (BN != 192) {     // an MN-major B half must be whole 64-column TMA boxes
-    if (!a.a_mn_major && a.b_mn_major) return launch_gemm2<BN, false, true, AUX>(a, p, pairs, s);
-    if constexpr (!AUX) return launch_gemm2<BN, true, true, false>(a, p, pairs, s);
+    if (!a.a_mn_major && a.b_mn_major) return launch_gemm2<BN, false, true, AUX>(a, p, ctas, s);
+    if constexpr (!AUX) return launch_gemm2<BN, true, true, false>(a, p, ctas, s);
   }
   return set_error(VITK_EINVAL, "gemm2: unsupported operand layout for this tile width / epilogue (tile_n 192 needs a K-major B; "
                                 "aux epilogues need a K-major A)");
 }
 
-// fc1 forward (+bias, GELU, optional GELU') as a 16-epilogue-warp instantiation with the epilogue fixed at compile time
-// (see the kernel's template comment): 2 MUFU + 13 FP32 operations per element are a chain of dependent latencies that
-// four warps per scheduler hide better than two — 51.4 → 47.1 µs at M = 9232 (profiles/r02_bench_gemm_ew16.txt), bit-identical
-// output (tests/test_gpu_gemm.py::test_sixteen_warp_epilogues_equal_eight_warp).  The same treatment of the multiplier
-// and fp32-residual epilogues was measured and dropped: those launches move 128 / 71 MB for 43.6 / 10.9 GF and sit on
-// the HBM side of the roofline, not on the epilogue's instruction latency (no change at 49.2 / 28.7 / 47.1 µs).
-// Variant 3 keeps the 8-warp instantiation (the reference the 16-warp one is tested against).
-static bool launch_heavy2(const vitk_gemm_args& a, const Gemm2Params& p, int bn, int pairs, cudaStream_t s, int* rc) {
-  if (a.variant == 3) return false;
-  if (a.epilogue == VITK_EPI_BIAS_GELUG_BF16 && !a.a_mn_major && !a.b_mn_major && bn == 256) {
-    *rc = launch_gemm2<256, false, false, false, 16, VITK_EPI_BIAS_GELUG_BF16>(a, p, pairs, s);
-    return true;
-  }
-  return false;
-}
-
-// cycles a CTA pair spends per 64-wide K block of a tile of `bn` columns (tools/gemm_timeline.py, B200): the MMAs of a
-// 256-wide tile occupy the tensor pipe for 4 × 122 cycles; narrower tiles are bound by operand delivery instead.
-// 192: A/B on the full step, 440 (192-wide tiles for K-major N = 768) beats 500 (mixed 256+128 there) by 0.9 %.
-static double kblock_cycles(int bn) { return bn == 256 ? 500.0 : (bn == 192 ? 440.0 : 390.0); }
-constexpr double kTileFixedCycles = 1500.0;   // accumulator hand-over + pipeline refill per tile
-
-static void choose_tiling2(const vitk_gemm_args& a, int pairs, int* bn_out, int* splits_out, int* n_half_out,
-                           double* cost_out = nullptr) {
-  const long long mt = (a.M + 2 * k2BM - 1) / (2 * k2BM);
-  const long long kb_total = (a.K + k2BK - 1) / k2BK;
-  double best = 1e30;
-  const int cands[3] = {256, 192, 128};
-  for (int bn : cands) {
-    if (a.N % bn) continue;
-    if (a.b_mn_major && bn == 192) continue;
-    if (a.tile_n && a.tile_n != bn) continue;
-    const long long tiles = mt * (a.N / bn);
-    int splits = 1;
-    if (a.epilogue == VITK_EPI_ACCUM_F32) {
-      if (a.split_k > 0) splits = a.split_k;
-      else if (tiles < pairs) {
-        splits = static_cast<int>(pairs / tiles);
-        const long long cap = kb_total / 4 > 0 ? kb_total / 4 : 1;
-        if (splits > cap) splits = static_cast<int>(cap);
-        if (splits < 1) splits = 1;
-      }
-    }
-    const long long kb_per = (kb_total + splits - 1) / splits;
-    const long long items = tiles * ((kb_total + kb_per - 1) / kb_per);
-    const long long waves = (items + pairs - 1) / pairs;
-    const double cost = static_cast<double>(waves) * (kb_per * kblock_cycles(bn) + kTileFixedCycles);
-    if (cost < best - 1e-9) { best = cost; *bn_out = bn; *splits_out = splits; *n_half_out = 0; }
-    // Mixed widths (BN = 256 only): replace some of each band's 256-column tiles by pairs of 128-column tiles so that
-    // the static round-robin order gives every CTA pair the same amount of work (e.g. N = 768 on 74 pairs: 3 full
-    // tiles per band = 1.5 waves of full tiles; 2 full + 2 half = one full and one half tile for every pair).
-    if (bn == 256 && splits == 1 && a.epilogue != VITK_EPI_ACCUM_F32 && a.tile_n == 0) {
-      const int n_tiles256 = static_cast<int>(a.N / 256);
-      const double cf = kb_total * kblock_cycles(256) + kTileFixedCycles, ch = kb_total * kblock_cycles(128) + kTileFixedCycles;
-      for (int nh = 2; nh <= 2 * n_tiles256; nh += 2) {
-        const int nf = n_tiles256 - nh / 2;
-        const long long full_items = mt * nf, all_items = mt * (nf + nh);
-        double worst = 0;
-        for (int pr = 0; pr < pairs && pr < all_items; ++pr) {
-          double c = 0;
-          for (long long w = pr; w < all_items; w += pairs) c += w < full_items ? cf : ch;
-          if (c > worst) worst = c;
-        }
-        if (worst < best - 1e-9) { best = worst; *bn_out = 256; *splits_out = 1; *n_half_out = nh; }
-      }
-    }
-  }
-  if (cost_out) *cost_out = best;
-}
-
-// Data-gradient GEMMs (K-major A, MN-major B, plain bf16 store) whose M is ragged against the pair kernel's 256-row bands
-// can quantise badly on 74 pairs yet perfectly on 148 single CTAs with 128-row bands — ViT-L at batch 8: M = 4616 → 19
-// bands × 4 tiles of 256 columns = 76 tiles (two pairs get a second tile) against 37 × 4 = 148 tiles = exactly one wave.
-// Measured there (tools/bench_gemm.py, VITK_BG_M=4616 VITK_BG_D=1024 VITK_BG_F=4096): fc1 dgrad 43.2 → 35.7 µs,
-// qkv dgrad 35.8 → 28.8 µs, out dgrad 19.5 → 16.5 µs.  Per K block a single CTA (which stages the whole B tile itself)
-// costs ≈ 1.1 × the pair kernel's 256-wide block for this operand layout.
-static bool single_cta_wins(const vitk_gemm_args& a, double pair_cost, int sms) {
-  if (a.variant != 0 || a.tile_n != 0 || a.max_ctas != 0 || a.a_mn_major || !a.b_mn_major || a.epilogue != VITK_EPI_STORE_BF16 ||
-      a.N % 256 != 0)
-    return false;
-  const long long tiles = ((a.M + 127) / 128) * (a.N / 256);
-  const long long waves = (tiles + sms - 1) / sms;
-  const long long kb = (a.K + k2BK - 1) / k2BK;
-  const double cost = static_cast<double>(waves) * (kb * 1.1 * kblock_cycles(256) + kTileFixedCycles);
-  return cost < 0.9 * pair_cost;
-}
-
-// Called by vitk_gemm_bf16 (gemm.cu) after argument validation.  Returns VITK_EINVAL-free 1 when the
-// problem is not eligible for the pair kernel so that the caller falls through to the 1-CTA kernel.
-int gemm2_try_launch(const vitk_gemm_args& a, cudaStream_t stream, bool* handled) {
-  *handled = false;
-  if (a.variant == 1) return 0;
-  const bool aux_epi = a.epilogue == VITK_EPI_BIAS_RESID_F32 || a.epilogue == VITK_EPI_MUL_BF16 || a.epilogue == VITK_EPI_DGELU_BF16;
-  const bool eligible = a.epilogue != VITK_EPI_PATCH_F32 && a.epilogue != VITK_EPI_UNPATCH_F32 && a.N % 128 == 0 && (a.max_ctas == 0 || a.max_ctas >= 2) &&
-                        !(aux_epi && a.a_mn_major) &&     // the aux instantiations exist for K-major A only
-                        (a.tile_n == 0 || a.tile_n == 128 || a.tile_n == 192 || a.tile_n == 256) &&
-                        !(a.tile_n == 192 && a.b_mn_major);
-  if (!eligible) {
-    VITK_REQUIRE(a.variant < 2, VITK_EINVAL, "gemm: the CTA-pair kernel does not support this problem (epilogue %d, tile_n %d)",
-                 a.epilogue, a.tile_n);
-    return 0;
-  }
-  const int sms = num_sms();
-  // max_ctas leaves SMs free for a concurrent NCCL all-reduce (tile choice then balances waves over fewer pairs)
-  const int pairs_avail = (a.max_ctas > 0 && a.max_ctas < sms ? a.max_ctas : sms) / 2;
-  int bn = 0, splits = 1, n_half = 0;
-  double pair_cost = 0;
-  choose_tiling2(a, pairs_avail, &bn, &splits, &n_half, &pair_cost);
-  if (bn == 0) {
-    VITK_REQUIRE(a.variant < 2, VITK_EINVAL, "gemm: no CTA-pair tiling for N=%lld tile_n=%d", (long long)a.N, a.tile_n);
-    return 0;
-  }
-  if (single_cta_wins(a, pair_cost, sms)) return 0;     // falls through to the single-CTA kernel (gemm.cu), 256-wide tiles
+int launch_pair(const vitk_gemm_args& a, const GemmPlan& plan, cudaStream_t stream) {
   Gemm2Params p;
   p.M = static_cast<int>(a.M); p.N = static_cast<int>(a.N); p.K = static_cast<int>(a.K);
-  const int m_tiles = (p.M + 2 * k2BM - 1) / (2 * k2BM);
-  p.n_half = n_half;
-  p.n_full = p.N / bn - n_half / 2;
-  p.n_tiles = p.n_full + p.n_half;
-  p.mn_tiles = m_tiles * p.n_tiles;
-  p.kb_total = (p.K + k2BK - 1) / k2BK;
-  if (splits > p.kb_total) splits = p.kb_total;
-  p.kb_per_split = (p.kb_total + splits - 1) / splits;
-  p.k_splits = (p.kb_total + p.kb_per_split - 1) / p.kb_per_split;
-  p.total_work = p.mn_tiles * p.k_splits;
+  p.n_tiles = plan.n_tiles; p.mn_tiles = plan.mn_tiles; p.k_splits = plan.k_splits;
+  p.kb_per_split = plan.kb_per_split; p.kb_total = plan.kb_total; p.total_work = plan.total_work;
+  p.n_half = plan.n_half;
+  p.n_full = plan.n_tiles - plan.n_half;
   p.epi = a.epilogue;
   p.has_d2 = a.d2 != nullptr;
   p.aux = a.aux;
@@ -834,39 +706,15 @@ int gemm2_try_launch(const vitk_gemm_args& a, cudaStream_t stream, bool* handled
   p.bias = a.bias;
   p.tl = g_timeline;
   p.tl_seq = g_timeline != nullptr ? g_timeline_seq++ : 0;
-  const int pairs = p.total_work < pairs_avail ? p.total_work : pairs_avail;
-  *handled = true;
-  {
-    int rc = 0;
-    if (launch_heavy2(a, p, bn, pairs, stream, &rc)) return rc;
-  }
-  switch (bn) {
-    case 256: return aux_epi ? dispatch_major2<256, true>(a, p, pairs, stream) : dispatch_major2<256, false>(a, p, pairs, stream);
-    case 192: return aux_epi ? dispatch_major2<192, true>(a, p, pairs, stream) : dispatch_major2<192, false>(a, p, pairs, stream);
-    default: return aux_epi ? dispatch_major2<128, true>(a, p, pairs, stream) : dispatch_major2<128, false>(a, p, pairs, stream);
+  const int ctas = plan.ctas;
+  if (plan.kernel == GEMM_PAIR_EW16)
+    return launch_gemm2<256, false, false, false, 16, VITK_EPI_BIAS_GELUG_BF16>(a, p, ctas, stream);
+  const bool aux = kEpiTraits[a.epilogue].aux;
+  switch (plan.bn) {
+    case 256: return aux ? dispatch_major2<256, true>(a, p, ctas, stream) : dispatch_major2<256, false>(a, p, ctas, stream);
+    case 192: return aux ? dispatch_major2<192, true>(a, p, ctas, stream) : dispatch_major2<192, false>(a, p, ctas, stream);
+    default: return aux ? dispatch_major2<128, true>(a, p, ctas, stream) : dispatch_major2<128, false>(a, p, ctas, stream);
   }
 }
 
 }  // namespace vitk
-
-// Host-only view of the tiling decision (no device needed): which tile width, split-K factor and number of
-// half-width tiles per 256-row band vitk_gemm_bf16 would use for this problem on a GPU with `sms` SMs.
-extern "C" VITK_API int vitk_gemm_plan(const vitk_gemm_args* a, int sms, int* tile_n, int* split_k, int* n_half, int* work_items) {
-  using namespace vitk;
-  VITK_REQUIRE(a != nullptr && tile_n && split_k && n_half && work_items && sms >= 2, VITK_EINVAL, "gemm_plan: bad argument");
-  VITK_REQUIRE(a->M > 0 && a->N > 0 && a->K > 0 && a->N % 128 == 0, VITK_EINVAL, "gemm_plan: the CTA-pair kernel needs N %% 128 == 0");
-  const int pairs = (a->max_ctas > 0 && a->max_ctas < sms ? a->max_ctas : sms) / 2;
-  int bn = 0, splits = 1, nh = 0;
-  choose_tiling2(*a, pairs, &bn, &splits, &nh);
-  VITK_REQUIRE(bn != 0, VITK_EINVAL, "gemm_plan: no CTA-pair tiling for N=%lld tile_n=%d", (long long)a->N, a->tile_n);
-  const long long m_tiles = (a->M + 2 * k2BM - 1) / (2 * k2BM);
-  const long long kb_total = (a->K + k2BK - 1) / k2BK;
-  if (splits > kb_total) splits = static_cast<int>(kb_total);
-  const long long kb_per = (kb_total + splits - 1) / splits;
-  *tile_n = bn;
-  *split_k = static_cast<int>((kb_total + kb_per - 1) / kb_per);
-  *n_half = nh;
-  *work_items = static_cast<int>(m_tiles * (a->N / bn - nh / 2 + nh) * *split_k);
-  return 0;
-}
-

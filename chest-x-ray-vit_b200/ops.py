@@ -168,15 +168,24 @@ def gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, d: torch.Tens
 
 
 def gemm_plan(M: int, N: int, K: int, *, epilogue: int, b_mn_major: bool = False, a_mn_major: bool = False,
-              split_k: int = 0, tile_n: int = 0, max_ctas: int = 0, sms: int = 148) -> dict:
-    """Host-only: the tiling vitk_gemm_bf16 would pick for this problem on a GPU with ``sms`` SMs (no device needed)."""
+              split_k: int = 0, tile_n: int = 0, max_ctas: int = 0, variant: int = 0, ldd: Optional[int] = None,
+              rows_in: int = 0, rows_out: int = 0, row_off: int = 0, sms: int = 148) -> dict:
+    """Host-only: the launch vitk_gemm_bf16 would make for this problem on a GPU with ``sms`` SMs (no device needed).
+    ``kernel`` is 1 (single CTA), 2 (CTA pair) or 3 (CTA pair, 16 epilogue warps); ``ctas`` is the grid.  Every operand
+    is a stand-in address (checked, never read) with the smallest valid leading dimension; ``ldd`` defaults to N."""
+    def up8(n):
+        return (n + 7) // 8 * 8
     g = GemmArgs()
+    g.a = g.b = g.d = g.d2 = g.aux = 1 << 20
     g.M, g.N, g.K = M, N, K
+    g.lda, g.ldb = up8(M if a_mn_major else K), up8(N if b_mn_major else K)
+    g.ldd, g.ld_aux = (ldd if ldd is not None else N), N
     g.a_mn_major, g.b_mn_major = int(a_mn_major), int(b_mn_major)
-    g.epilogue, g.split_k, g.tile_n, g.max_ctas = epilogue, split_k, tile_n, max_ctas
-    tn, sk, nh, items = C.c_int(), C.c_int(), C.c_int(), C.c_int()
-    _lib.check(_lib.lib().vitk_gemm_plan(C.byref(g), sms, C.byref(tn), C.byref(sk), C.byref(nh), C.byref(items)), "gemm_plan")
-    return {"tile_n": tn.value, "split_k": sk.value, "n_half": nh.value, "work_items": items.value}
+    g.epilogue, g.split_k, g.tile_n, g.max_ctas, g.variant = epilogue, split_k, tile_n, max_ctas, variant
+    g.rows_in, g.rows_out, g.row_off = rows_in, rows_out, row_off
+    out = [C.c_int() for _ in range(6)]
+    _lib.check(_lib.lib().vitk_gemm_plan(C.byref(g), sms, *(C.byref(o) for o in out)), "gemm_plan")
+    return dict(zip(("tile_n", "split_k", "n_half", "work_items", "kernel", "ctas"), (o.value for o in out)))
 
 
 def colsum(x: torch.Tensor, out: torch.Tensor) -> torch.Tensor:

@@ -239,10 +239,14 @@ VITK_API int vitk_clip_scale(const float* sumsq, float max_norm, float* scale, v
  * bf16 shadow refresh after optimizer.step(): dst_bf16[i] = bf16(src[i]). n multiple of 8. */
 VITK_API int vitk_cast_f32_bf16(const float* src, void* dst_bf16, int64_t n, vitk_stream_t stream);
 VITK_API int vitk_fill_zero(void* ptr, size_t bytes, vitk_stream_t stream);
-/* Host-only: the tiling vitk_gemm_bf16 would choose for this problem on a GPU with `sms` SMs — tile width (128 /
- * 192 / 256 columns), split-K factor, half-width tiles per 256-row band (mixed 256+128 schedule) and the number of
- * work items dealt round-robin to sms/2 CTA pairs.  Needs no device; used by the CPU tests of the schedule. */
-VITK_API int vitk_gemm_plan(const vitk_gemm_args* args, int sms, int* tile_n, int* split_k, int* n_half, int* work_items);
+/* Host-only: the launch vitk_gemm_bf16 makes for these arguments on a GPU with `sms` SMs, decided by the same code
+ * and rejected with the same error where vitk_gemm_bf16 would reject them (operand pointers are checked for NULL and
+ * alignment, never dereferenced).  kernel: 1 = single-CTA, 2 = CTA pair, 3 = CTA pair with 16 epilogue warps; tile
+ * width (128 / 192 / 256 columns), split-K factor, half-width tiles per 256-row band (mixed 256+128 schedule of the
+ * pair kernel; 0 for the single-CTA kernel), work items dealt round-robin over the grid, and the grid in CTAs.
+ * Needs no device; used by the CPU tests of the schedule. */
+VITK_API int vitk_gemm_plan(const vitk_gemm_args* args, int sms, int* tile_n, int* split_k, int* n_half, int* work_items,
+                            int* kernel, int* ctas);
 /* Diagnostics: when device_buf is non-NULL, CTA (0,0,0) of vitk_attn_bwd records clock64() stamps of its pipeline
  * phases into it (>= 1024 int64; slot = 16·query_block + phase) and the CTA-pair GEMM records per-K-block / per-tile /
  * per-CTA stamps (>= 8192 int64; layout in csrc/gemm2.cu); NULL (default) disables. */
