@@ -60,6 +60,8 @@ _PROTOS = {
     "vitk_attn_bwd": (C.c_int, [_p, _p, _p, _p, _i64, _i64, _i64, _f, _p, _p, _p]),
     "vitk_embed_cls": (C.c_int, [_p, _p, _i64, _i64, _i64, _p, _p]),
     "vitk_embed_bwd": (C.c_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _p]),
+    "vitk_pos_interp": (C.c_int, [_p, _i64, _i64, _i64, _i64, _i64, _p, _p]),
+    "vitk_pos_interp_bwd": (C.c_int, [_p, _i64, _i64, _i64, _i64, _i64, _p, _p]),
     "vitk_head_fwd": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _p, _f, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "vitk_head_bwd": (C.c_int, [_p, _p, _p, _p, _p, _p, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p, _p, _p]),
     "vitk_multilabel_counts": (C.c_int, [_p, _p, _i64, _i64, _f, _p, _p]),

@@ -161,7 +161,8 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, int row, int
 // VITK_EPI_UNPATCH_F32 (the input gradient, col2im of dh·Wp), in kernel instantiations of its own: a further case in
 // epilogue_chunk costs the existing instantiations 36-40 registers, even left unused.  Row = token t of image g; tokens
 // before row_off (CLS) carry no pixels.  Columns col0 … col0+31 are channel c, patch rows ky and ky+1
-// (k = c·256 + ky·16 + kx): two 64-byte runs of the NCHW image, whose width is ldd = 16·G.
+// (k = c·256 + ky·16 + kx): two 64-byte runs of the NCHW image, whose width is ldd = 16·G (G patches per row) and
+// whose height the host passes in p.rows_in.
 __device__ __forceinline__ void unpatch_chunk(const GemmParams& p, int row, int col0, const float (&v)[32]) {
   if (row >= p.M) return;
   const int g = row / p.rows_out;
@@ -171,7 +172,7 @@ __device__ __forceinline__ void unpatch_chunk(const GemmParams& p, int row, int 
   const int py = t / G, px = t - py * G;
   const int c = col0 >> 8, ky = (col0 >> 4) & 15;
   float4* o4 = reinterpret_cast<float4*>(reinterpret_cast<float*>(p.d) +
-                                         ((static_cast<long long>(g) * 3 + c) * p.ldd + py * 16 + ky) * p.ldd + px * 16);
+                                         ((static_cast<long long>(g) * 3 + c) * p.rows_in + py * 16 + ky) * p.ldd + px * 16);
   const long long next = p.ldd >> 2;    // one image row, in float4
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
@@ -495,11 +496,19 @@ int plan_gemm(const vitk_gemm_args& a, int sms, GemmPlan* out) {
                  "gemm: UNPATCH_F32 needs rows_out > row_off >= 0 (rows_out=%lld, row_off=%lld)", (long long)a.rows_out,
                  (long long)a.row_off);
     const long long P = a.rows_out - a.row_off;
-    long long G = 0;
-    while ((G + 1) * (G + 1) <= P) ++G;
-    VITK_REQUIRE(G * G == P, VITK_EINVAL, "gemm: UNPATCH_F32 needs a square number of patches, got rows_out - row_off = %lld", P);
-    VITK_REQUIRE(a.ldd == 16 * G, VITK_EINVAL, "gemm: UNPATCH_F32 needs ldd = image width = 16·%lld, got ldd=%lld", G,
-                 (long long)a.ldd);
+    if (a.rows_in == 0) {                    // a square grid of G×G patches
+      long long G = 0;
+      while ((G + 1) * (G + 1) <= P) ++G;
+      VITK_REQUIRE(G * G == P, VITK_EINVAL, "gemm: UNPATCH_F32 needs a square number of patches, got rows_out - row_off = %lld", P);
+      VITK_REQUIRE(a.ldd == 16 * G, VITK_EINVAL, "gemm: UNPATCH_F32 needs ldd = image width = 16·%lld, got ldd=%lld", G,
+                   (long long)a.ldd);
+    } else {                                 // rows_in patches per image row, P / rows_in rows of them
+      VITK_REQUIRE(a.rows_in > 0 && P % a.rows_in == 0, VITK_EINVAL,
+                   "gemm: UNPATCH_F32 needs rows_in (patches per image row) > 0 dividing rows_out - row_off = %lld, got "
+                   "rows_in=%lld", P, (long long)a.rows_in);
+      VITK_REQUIRE(a.ldd == 16 * a.rows_in, VITK_EINVAL, "gemm: UNPATCH_F32 needs ldd = image width = 16·%lld, got ldd=%lld",
+                   (long long)a.rows_in, (long long)a.ldd);
+    }
     VITK_REQUIRE(a.M % a.rows_out == 0, VITK_EINVAL, "gemm: UNPATCH_F32 needs M %% rows_out == 0 (M=%lld, rows_out=%lld)",
                  (long long)a.M, (long long)a.rows_out);
   } else {
@@ -607,6 +616,8 @@ extern "C" VITK_API int vitk_gemm_bf16(const vitk_gemm_args* args, vitk_stream_t
   p.rows_in = static_cast<int>(a.rows_in); p.rows_out = static_cast<int>(a.rows_out); p.row_off = static_cast<int>(a.row_off);
   const int grid = plan.ctas;
   const bool unpatch = a.epilogue == VITK_EPI_UNPATCH_F32;
+  // UNPATCH_F32 reads rows_in as the image height in pixels: 16 · patches / patches per row (ldd / 16 for a square grid)
+  if (unpatch) p.rows_in = static_cast<int>(16 * (a.rows_out - a.row_off) / (a.rows_in ? a.rows_in : a.ldd / 16));
   switch (plan.bn) {
     case 256: return unpatch ? dispatch_major<256, true>(a, p, grid, stream) : dispatch_major<256, false>(a, p, grid, stream);
     case 192: return unpatch ? dispatch_major<192, true>(a, p, grid, stream) : dispatch_major<192, false>(a, p, grid, stream);

@@ -165,15 +165,27 @@ def _p(t: Optional[torch.Tensor]):
 
 
 class Arena:
-    """Activation + scratch buffers and launch plans for one (batch size, training?) pair."""
+    """Activation + scratch buffers and launch plans for one (batch size, training?, patch grid) triple.
 
-    def __init__(self, eng: "Engine", B: int, train: bool):
+    The token geometry lives here: an arena at the gh × gw patch grid has P = gh·gw patches and T = P + 1 tokens, and
+    every shape below is taken from it.  At the checkpoint's grid (``image_size / 16`` on each side) the position table
+    is the parameter itself.  At any other grid (HF ``interpolate_pos_encoding``, modeling_vit.py:60-99) the arena owns
+    a resized table [T, D] that ``vitk_pos_interp`` rewrites as the first launch of every forward plan, and the training
+    backward sends the embeddings' position gradient through ``vitk_pos_interp_bwd`` into the parameter's [T0, D]."""
+
+    def __init__(self, eng: "Engine", B: int, train: bool, gh: int, gw: int):
         cfg = eng.cfg
         dev = eng.dev
         D, Fi, H, L, Cn = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.num_labels
-        T, P = cfg.seq_len, cfg.num_patches
+        P = gh * gw
+        T = P + 1
         M = B * T
         self.B, self.train, self.M = B, train, M
+        self.gh, self.gw, self.T, self.P = gh, gw, T, P
+        self.g0 = cfg.image_size // cfg.patch_size            # the checkpoint's grid, g0 × g0
+        self.interp = (gh, gw) != (self.g0, self.g0)
+        # the CLS-row kernels of the top layer take T <= 4096; above that the top layer runs densely
+        self.cls_top = eng.cls_only_top and T <= 4096
         self.ticket = -1
 
         def new(shape, dt):
@@ -196,6 +208,7 @@ class Arena:
         self.loss = new((1,), f32)
         self.dlogits = new((B, Cn), f32)
         self.hstat = new((2, B), f32)
+        self.pos = new((T, D), f32) if self.interp else eng.w["pos"]      # the position table this grid adds
         self.fwd = self._build_forward(eng, with_labels=False)
         self.fwd_loss = self._build_forward(eng, with_labels=True)
         self._eng = eng
@@ -213,6 +226,7 @@ class Arena:
             self.dpatch = new((B * P, D), bf16)
             self.dloss = new((1,), f32)
             self.dlogits_in = new((B, Cn), f32)
+            self.dpos = new((T, D), f32) if self.interp else None     # position gradient at this grid, before the adjoint
             self._bwd_plans: Dict[Tuple[bool, bool], _Plan] = {}
             self._data_plans: Dict[bool, _Plan] = {}
             self._sink: Optional[dict] = None
@@ -257,7 +271,7 @@ class Arena:
         if pl is None:
             eng = self._eng
             cfg = eng.cfg
-            D, H, L, T = cfg.hidden_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.seq_len
+            D, H, L, T = cfg.hidden_size, cfg.num_attention_heads, cfg.num_hidden_layers, self.T
             if not self.train and self.hs is None:
                 self.hs = torch.empty((L + 1, self.M, D), dtype=f32, device=eng.dev)
                 self.qkv_all = [torch.empty((self.M, 3 * D), dtype=bf16, device=eng.dev) for _ in range(L)]
@@ -268,7 +282,7 @@ class Arena:
     def hidden_states(self) -> Tuple[torch.Tensor, ...]:
         """Copies of the L+1 residual-stream tensors an outputs plan left behind, each fp32 [B, T, D]."""
         cfg = self._eng.cfg
-        L, T, D = cfg.num_hidden_layers, cfg.seq_len, cfg.hidden_size
+        L, T, D = cfg.num_hidden_layers, self.T, cfg.hidden_size
         hs = torch.stack(self.h) if self.train else self.hs.clone()
         return hs.view(L + 1, self.B, T, D).unbind(0)
 
@@ -276,7 +290,7 @@ class Arena:
     def _build_forward(self, eng: "Engine", with_labels: bool, outputs: bool = False) -> _Plan:
         cfg, w = eng.cfg, eng.w
         D, Fi, H, L, Cn = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.num_labels
-        T, P, B, M = cfg.seq_len, cfg.num_patches, self.B, self.M
+        T, P, B, M = self.T, self.P, self.B, self.M
         eps = cfg.layer_norm_eps
         scale = 64 ** -0.5
         pl = _Plan()
@@ -289,8 +303,10 @@ class Arena:
         else:
             hs, qkv, lse = [self.h[0]] * (L + 1), [self.qkv[0]] * L, [self.lse[0]] * L
         h0 = hs[0]
-        pl.add("vitk_embed_cls", _p(w["cls"]), _p(w["pos"]), B, T, D, _p(h0))
-        pl.gemm(self.apatch, w["wp16"], B * P, D, 768, h0, EPI_PATCH_F32, bias=w["bp"], aux=w["pos"], rows_in=P, rows_out=T,
+        if self.interp:      # the parameters change every step: resize the table in every forward
+            pl.add("vitk_pos_interp", _p(w["pos"]), self.g0, self.g0, self.gh, self.gw, D, _p(self.pos))
+        pl.add("vitk_embed_cls", _p(w["cls"]), _p(self.pos), B, T, D, _p(h0))
+        pl.gemm(self.apatch, w["wp16"], B * P, D, 768, h0, EPI_PATCH_F32, bias=w["bp"], aux=self.pos, rows_in=P, rows_out=T,
                 row_off=1, ldd=D, ld_aux=D)
         def cls_rows(t: torch.Tensor) -> torch.Tensor:      # the B CLS rows of a [B·T, width] buffer, in place (row stride T·width)
             width = t.shape[1]
@@ -304,7 +320,7 @@ class Arena:
             st = self.st[i]
             pl.add("vitk_layernorm_fwd", _p(hin), D, _p(lw["g1"]), _p(lw["b1"]), eps, M, D, _p(self.n1[i]), _p(st[0]), _p(st[1]))
             pl.gemm(self.n1[i], lw["wqkv16"], M, 3 * D, D, qkv[l], EPI_BIAS_BF16, bias=lw["bqkv"])
-            if l == L - 1 and eng.cls_only_top and not outputs:
+            if l == L - 1 and self.cls_top and not outputs:
                 # ---- top layer: the classifier reads sequence_output[:, 0] only (HF modeling_vit.py:641), so after the keys
                 # and values of all tokens exist, everything else of this layer is computed for the B CLS rows alone —
                 # attention of one query per head, then out-proj / LN / MLP on strided [B, ·] views that leave the rows
@@ -342,7 +358,7 @@ class Arena:
         """data_only: leave out every launch that only produces parameter gradients (see data_backward_plan)."""
         cfg, w = eng.cfg, eng.w
         D, Fi, H, L, Cn = cfg.hidden_size, cfg.intermediate_size, cfg.num_attention_heads, cfg.num_hidden_layers, cfg.num_labels
-        T, P, B, M = cfg.seq_len, cfg.num_patches, self.B, self.M
+        T, P, B, M = self.T, self.P, self.B, self.M
         scale = 64 ** -0.5
         wgrad = not data_only
         pl = _Plan(eng.side_stream if wgrad else None)
@@ -385,7 +401,7 @@ class Arena:
                _p(dh1), _p(lg["g2"]), _p(lg["b2"]), _p(lg["bo"]))
         if wgrad:
             pl.gemm(dh1_c, o_c, D, D, B, lg["wo"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
-        if eng.cls_only_top:
+        if self.cls_top:
             pl.gemm(dh1_c, lw["wo16"], B, D, D, do_c, EPI_STORE_BF16, b_mn_major=True)
             pl.add("vitk_attn_cls_bwd", _p(self.qkv[l]), _p(self.o[l]), _p(self.do), _p(self.lse[l]), B, T, H, scale, _p(self.dqkv))
         else:
@@ -445,7 +461,12 @@ class Arena:
                    _p(dh), _p(lg["g1"]), _p(lg["b1"]), _p(g["layers"][l - 1]["bf2"]) if l > 0 else None)
             layer_done(l)
         if wgrad:
-            pl.add("vitk_embed_bwd", _p(dh), B, T, D, _p(g["pos"]), _p(g["cls"]), _p(g["bp"]), _p(self.dpatch))
+            if self.interp:      # the position gradient at this grid, then its adjoint resize onto the parameter
+                pl.add("vitk_fill_zero", _p(self.dpos), self.dpos.numel() * 4)
+                pl.add("vitk_embed_bwd", _p(dh), B, T, D, _p(self.dpos), _p(g["cls"]), _p(g["bp"]), _p(self.dpatch))
+                pl.add("vitk_pos_interp_bwd", _p(self.dpos), self.gh, self.gw, self.g0, self.g0, D, _p(g["pos"]))
+            else:
+                pl.add("vitk_embed_bwd", _p(dh), B, T, D, _p(g["pos"]), _p(g["cls"]), _p(g["bp"]), _p(self.dpatch))
             pl.gemm(self.dpatch, self.apatch, D, 768, B * P, g["wp"], EPI_ACCUM_F32, a_mn_major=True, b_mn_major=True)
             if eng.grad_sync is not None:
                 pl.sync_point(lambda ev: eng._rest_grads_ready(ev))
@@ -458,7 +479,7 @@ class Engine:
         self.cfg = model.config
         self.dev = model.flat_parameters().device
         self.ticket = 0
-        self.arenas: Dict[Tuple[int, bool], Arena] = {}
+        self.arenas: Dict[Tuple[int, bool, int, int], Arena] = {}
         self.grad_sync = None            # parallel.GradSync, set by the caller for N>1
         self.side_stream = torch.cuda.Stream(device=self.dev)    # weight-gradient work of the backward plans
         # top encoder layer computed for the CLS rows only (forward and backward); VITK_CLS_ONLY_TOP=0 runs it densely
@@ -519,11 +540,13 @@ class Engine:
                 "g2": v(p + "layernorm_after.weight"), "b2": v(p + "layernorm_after.bias")})
         return out
 
-    def arena(self, B: int, train: bool) -> Arena:
-        key = (B, train)
+    def arena(self, B: int, train: bool, gh: Optional[int] = None, gw: Optional[int] = None) -> Arena:
+        """The arena of batch size B at the gh × gw patch grid (default: the config's), built on first use."""
+        g0 = self.cfg.image_size // self.cfg.patch_size
+        key = (B, train, g0 if gh is None else gh, g0 if gw is None else gw)
         a = self.arenas.get(key)
         if a is None:
-            a = self.arenas[key] = Arena(self, B, train)
+            a = self.arenas[key] = Arena(self, *key)
         return a
 
     # ------------------------------------------------------------------ forward
@@ -531,15 +554,17 @@ class Engine:
                 output_hidden_states: bool = False):
         """Runs the forward plan → (loss | None, logits, hidden_states | None, attentions | None), all fresh tensors.
         Either flag selects the arena's outputs plan; the attention maps are then recomputed per layer by
-        vitk_attn_probs straight into one [L, B, H, T, T] allocation."""
+        vitk_attn_probs straight into one [L, B, H, T, T] allocation.  The arena is the one of the input's patch grid
+        (H/16 × W/16; the module has checked the size)."""
         cfg = self.cfg
         B = pixel_values.shape[0]
-        ar = self.arena(B, save)
+        Hi, Wi = pixel_values.shape[-2:]
+        ar = self.arena(B, save, Hi // 16, Wi // 16)
         if pixel_values.device != self.dev:
             pixel_values = pixel_values.to(self.dev, non_blocking=True)
         self.model.shadow()                                   # refresh bf16 weights if the masters moved
         if pixel_values.dtype == torch.uint8:
-            x = pixel_values.reshape(B, cfg.image_size, cfg.image_size)
+            x = pixel_values.reshape(B, Hi, Wi)
             ops.patchify_u8(x if x.is_contiguous() else x.contiguous(), cfg.image_mean, cfg.image_std, out=ar.apatch)
         else:
             x = pixel_values if pixel_values.dtype == f32 else pixel_values.to(f32)     # HF:444-446 casts to the weight dtype
@@ -557,7 +582,7 @@ class Engine:
         hidden = ar.hidden_states() if output_hidden_states else None
         attn = None
         if output_attentions:
-            H, L, T = cfg.num_attention_heads, cfg.num_hidden_layers, cfg.seq_len
+            H, L, T = cfg.num_attention_heads, cfg.num_hidden_layers, ar.T
             probs = torch.empty((L, B, H, T, T), dtype=f32, device=self.dev)
             for l in range(L):
                 ops.attn_probs(ar.qkv_all[l], ar.lse_all[l], B, T, H, 64 ** -0.5, out=probs[l])
@@ -584,7 +609,7 @@ class Engine:
         copy); otherwise — gradient accumulation — the kernels write the staging buffer and autograd adds it onto
         ``param.grad``.  When no parameter needs a gradient and ``input_grad`` is set, the arena's data-only plan runs
         instead: no weight-gradient work, no flat gradient buffer and no gradient sync.  With ``input_grad`` the input
-        gradient fp32 [B, 3, S, S] is one UNPATCH_F32 GEMM from the final ``dh`` into a fresh tensor."""
+        gradient fp32 [B, 3, H, W] is one UNPATCH_F32 GEMM from the final ``dh`` into a fresh tensor."""
         ar = next((a for a in self.arenas.values() if a.train and a.ticket == ticket), None)
         if ar is None:
             raise RuntimeError("chest_x_ray_vit_b200: the activations of this forward were overwritten by a later "
@@ -634,14 +659,14 @@ class Engine:
 
     def _input_grad(self, ar: Arena) -> torch.Tensor:
         """d loss / d pixel_values = col2im(dh[:, 1:] · Wp): the final ``dh`` (layer 0's LayerNorm backward wrote it) times
-        the bf16 patch weight [D, 768], scattered into a fresh fp32 [B, 3, S, S] tensor by the UNPATCH_F32 epilogue.
-        vitk_patchify_f32 only reorders and rounds its input, so this is the gradient of the fp32 pixels as passed.
-        Fresh because autograd adopts it as ``x.grad`` without a copy."""
+        the bf16 patch weight [D, 768], scattered into a fresh fp32 [B, 3, 16·gh, 16·gw] tensor by the UNPATCH_F32
+        epilogue (rows_in = patches per image row for a rectangular grid, 0 for a square one).  vitk_patchify_f32 only
+        reorders and rounds its input, so this is the gradient of the fp32 pixels as passed.  Fresh because autograd
+        adopts it as ``x.grad`` without a copy."""
         cfg = self.cfg
-        S = cfg.image_size
-        dx = torch.empty((ar.B, 3, S, S), dtype=f32, device=self.dev)
+        dx = torch.empty((ar.B, 3, 16 * ar.gh, 16 * ar.gw), dtype=f32, device=self.dev)
         ops.gemm(ar.dh[0], self.w["wp16"], ar.M, 768, cfg.hidden_size, dx, epilogue=EPI_UNPATCH_F32, b_mn_major=True,
-                 ldd=S, rows_out=cfg.seq_len, row_off=1)
+                 ldd=16 * ar.gw, rows_out=ar.T, row_off=1, rows_in=0 if ar.gh == ar.gw else ar.gw)
         return dx
 
     def _layers_grads_ready(self, lo: int, hi: int, ev=None) -> None:

@@ -10,6 +10,8 @@ transformers/models/vit/modeling_vit.py:605-653 (HF 5.5.0):
     x.requires_grad_(); model(pixel_values=x).logits[:, c].sum().backward()   # x.grad: saliency / attribution
     out = model(pixel_values=x, output_attentions=True,  # + hidden_states (L+1 × [B,T,D]) and attentions
               output_hidden_states=True)                 #   (L × [B,H,T,T]), as HF's eager attention returns them
+    out = model(pixel_values=x512, labels=y,             # another resolution: the position embeddings resized
+                interpolate_pos_encoding=True)           #   bicubically to the input's patch grid, as in HF
 
 Every FLOP and byte of forward/backward runs in libvitk's sm_100a kernels through the C ABI
 (include/vitk.h); PyTorch provides device memory, streams and the autograd hook only.  There is
@@ -355,7 +357,7 @@ class ViTForImageClassification(nn.Module):
         return self._engine
 
     # ------------------------------------------------------------------ forward
-    def _check_inputs(self, pixel_values: torch.Tensor) -> None:
+    def _check_inputs(self, pixel_values: torch.Tensor, interpolate_pos_encoding: bool = False) -> None:
         cfg = self.config
         if pixel_values.dtype == torch.uint8:
             if pixel_values.dim() == 4 and pixel_values.shape[1] == 1:
@@ -371,7 +373,12 @@ class ViTForImageClassification(nn.Module):
                     "Make sure that the channel dimension of the pixel values match with the one set in the configuration."
                     f" Expected {cfg.num_channels} but got {pixel_values.shape[1]}.")       # HF:155-160
             h, w = pixel_values.shape[-2:]
-        if h != cfg.image_size or w != cfg.image_size:
+        if interpolate_pos_encoding:
+            # HF floors H and W to whole patches (HF:166, 81-82) and drops the remainder pixels; this path does not
+            if h % cfg.patch_size or w % cfg.patch_size or h < cfg.patch_size or w < cfg.patch_size:
+                raise ValueError(f"interpolate_pos_encoding=True needs a height and width that are positive multiples of "
+                                 f"{cfg.patch_size}, got {h}*{w}: crop or pad the image to whole patches")
+        elif h != cfg.image_size or w != cfg.image_size:
             raise ValueError(f"Input image size ({h}*{w}) doesn't match model ({cfg.image_size}*{cfg.image_size}).")  # HF:161-165
 
     def forward(self, pixel_values: Optional[torch.Tensor] = None, labels: Optional[torch.Tensor] = None,
@@ -393,15 +400,26 @@ class ViTForImageClassification(nn.Module):
         respect to ``pixel_values`` as passed (for the collate_fn contract, the normalised image), in its dtype and on its
         device — saliency maps, SmoothGrad, Integrated Gradients.  With every parameter frozen
         (``model.requires_grad_(False)``) backward computes only that gradient: no weight gradients, no ``param.grad``,
-        no data-parallel gradient sync.  uint8 input cannot require grad (torch forbids it)."""
+        no data-parallel gradient sync.  uint8 input cannot require grad (torch forbids it).
+
+        ``interpolate_pos_encoding=True`` (HF modeling_vit.py:60-99) accepts any H×W that is a multiple of 16 on both
+        sides, for every input kind above, in train() and eval(), with labels, hidden states, attention maps and an input
+        gradient.  The H/16 × W/16 patch grid gets position embeddings resized bicubically from the checkpoint's grid
+        (``vitk_pos_interp``), and training sends their gradient back through the resize into ``position_embeddings``,
+        which keeps its checkpoint shape.  As in HF, a square input of the config's size is not resized: it runs exactly
+        the plain call.  Unlike HF, which floors H and W to whole patches, a size that is not a multiple of 16 is rejected.
+        Each grid gets its own activation buffers and launch plans (built on the first call at that size); T = H·W/256 + 1
+        above 4096 runs the top encoder layer on every token.  Hidden states are [B,T,D], attention maps [B,H,T,T] and
+        ``x.grad`` has the input's shape.  The CUDA-graph wrappers of ``graph.py`` stay at the config size."""
         if pixel_values is None:
             raise ValueError("You have to specify pixel_values")                               # HF:440-441
-        if interpolate_pos_encoding:
-            raise ValueError("interpolate_pos_encoding is not supported by the B200 kernel path")
         cfg = self.config
         want_attn = bool(cfg.output_attentions if output_attentions is None else output_attentions)
         want_hidden = bool(cfg.output_hidden_states if output_hidden_states is None else output_hidden_states)
-        self._check_inputs(pixel_values)
+        self._check_inputs(pixel_values, bool(interpolate_pos_encoding))
+        if interpolate_pos_encoding and self._flat_params.device.type != "cuda":
+            raise ValueError("interpolate_pos_encoding=True runs on the CUDA kernel path only: move the model with .cuda() "
+                             "first — there is no CPU path")
         eng = self.engine()
         if labels is not None and cfg.problem_type is None:
             cfg.problem_type = "multi_label_classification"     # HF loss_utils.py:92-98 (float labels)

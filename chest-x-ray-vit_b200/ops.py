@@ -266,6 +266,32 @@ def embed_bwd(dh, B: int, T: int, D: int, dpos, dcls, dbias, dpatch):
     return dpatch
 
 
+def pos_interp(pos: torch.Tensor, gh0: int, gw0: int, gh: int, gw: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Position table fp32 [1 + gh0·gw0, D] at the gh×gw patch grid: row 0 copied, rows 1.. resized bicubically as HF's
+    interpolate_pos_encoding does (modeling_vit.py:60-99) → fp32 [1 + gh·gw, D]."""
+    D = pos.shape[-1]
+    assert pos.dtype == f32 and pos.is_cuda and pos.is_contiguous() and pos.numel() == (1 + gh0 * gw0) * D, \
+        "pos_interp: pos must be a contiguous fp32 CUDA tensor of (1 + gh0·gw0)·D elements"
+    if out is None:
+        out = torch.empty((1 + gh * gw, D), dtype=f32, device=pos.device)
+    assert out.dtype == f32 and out.is_cuda and out.is_contiguous() and out.numel() == (1 + gh * gw) * D, \
+        "pos_interp: out must be a contiguous fp32 CUDA tensor of (1 + gh·gw)·D elements"
+    _lib.check(_lib.lib().vitk_pos_interp(pos.data_ptr(), gh0, gw0, gh, gw, D, out.data_ptr(), _stream()), "pos_interp")
+    return out
+
+
+def pos_interp_bwd(dout: torch.Tensor, gh: int, gw: int, gh0: int, gw0: int, dpos: torch.Tensor) -> torch.Tensor:
+    """Adjoint of pos_interp, accumulated: dpos fp32 [1 + gh0·gw0, D] += Rᵀ · dout fp32 [1 + gh·gw, D] (bit-reproducible)."""
+    D = dout.shape[-1]
+    assert dout.dtype == f32 and dout.is_cuda and dout.is_contiguous() and dout.numel() == (1 + gh * gw) * D, \
+        "pos_interp_bwd: dout must be a contiguous fp32 CUDA tensor of (1 + gh·gw)·D elements"
+    assert dpos.dtype == f32 and dpos.is_cuda and dpos.is_contiguous() and dpos.numel() == (1 + gh0 * gw0) * D, \
+        "pos_interp_bwd: dpos must be a contiguous fp32 CUDA tensor of (1 + gh0·gw0)·D elements"
+    _lib.check(_lib.lib().vitk_pos_interp_bwd(dout.data_ptr(), gh, gw, gh0, gw0, D, dpos.data_ptr(), _stream()),
+               "pos_interp_bwd")
+    return dpos
+
+
 # ----------------------------------------------------------------------------- head + loss
 def head_fwd(h, B: int, T: int, D: int, Cn: int, gamma, beta, eps: float, Wc, bc, labels, logits, loss, dlogits,
              mean, rstd):

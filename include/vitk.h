@@ -112,7 +112,10 @@ enum vitk_epilogue {
                                    q = t − row_off sits at (q / G, q % G) with G² = rows_out − row_off; column
                                    n = c·256 + ky·16 + kx goes to d f32 [g, c, 16·(q/G) + ky, 16·(q%G) + kx] of the NCHW
                                    image [M/rows_out, 3, 16G, 16G].  N = 768, ldd = 16G (the image width),
-                                   M % rows_out == 0; no bias, no aux; every element of d written exactly once */
+                                   M % rows_out == 0; no bias, no aux; every element of d written exactly once.
+                                   rows_in = 0: a square grid, as above.  rows_in > 0: a rectangular grid of rows_in
+                                   patches per image row (G = rows_in, (rows_out − row_off) / rows_in patch rows), so d is
+                                   [M/rows_out, 3, 16·(rows_out − row_off)/rows_in, 16·rows_in] and ldd = 16·rows_in */
 };
 
 typedef struct vitk_gemm_args {
@@ -129,7 +132,8 @@ typedef struct vitk_gemm_args {
   const float* bias;     /* [N] or NULL */
   const void* aux;       /* residual f32 / pos f32 / pre-activation bf16, row stride ld_aux */
   int64_t ld_aux;
-  int64_t rows_in, rows_out, row_off; /* VITK_EPI_PATCH_F32 row remap */
+  int64_t rows_in, rows_out, row_off; /* VITK_EPI_PATCH_F32 row remap; VITK_EPI_UNPATCH_F32 grid (rows_in: patches per
+                                         image row, 0 = square) */
   int32_t tile_n;        /* 0 = library chooses; else 128, 192 or 256 */
   int32_t max_ctas;      /* 0 = all SMs; else cap on the persistent grid, leaving SMs to a concurrent collective */
   int32_t variant;       /* 0 = library chooses; 1 = single-CTA 128×N tiles (gemm.cu); 2 = CTA pair,
@@ -167,6 +171,20 @@ VITK_API int vitk_embed_cls(const float* cls, const float* pos, int64_t B, int64
  * dbias += Σ_{b,t>=1} dh[b,t]; dpatch bf16 [B*(T-1), D] = dh[b,1+p] (compact, for the wgrad GEMM). */
 VITK_API int vitk_embed_bwd(const void* dh_bf16, int64_t B, int64_t T, int64_t D, float* dpos, float* dcls, float* dbias,
                    void* dpatch_bf16, vitk_stream_t stream);
+
+/* Position embeddings at another patch grid (HF ViTEmbeddings.interpolate_pos_encoding, modeling_vit.py:60-99): replaces
+ * the cat(pos[:, :1], F.interpolate(pos[:, 1:].reshape(1, s, s, D).permute(0, 3, 1, 2), size=(gh, gw), mode="bicubic",
+ * align_corners=False).permute(0, 2, 3, 1).view(1, -1, D)) of HF:79-99 and its autograd backward.
+ * vitk_pos_interp: pos fp32 [1 + gh0·gw0, D] → out fp32 [1 + gh·gw, D]; out[0] = pos[0], rows 1.. the gh0×gw0 grid
+ *   resized to gh×gw: out = Wy · pos · Wxᵀ per channel, with Wy [gh, gh0] and Wx [gw, gw0] torch's bicubic matrices
+ *   (cubic convolution, A = −0.75, source coordinate (o + 0.5)·in/out − 0.5, taps clamped to the grid).
+ * vitk_pos_interp_bwd: the exact adjoint, ACCUMULATED: dpos[0] += dout[0], dpos[1..] += Wyᵀ · dout[1..] · Wx per channel;
+ *   every dpos element is summed by one thread in a fixed order (no atomics: two runs give the same bits).
+ * Both: grids 1..4096 per side, D a multiple of 4 up to 4096, buffers 16-byte aligned and not overlapping. */
+VITK_API int vitk_pos_interp(const float* pos, int64_t gh0, int64_t gw0, int64_t gh, int64_t gw, int64_t D, float* out,
+                             vitk_stream_t stream);
+VITK_API int vitk_pos_interp_bwd(const float* dout, int64_t gh, int64_t gw, int64_t gh0, int64_t gw0, int64_t D, float* dpos,
+                                 vitk_stream_t stream);
 
 /* ------------------------------------------------------------------ head + loss
  * Replaces final LayerNorm on the CLS rows, classifier Linear(D→C) and BCEWithLogitsLoss (mean)
